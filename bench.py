@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N ...            # the reference's CPU path (oracle port)
     python bench.py --config C2|C3|C4|C5 ...                 # another BASELINE config (C3 is the headline)
     python bench.py --scaling strong ...                     # the config's reads split over the ranks
+    python bench.py --dump-outputs DIR ...                   # also write the last timed step's table as DIR/*.npy
 
 Workload (config.workload): BASELINE config #3 — 100 M synthetic 250-bp merged amplicon reads
 per GPU, 20-nt adapters, 30 % of adapters mutated with at least one indel (alignment-heavy),
@@ -262,10 +263,13 @@ def run_reference(args):
     cells = 0
     for it in range(args.warmup + args.steps):
         t0 = time.perf_counter()
-        _, _, cells = oracle.process_reads(p, text, off, ln, n_threads=threads, simd=True, as_dict=False)
+        table, _, cells = oracle.process_reads(p, text, off, ln, n_threads=threads, simd=True, as_dict=False)
         dt = time.perf_counter() - t0
         if it >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        import numpy as np
+        dump_outputs(np, args.dump_outputs, [table_sample(np, *table)])
     total = sum(times)
     value = n * len(times) / total
     # the same port one alignment at a time, beside it (a short sample, not part of the timed steps)
@@ -300,27 +304,81 @@ def emit(line):
 REAL_STDOUT = 1
 
 
-def table_checksum(np, offsets, data, counts):
+def key_hashes(np, offsets, data, block_rows=1 << 18):
+    """uint64 mix(key bytes, length) of every row of a (sequence, count) table, a block of rows at a time so that a table
+    of millions of keys needs no more than a few hundred MB of temporaries."""
+    rows = len(offsets) - 1
+    out = np.zeros(max(rows, 0), dtype=np.uint64)
+    for r0 in range(0, rows, block_rows):
+        r1 = min(rows, r0 + block_rows)
+        offs = offsets[r0:r1 + 1].astype(np.int64)
+        d = data[offs[0]:offs[-1]]
+        offs = offs - offs[0]
+        lens = (offs[1:] - offs[:-1]).astype(np.int64)
+        pos = np.arange(len(d), dtype=np.int64) - np.repeat(offs[:-1], lens)
+        w = (pos.astype(np.uint64) * np.uint64(0x9E3779B97F4A7C15) + np.uint64(0xD1342543DE82EF95)) | np.uint64(1)
+        with np.errstate(over="ignore"):
+            terms = (d.astype(np.uint64) + np.uint64(1)) * w
+            nz = lens > 0
+            rowsum = np.zeros(r1 - r0, dtype=np.uint64)
+            if nz.any():
+                rowsum[nz] = np.add.reduceat(terms, offs[:-1][nz])
+            mixed = (rowsum ^ lens.astype(np.uint64)) * np.uint64(0xBF58476D1CE4E5B9)
+            mixed ^= mixed >> np.uint64(29)
+        out[r0:r1] = mixed
+    return out
+
+
+def table_checksum(np, offsets, data, counts, hashes=None):
     """Order-independent 64-bit checksum of a (sequence, count) table: sum over rows of mix(key bytes, length) * (2 count + 1)."""
     rows = len(counts)
     if rows == 0:
         return 0, 0, 0
-    offs = offsets.astype(np.int64)
-    lens = (offs[1:] - offs[:-1]).astype(np.int64)
-    pos = np.arange(len(data), dtype=np.int64) - np.repeat(offs[:-1], lens)
-    w = (pos.astype(np.uint64) * np.uint64(0x9E3779B97F4A7C15) + np.uint64(0xD1342543DE82EF95)) | np.uint64(1)
+    hashes = key_hashes(np, offsets, data) if hashes is None else hashes
     with np.errstate(over="ignore"):
-        terms = (data.astype(np.uint64) + np.uint64(1)) * w
-        starts = offs[:-1].copy()
-        nz = lens > 0
-        rowsum = np.zeros(rows, dtype=np.uint64)
-        if nz.any():
-            red = np.add.reduceat(terms, starts[nz])
-            rowsum[nz] = red
-        mixed = (rowsum ^ lens.astype(np.uint64)) * np.uint64(0xBF58476D1CE4E5B9)
-        mixed ^= mixed >> np.uint64(29)
-        total = (mixed * (counts.astype(np.uint64) * np.uint64(2) + np.uint64(1))).sum(dtype=np.uint64)
+        total = (hashes * (counts.astype(np.uint64) * np.uint64(2) + np.uint64(1))).sum(dtype=np.uint64)
     return int(total), int(rows), int(counts.sum())
+
+
+DUMP_ROWS = 1 << 15         # rows of the table --dump-outputs writes: keys of <= 300 bytes as float32 stay under 40 MB
+DUMP_SEED = 0x5EED5A3B1E0F
+
+
+def table_sample(np, offsets, data, counts, n_rows=DUMP_ROWS):
+    """What --dump-outputs keeps of a (sequence, count) table: its checksum triple and [(rank hash, key, count)] of the
+    n_rows rows of smallest seeded key hash.  Which rows those are depends on the keys alone, not on the table's row order
+    or on how its keys are split over ranks, so two builds are compared row for row."""
+    k = key_hashes(np, offsets, data)
+    with np.errstate(over="ignore"):
+        h = (k ^ np.uint64(DUMP_SEED)) * np.uint64(0x94D049BB133111EB)
+        h ^= h >> np.uint64(31)
+    sel = np.arange(len(h))
+    if len(h) > n_rows:
+        sel = np.nonzero(h <= np.partition(h, n_rows - 1)[n_rows - 1])[0]
+    rows = [(int(h[i]), data[int(offsets[i]):int(offsets[i + 1])].tobytes(), int(counts[i])) for i in sel]
+    return table_checksum(np, offsets, data, counts, k), rows
+
+
+def dump_outputs(np, out_dir, parts, n_rows=DUMP_ROWS):
+    """Writes the table the timed path computed, from the table_sample() of every rank's share of it:
+    table.npy    float64 [rows, counted reads, checksum bits 0-31, checksum bits 32-63] of the whole table;
+    offsets.npy  float64 [n+1], data.npy float32 [key bytes], counts.npy float64 [n]: the sampled rows sorted by key,
+                 in the layout of Context.finish_arrays()."""
+    checksum = sum(p[0][0] for p in parts) % (1 << 64)
+    rows = sorted((r for p in parts for r in p[1]))[:n_rows]       # the global smallest hashes; ties are 1 in 2^64
+    rows.sort(key=lambda r: r[1])
+    lens = [len(r[1]) for r in rows]
+    arrays = {
+        "table": np.array([sum(p[0][1] for p in parts), sum(p[0][2] for p in parts), checksum & 0xFFFFFFFF, checksum >> 32],
+                          dtype=np.float64),
+        "offsets": np.concatenate([[0], np.cumsum(lens)]).astype(np.float64),
+        "data": np.frombuffer(b"".join(r[1] for r in rows), dtype=np.uint8).astype(np.float32),
+        "counts": np.array([r[2] for r in rows], dtype=np.float64),
+    }
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def traffic_record(kernel_file_of):
@@ -369,7 +427,11 @@ def main():
     ap.add_argument("--table-hint", type=int, default=40_000_000, help="expected distinct variants per GPU (table capacity hint)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the table of the last step as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
@@ -498,6 +560,14 @@ def main():
         merge_ms = sum(a.elapsed_time(b) for a, b in merge_events) / max(1, len(merge_events)) if merge_events else 0.0
         clocks = sampler.stop() if rank == 0 else None
         st_timed = ctx.stats()
+        if args.dump_outputs:
+            # the table of the last timed step; after the merge each rank holds the keys it owns
+            part = table_sample(np, *ctx.finish_arrays(copy=False))
+            parts = [part] if world == 1 else [None] * world
+            if world > 1:
+                dist.all_gather_object(parts, part)
+            if rank == 0:
+                dump_outputs(np, args.dump_outputs, parts)
         # per-kernel times for the rooflines: the same steps once more with the batches back to back on ONE stream
         # (in the timed region above consecutive batches overlap on two lanes, so a kernel's duration there includes
         # whatever shared the SMs with it)
@@ -578,7 +648,7 @@ def main():
             t0 = time.perf_counter()
             f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             f0.record(stream)
-            esteps = max(1, min(args.steps, 3))
+            esteps = args.steps
             for _ in range(esteps):
                 d2h = step_e2e()
             f1.record(stream)
