@@ -436,6 +436,13 @@ def test_empty_and_degenerate_inputs():
     otable, odiag, _ = oracle_run(seqs, ad)
     assert_diag_equal(diag, odiag)
     assert table == otable
+    # batches of 64 reads: reads 320-447 and 832-895 make batches of empty reads only (no text at all), between
+    # ordinary ones
+    rng = random.Random(19)
+    seqs = make_reads(rng, PREFIX, SUFFIX, 300) + [b""] * 200 + make_reads(rng, PREFIX, SUFFIX, 300) + [b""] * 100
+    for skip in (False, True):
+        table = gpu_run(seqs, ad, want_diag=False, batch_reads=64, skip_translation=skip)[0]
+        assert table == oracle_run(seqs, ad, skip_translation=skip)[0]
 
 
 def test_ragged_lengths_and_long_reads():

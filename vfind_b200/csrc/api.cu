@@ -613,15 +613,12 @@ int vfb_create(const vfb_params *p, vfb_ctx **out)
         ev_ok = ev_ok && new_event(&ln.done) && new_event(&ln.ev_scanned) && new_event(&ln.ev_aligned) &&
                 (e = cudaStreamCreateWithPriority(&ln.st, cudaStreamNonBlocking, prio_hi)) == cudaSuccess &&
                 (e = cudaStreamCreateWithPriority(&ln.st_dp, cudaStreamNonBlocking, prio_lo)) == cudaSuccess;
-    c->split_dp = true;
-    if (const char *se = getenv("VFB_SPLIT_DP")) c->split_dp = atoi(se) != 0;
     c->fused_count = true;
     if (const char *se = getenv("VFB_FUSED_COUNT")) c->fused_count = atoi(se) != 0;
     if (!ev_ok) return fail(cuda_fail(e, "cudaEventCreate / cudaStreamCreate", __FILE__, __LINE__));
-    // two lanes unless the per-read diagnostics of "the last batch" are wanted (or VFB_LANES=1 says so)
+    // two lanes unless the per-read diagnostics of "the last batch" are wanted
     c->n_lanes = VFB_LANES;
     if (p->diagnostics) c->n_lanes = 1;
-    if (const char *le = getenv("VFB_LANES")) if (atoi(le) == 1) c->n_lanes = 1;
 
     // DP setup: packed layout when the scores fit, else the fallback kernel
     const bool force_generic = p->force_generic_dp != 0;
@@ -842,7 +839,6 @@ static int run_dp(vfb_ctx *c, Lane &ln, cudaStream_t st, const uint8_t *d_text, 
         gj.base = job;
         gj.base.worklist = fb;
         gj.base.n_items = nfb;
-        gj.base.cells = nullptr;     // already counted by the packed kernel? no: it skipped them
         gj.base.cells = job.cells;
         if ((rc = launch_dp_generic(gj, c->sm_count, st))) return rc;
         c->stats.dp_kernel_launches += 2;
@@ -933,7 +929,7 @@ static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_sp
     // either way, src/lib.rs:288), reads it accepts join the suffix worklist if they need one.
     // split mode: the (ALU-bound) alignment kernels of the batch run on the lane's lower-priority stream, so that the
     // other lane's memory-bound kernels get SM resources as soon as alignment blocks retire
-    const bool split = c->split_dp && c->n_lanes > 1 && !prof;
+    const bool split = c->n_lanes > 1 && !prof;
     cudaStream_t sd = split ? ln.st_dp : st;
     if (split) {
         VFB_CUDA(cudaEventRecord(ln.ev_scanned, st));

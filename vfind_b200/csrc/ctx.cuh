@@ -149,8 +149,7 @@ struct vfb_ctx {
 
     // per-batch scratch, one set per lane
     vfb::Lane lanes[VFB_LANES];
-    int n_lanes = VFB_LANES;                    // 1: every batch on the compute stream itself (diagnostics, VFB_LANES=1)
-    bool split_dp = true;                       // a lane's alignment kernels on a lower-priority stream (VFB_SPLIT_DP=0: off)
+    int n_lanes = VFB_LANES;                    // 1: every batch on the compute stream itself (diagnostics, vfb_set_lanes)
     bool fused_count = true;                    // the key kernel probes the table itself (VFB_FUSED_COUNT=0: K3 then K4 over every read)
     uint64_t lane_seq = 0;
     cudaEvent_t ev_fork = nullptr, ev_k4 = nullptr;   // compute stream -> lane; the previous batch's insert is done

@@ -1068,7 +1068,6 @@ int vfb_internal_run_file(vfb_ctx **ctxs, uint32_t n_ctx, const char *path, uint
 
     constexpr int NCH = 3;
     Chunk ch[NCH];
-    const bool dev_handoff = !(getenv("VFB_GUNZIP_HANDOFF") && getenv("VFB_GUNZIP_HANDOFF")[0] == '0');
     std::vector<cudaEvent_t> ch_events((size_t)NCH * n_ctx, nullptr);     // [chunk][context]: an event belongs to a device
     int ch_ctx[NCH] = {0, 0, 0};
     Pipe pp;
@@ -1104,7 +1103,7 @@ int vfb_internal_run_file(vfb_ctx **ctxs, uint32_t n_ctx, const char *path, uint
             }
             bool last = false;
             const auto t0 = std::chrono::steady_clock::now();
-            const int prc = prod.next(ch[k].buf, cap, &ch[k].cut, &ch[k].lines, &last, dev_handoff ? &ch[k].dev : nullptr, &ch[k].dev_len);
+            const int prc = prod.next(ch[k].buf, cap, &ch[k].cut, &ch[k].lines, &last, &ch[k].dev, &ch[k].dev_len);
             if (trace) fprintf(stderr, "[vfb ingest] chunk %zu bytes %zu lines inflated in %.1f ms\n", ch[k].cut, ch[k].lines,
                                std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
             std::lock_guard<std::mutex> lk(pp.mu);

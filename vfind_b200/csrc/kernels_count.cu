@@ -9,8 +9,6 @@
 #include "translate_fast.h"
 #include "vfb_internal.cuh"
 
-#include <stdlib.h>
-
 namespace vfb {
 
 // ------------------------------------------------------------------------------------ K3
@@ -65,175 +63,9 @@ __device__ bool utf8_valid(const uint8_t *s, uint32_t n)
     return true;
 }
 
-#define KEY_THREADS 256
-#define KEY_WARPS (KEY_THREADS / 32)
-#define KEY_GROUP 4                 // lanes per read in the translate phase
-#define KEY_RPS (32 / KEY_GROUP)    // reads per sub-step of the translate phase
 #define KEY_MULTS 128               // hash multipliers kept in shared memory
 
-struct KeyTables {
-    // byte -> base index 0..4 (bytes >= 128 -> 4), premultiplied for the three codon positions
-    uint8_t lut25[256], lut5[256], lut1[256];
-    uint8_t aa[128];                // c0*25 + c1*5 + c2 -> amino acid, 'X' if any index is 4
-    uint64_t mult[KEY_MULTS];       // vfb_hash_mult(i)
-    uint8_t order[KEY_WARPS][32];   // per warp: lanes that own a key, compacted
-};
-
-__device__ __forceinline__ uint64_t key_mult(const KeyTables *T, uint32_t i)
-{
-    return i < KEY_MULTS ? T->mult[i] : vfb_hash_mult(i);
-}
-
-// 12 (or 4) consecutive text bytes starting at `a` as little-endian words, from aligned loads
-// that never touch a word at or beyond `limit` (the 4-aligned end of the region's last byte).
-template <int NW>
-__device__ __forceinline__ void load_unaligned(const uint8_t *a, const uint8_t *limit, uint32_t *out)
-{
-    const uint32_t sh = (uint32_t)(reinterpret_cast<uintptr_t>(a) & 3u) * 8u;
-    const uint32_t *w = reinterpret_cast<const uint32_t *>(a - (sh >> 3));
-    uint32_t t[NW + 1];
-#pragma unroll
-    for (int j = 0; j <= NW; ++j)
-        t[j] = reinterpret_cast<const uint8_t *>(w + j) < limit ? __ldg(w + j) : 0u;
-#pragma unroll
-    for (int j = 0; j < NW; ++j) out[j] = __funnelshift_r(t[j], t[j + 1], sh);
-}
-
-// Phase A: one lane per read decides the key length and claims key space (one atomic per
-// 32 reads); the lanes that own a key are compacted.  Phase B: lane groups of 4 translate 8
-// of those reads at a time, one 32-bit word of key (4 amino acids = 12 bases) per lane per
-// step, hashing the words they hold.
-__global__ void __launch_bounds__(KEY_THREADS)
-k3_keys(const __grid_constant__ KeyJob job)
-{
-    __shared__ KeyTables T;
-    for (int i = threadIdx.x; i < 256; i += blockDim.x) {
-        const uint32_t c = i >= 128 ? 4u : tr_index((uint8_t)i);
-        T.lut25[i] = (uint8_t)(25u * c); T.lut5[i] = (uint8_t)(5u * c); T.lut1[i] = (uint8_t)c;
-    }
-    for (int i = threadIdx.x; i < 128; i += blockDim.x) {
-        const int c0 = i / 25, c1 = (i / 5) % 5, c2 = i % 5;
-        T.aa[i] = (i >= 125 || c0 == 4 || c1 == 4 || c2 == 4) ? (uint8_t)'X' : (uint8_t)c_aa[c0 * 16 + c1 * 4 + c2];
-    }
-    for (int i = threadIdx.x; i < KEY_MULTS; i += blockDim.x) T.mult[i] = vfb_hash_mult((uint32_t)i);
-    __syncthreads();
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int g = lane & (KEY_GROUP - 1), grp = lane / KEY_GROUP;
-    const uint32_t warps_total = gridDim.x * KEY_WARPS;
-    const uint32_t n_rounds = (job.n_reads + 31) / 32;
-    for (uint32_t round = blockIdx.x * KEY_WARPS + warp; round < n_rounds; round += warps_total) {
-        // ---- phase A
-        const uint32_t r = round * 32 + lane;
-        uint32_t klen = 0, V = 0;
-        const uint8_t *var = job.text;
-        if (r < job.n_reads) {
-            const uint32_t s = job.start[r], e = job.end[r];
-            // src/lib.rs:288: both located and start < end (strict).  end <= len always holds
-            // for located suffix boundaries; a prefix boundary beyond it fails start < end.
-            if (s != VFB_NONE && e != VFB_NONE && s < e) {
-                const vfb_span sp = job.spans[r];
-                if (e <= sp.len) {
-                    V = e - s;
-                    var = job.text + sp.off + s;
-                    if (job.skip_translation) klen = V;
-                    else if (V % 3 == 0) klen = V / 3;                 // :17-19 partial codon -> None
-                }
-            }
-        }
-        const unsigned owners = __ballot_sync(0xffffffffu, klen != 0);
-        if (owners == 0) {
-            if (r < job.n_reads) job.klen[r] = 0;
-            continue;
-        }
-        const uint32_t padded = (klen + 15u) & ~15u;
-        uint32_t incl = padded;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += t;
-        }
-        unsigned long long base = 0;
-        const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
-        if (lane == 31) base = atomicAdd(job.key_cursor, (unsigned long long)total);
-        base = __shfl_sync(0xffffffffu, base, 31);
-        const unsigned long long koff = base + (incl - padded);
-        if (klen) {
-            job.koff[r] = koff;
-            T.order[warp][__popc(owners & ((1u << lane) - 1u))] = (uint8_t)lane;
-        }
-        __syncwarp();
-        const int n_own = __popc(owners);
-        uint32_t bad_mask = 0;       // reads whose raw region is not valid UTF-8 (skip_translation only)
-        // ---- phase B
-#pragma unroll 1
-        for (int sub = 0; sub * KEY_RPS < n_own; ++sub) {
-            const int k = sub * KEY_RPS + grp;
-            const bool have = k < n_own;
-            const int owner = have ? T.order[warp][k] : 0;
-            const uint32_t kl_owner = __shfl_sync(0xffffffffu, klen, owner);
-            const uint32_t kl = have ? kl_owner : 0u;
-            const uint32_t vv = __shfl_sync(0xffffffffu, V, owner);
-            const unsigned long long ko = __shfl_sync(0xffffffffu, koff, owner);
-            const uintptr_t va = __shfl_sync(0xffffffffu, (unsigned long long)reinterpret_cast<uintptr_t>(var), owner);
-            const uint8_t *src = reinterpret_cast<const uint8_t *>(va);
-            const uint8_t *limit = reinterpret_cast<const uint8_t *>((va + vv + 3) & ~(uintptr_t)3);
-            uint32_t *key = reinterpret_cast<uint32_t *>(job.keys + ko);
-            const uint32_t nw = (kl + 3) >> 2, npad = ((kl + 15u) & ~15u) >> 2;
-            uint64_t acc = 0;
-            uint32_t high = 0;
-            for (uint32_t wi = g; wi < npad; wi += KEY_GROUP) {
-                uint32_t word = 0;
-                if (wi < nw) {
-                    if (!job.skip_translation) {
-                        uint32_t x[3];
-                        load_unaligned<3>(src + 12 * wi, limit, x);
-                        // codon a = bytes 3a .. 3a+2 of the 12
-                        const uint32_t i0 = T.lut25[x[0] & 0xFFu] + T.lut5[(x[0] >> 8) & 0xFFu] + T.lut1[(x[0] >> 16) & 0xFFu];
-                        const uint32_t i1 = T.lut25[x[0] >> 24] + T.lut5[x[1] & 0xFFu] + T.lut1[(x[1] >> 8) & 0xFFu];
-                        const uint32_t i2 = T.lut25[(x[1] >> 16) & 0xFFu] + T.lut5[x[1] >> 24] + T.lut1[x[2] & 0xFFu];
-                        const uint32_t i3 = T.lut25[(x[2] >> 8) & 0xFFu] + T.lut5[(x[2] >> 16) & 0xFFu] + T.lut1[x[2] >> 24];
-                        word = (uint32_t)T.aa[i0] | ((uint32_t)T.aa[i1] << 8) | ((uint32_t)T.aa[i2] << 16) | ((uint32_t)T.aa[i3] << 24);
-                        const uint32_t n_aa = kl - 4 * wi;             // >= 1
-                        if (n_aa < 4) word &= (1u << (8 * n_aa)) - 1u;
-                    } else {
-                        load_unaligned<1>(src + 4 * wi, limit, &word);
-                        const uint32_t nb = min(4u, kl - 4 * wi);
-                        if (nb < 4) word &= (1u << (8 * nb)) - 1u;
-                        high |= word & 0x80808080u;
-                    }
-                    acc += (uint64_t)(word ^ VFB_HASH_K) * key_mult(&T, wi);
-                }
-                key[wi] = word;
-            }
-#pragma unroll
-            for (int o = KEY_GROUP / 2; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-            if (g == 0 && kl) {
-                uint64_t h = vfb_hash_finish(acc, kl);
-                if (job.hash_bits > 0 && job.hash_bits < 64) h &= (1ull << job.hash_bits) - 1;
-                job.khash[round * 32 + owner] = h;
-            }
-            if (job.skip_translation) {
-                // String::from_utf8 (:295): only regions holding a byte >= 0x80 need the validator
-#pragma unroll
-                for (int o = KEY_GROUP / 2; o > 0; o >>= 1) high |= __shfl_xor_sync(0xffffffffu, high, o);
-                bool bad = false;
-                if (g == 0 && kl && high) bad = !utf8_valid(src, vv);
-                const unsigned bm = __ballot_sync(0xffffffffu, bad);
-#pragma unroll
-                for (int q = 0; q < KEY_RPS; ++q) {
-                    const uint32_t q_owner = __shfl_sync(0xffffffffu, (uint32_t)owner, q * KEY_GROUP);
-                    if (bm & (1u << (q * KEY_GROUP))) bad_mask |= 1u << q_owner;
-                }
-            }
-        }
-        __syncwarp();
-        if (bad_mask & (1u << lane)) klen = 0;
-        if (r < job.n_reads) job.klen[r] = klen;
-    }
-}
-
-// ---- tile version: the text range that covers the regions of a warp's 32 reads is staged in shared
+// ---- k3_keys_tile: the text range that covers the regions of a warp's 32 reads is staged in shared
 // memory by one bulk copy (TMA, completion on an mbarrier), as in k1_scan_tile; one lane owns one read
 // and walks its region out of shared memory (no global-load latency inside the translate loop); the
 // unit's keys are assembled in shared memory and leave with coalesced 16-byte stores; koff / klen /
@@ -415,21 +247,25 @@ k3_keys_tile(const __grid_constant__ KeyJob job, const uint32_t tile_bytes)
     }
 }
 
+// Shared memory of a k3_keys_tile block of `w` warps: their tiles and key staging (dynamic), the tables and barriers,
+// and a reserve.
+static constexpr size_t keys_tile_block_smem(size_t tile, int w)
+{
+    return (size_t)w * (tile + K3T_SLACK + K3T_OUT_BYTES) + sizeof(Key3Tables) + 64 + 1024;
+}
+static_assert(keys_tile_block_smem(VFB_TILE_BYTES_MAX, 1) <= VFB_SMEM_BLOCK_MAX, "a block of one warp fits any tile");
+
 template <bool TRANSLATE>
 static int launch_keys_tile(const KeyJob &job, cudaStream_t st)
 {
     const uint32_t tile = vfb_tile_bytes_for(job.text_bytes, job.n_reads);
-    const size_t smem_cap = 227 * 1024;
-    const size_t per_warp = (size_t)tile + K3T_SLACK + K3T_OUT_BYTES;
-    int best_w = 0, best_total = 0;
+    int best_w = 1, best_total = 0;
     for (int w = K3T_WARPS_MAX; w >= 1; w >>= 1) {
-        const size_t per_block = (size_t)w * per_warp + sizeof(Key3Tables) + 64 + 1024;
-        int bps = (int)(smem_cap / per_block);
+        int bps = (int)(VFB_SMEM_BLOCK_MAX / keys_tile_block_smem(tile, w));
         if (bps * w > 32) bps = 32 / w;
         if (bps * w > best_total) { best_total = bps * w; best_w = w; }
     }
-    if (best_total == 0) return -1;
-    const size_t smem = (size_t)best_w * per_warp;
+    const size_t smem = (size_t)best_w * (tile + K3T_SLACK + K3T_OUT_BYTES);
     VFB_CUDA(cudaFuncSetAttribute(k3_keys_tile<TRANSLATE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const uint32_t units = (job.n_reads + 31) / 32;
     uint32_t blocks = (units + best_w - 1) / best_w;
@@ -441,21 +277,9 @@ static int launch_keys_tile(const KeyJob &job, cudaStream_t st)
 
 int launch_keys(const KeyJob &job, cudaStream_t st)
 {
-    static const bool old_keys = getenv("VFB_KEYS_TILE") && atoi(getenv("VFB_KEYS_TILE")) == 0;
-    if (job.n_reads && job.text_bytes && !old_keys) {
-        const int rc = job.skip_translation ? launch_keys_tile<false>(job, st) : launch_keys_tile<true>(job, st);
-        if (rc > 0) return rc;
-        if (rc == VFB_OK) {
-            ++g_launches;
-            VFB_CUDA(cudaGetLastError());
-            return VFB_OK;
-        }
-    }
     if (job.n_reads == 0) return VFB_OK;
-    uint32_t blocks = (job.n_reads / 32 + (KEY_THREADS / 32)) / (KEY_THREADS / 32);
-    if (blocks > 148 * 8) blocks = 148 * 8;
-    if (blocks < 1) blocks = 1;
-    k3_keys<<<blocks, KEY_THREADS, 0, st>>>(job);
+    const int rc = job.skip_translation ? launch_keys_tile<false>(job, st) : launch_keys_tile<true>(job, st);
+    if (rc != VFB_OK) return rc;
     ++g_launches;
     VFB_CUDA(cudaGetLastError());
     return VFB_OK;
@@ -1032,13 +856,12 @@ static int launch_keys_count_t(const KeyJob &job, const DevTable &tab, uint32_t 
     uint32_t out_bytes = (uint32_t)(32 * ((key_ub + 15) & ~15ull));
     if (out_bytes < 1024) out_bytes = 1024;
     if (out_bytes > 4096u) out_bytes = 4096u;
-    const size_t smem_cap = 227 * 1024;
     const size_t per_warp = (size_t)tile + K3T_SLACK + 3 * (size_t)out_bytes + K34_STAGE_BYTES;
     // as many warps per SM as the shared memory allows; the tables are per block, so few large blocks
     int best_w = 0, best_total = 0;
     for (int w = K34_WARPS_MAX; w >= 1; --w) {
         const size_t per_block = (size_t)w * per_warp + sizeof(Key34Tables) + 8 * K34_WARPS_MAX + 1024;
-        int bps = (int)(smem_cap / per_block);
+        int bps = (int)(VFB_SMEM_BLOCK_MAX / per_block);
         if (bps * w > 16) bps = 16 / w;               // 128 registers per thread: 16 warps fit the register file
         if (bps * w > best_total) { best_total = bps * w; best_w = w; }
     }

@@ -1,27 +1,24 @@
-// GPU inflate of block-gzip members (ingest, SURVEY §8(f) next-1: "GPU inflate for multi-member
-// (BGZF-style) input").
+// GPU inflate of gzip input (ingest, SURVEY §8(f) next-1: replaces flate2's MultiGzDecoder).
 //
-// Replaces flate2's MultiGzDecoder (/root/reference/src/lib.rs:233) for input whose members
-// carry their own compressed size (BGZF "BC" extra field) and are therefore independent streams
-// of at most 64 KiB: one thread inflates one member, thousands of members per launch.  The
-// decoder is a plain RFC 1951 decoder (stored / fixed / dynamic blocks, canonical Huffman codes
-// decoded length by length); per-thread tables live in local memory, the four base/extra
-// tables in shared memory.  Each member's CRC-32 and ISIZE (RFC 1952 trailer) are checked, as
-// flate2 does; the first bad member is reported.
-#include <cstdlib>
-
+// k_inflate_warp inflates block-gzip (BGZF-style) members, which carry their own compressed size ("BC" extra field)
+// and are therefore independent streams of at most 64 KiB: one WARP per member, thousands of members per launch,
+// table-driven.  All 32 lanes run the same decode (same bit buffer, same tables: no divergence, no broadcasts); the
+// lanes differ only where a warp helps: the compressed input arrives through a 512-byte shared-memory ring that the
+// lanes top up with coalesced 128-byte loads ahead of the bit reader, Huffman decode is one shared-memory lookup per
+// symbol (9-bit table for literal/length codes, 8-bit for distances, built by all lanes from the canonical code;
+// longer codes fall back to the bit-by-bit canonical decode), a match is copied by all lanes at once (period `dist`
+// when it overlaps itself), and the CRC-32 is computed after the decode, each lane over 1/32 of the output, the
+// partial CRCs combined with x^(8n) mod P multiplications.  Each member's CRC-32 and ISIZE (RFC 1952 trailer) are
+// checked, as flate2 does; the first bad member is reported.
+//
+// The k_gz_* kernels further down decode ONE long deflate stream (what `gzip` writes) from speculative block starts,
+// with the same warp decoder's tables and symbol loop.
 #include "vfb_internal.cuh"
 
 namespace vfb {
 
 #define INF_MAXBITS 15
 #define INF_MAXL 288
-#define INF_MAXD 30
-
-struct Huff {
-    short count[INF_MAXBITS + 1];
-    short symbol[INF_MAXL];
-};
 
 struct InfTables {
     unsigned short lbase[29], lext[29], dbase[30], dext[30];
@@ -29,246 +26,14 @@ struct InfTables {
     uint32_t crc[256];
 };
 
-struct BitReader {
-    const uint8_t *in, *end;
-    uint64_t buf;
-    int cnt;
-    bool over;     // ran past the end of the member
-};
-
-__device__ __forceinline__ void br_refill(BitReader &b)
-{
-    while (b.cnt <= 56) {
-        if (b.in < b.end) b.buf |= (uint64_t)(*b.in++) << b.cnt;
-        else if (b.in >= b.end + 8) { b.over = true; }
-        else ++b.in;                                   // zero padding past the end, bounded
-        b.cnt += 8;
-    }
-}
-
-__device__ __forceinline__ uint32_t br_bits(BitReader &b, int n)
-{
-    if (b.cnt < n) br_refill(b);
-    const uint32_t v = (uint32_t)(b.buf & ((1ull << n) - 1ull));
-    b.buf >>= n;
-    b.cnt -= n;
-    return v;
-}
-
-// Canonical Huffman decode, one bit at a time (codes are stored MSB first).
-__device__ __forceinline__ int huff_decode(BitReader &b, const Huff &h)
-{
-    if (b.cnt < INF_MAXBITS) br_refill(b);
-    int code = 0, first = 0, index = 0;
-    uint64_t bits = b.buf;
-    for (int len = 1; len <= INF_MAXBITS; ++len) {
-        code |= (int)(bits & 1u);
-        bits >>= 1;
-        const int count = h.count[len];
-        if (code - count < first) {
-            b.buf >>= len;
-            b.cnt -= len;
-            return h.symbol[index + (code - first)];
-        }
-        index += count;
-        first += count;
-        first <<= 1;
-        code <<= 1;
-    }
-    return -1;
-}
-
-// Build a canonical code from code lengths.  Returns <0 if over-subscribed, >0 if incomplete.
-__device__ int huff_construct(Huff &h, const short *length, int n)
-{
-    short offs[INF_MAXBITS + 1];
-    for (int len = 0; len <= INF_MAXBITS; ++len) h.count[len] = 0;
-    for (int s = 0; s < n; ++s) h.count[length[s]]++;
-    if (h.count[0] == n) return 0;
-    int left = 1;
-    for (int len = 1; len <= INF_MAXBITS; ++len) {
-        left <<= 1;
-        left -= h.count[len];
-        if (left < 0) return left;
-    }
-    offs[1] = 0;
-    for (int len = 1; len < INF_MAXBITS; ++len) offs[len + 1] = offs[len] + h.count[len];
-    for (int s = 0; s < n; ++s)
-        if (length[s] != 0) h.symbol[offs[length[s]]++] = (short)s;
-    return left;
-}
-
 struct InflateArgs {
     const uint8_t *z;            // compressed members, back to back as read from the file
     const vfb_member *members;   // per member: offset/size in z, offset in out, ISIZE
     uint32_t n_members;
     uint8_t *out;
     uint32_t *first_bad;         // atomicMin of the first member that failed
-    uint32_t lanes;              // lanes of each warp that decode (1 = lane 0 only)
 };
 
-// error codes are only used to tell "ok" from "bad"
-__device__ int inflate_member(const InfTables *T, const uint8_t *zin, uint32_t zlen, uint8_t *out, uint32_t isize)
-{
-    // gzip header (RFC 1952): fixed 10 bytes, optional FEXTRA / FNAME / FCOMMENT / FHCRC
-    if (zlen < 18 || zin[0] != 0x1f || zin[1] != 0x8b || zin[2] != 8) return -1;
-    const uint32_t flg = zin[3];
-    uint32_t p = 10;
-    if (flg & 4) { if (p + 2 > zlen) return -1; p += 2 + (zin[p] | (zin[p + 1] << 8)); }
-    if (flg & 8) { while (p < zlen && zin[p]) ++p; ++p; }
-    if (flg & 16) { while (p < zlen && zin[p]) ++p; ++p; }
-    if (flg & 2) p += 2;
-    if (p + 8 > zlen) return -1;
-    const uint8_t *tr = zin + zlen - 8;
-    const uint32_t want_crc = tr[0] | (tr[1] << 8) | (tr[2] << 16) | ((uint32_t)tr[3] << 24);
-    const uint32_t want_len = tr[4] | (tr[5] << 8) | (tr[6] << 16) | ((uint32_t)tr[7] << 24);
-    if (want_len != isize) return -2;
-
-    BitReader b;
-    b.in = zin + p; b.end = zin + zlen - 8; b.buf = 0; b.cnt = 0; b.over = false;
-    Huff lencode, distcode;
-    short lengths[INF_MAXL + INF_MAXD];
-    uint32_t n_out = 0, crc = 0xFFFFFFFFu;
-    int last;
-    do {
-        last = (int)br_bits(b, 1);
-        const uint32_t type = br_bits(b, 2);
-        if (type == 0) {
-            // stored: skip to a byte boundary, LEN, NLEN, bytes
-            const int drop = b.cnt & 7;
-            b.buf >>= drop; b.cnt -= drop;
-            const uint32_t len = br_bits(b, 16), nlen = br_bits(b, 16);
-            if ((len ^ 0xFFFFu) != nlen) return -3;
-            if (n_out + len > isize) return -4;
-            for (uint32_t i = 0; i < len; ++i) {
-                const uint32_t c = br_bits(b, 8);
-                out[n_out++] = (uint8_t)c;
-                crc = T->crc[(crc ^ c) & 0xFFu] ^ (crc >> 8);
-            }
-        } else if (type == 1 || type == 2) {
-            if (type == 1) {
-                int s = 0;
-                for (; s < 144; ++s) lengths[s] = 8;
-                for (; s < 256; ++s) lengths[s] = 9;
-                for (; s < 280; ++s) lengths[s] = 7;
-                for (; s < 288; ++s) lengths[s] = 8;
-                huff_construct(lencode, lengths, 288);
-                for (s = 0; s < 30; ++s) lengths[s] = 5;
-                huff_construct(distcode, lengths, 30);
-            } else {
-                const int nlen = (int)br_bits(b, 5) + 257, ndist = (int)br_bits(b, 5) + 1, ncode = (int)br_bits(b, 4) + 4;
-                if (nlen > 286 || ndist > 30) return -5;
-                int idx = 0;
-                for (; idx < ncode; ++idx) lengths[T->order[idx]] = (short)br_bits(b, 3);
-                for (; idx < 19; ++idx) lengths[T->order[idx]] = 0;
-                if (huff_construct(lencode, lengths, 19) != 0) return -6;     // must be complete
-                idx = 0;
-                while (idx < nlen + ndist) {
-                    int sym = huff_decode(b, lencode);
-                    if (sym < 0) return -7;
-                    if (sym < 16) {
-                        lengths[idx++] = (short)sym;
-                    } else {
-                        int len = 0, rep;
-                        if (sym == 16) {
-                            if (idx == 0) return -8;
-                            len = lengths[idx - 1];
-                            rep = 3 + (int)br_bits(b, 2);
-                        } else if (sym == 17) rep = 3 + (int)br_bits(b, 3);
-                        else rep = 11 + (int)br_bits(b, 7);
-                        if (idx + rep > nlen + ndist) return -9;
-                        while (rep--) lengths[idx++] = (short)len;
-                    }
-                }
-                if (lengths[256] == 0) return -10;
-                int err = huff_construct(lencode, lengths, nlen);
-                if (err < 0 || (err > 0 && nlen - lencode.count[0] != 1)) return -11;
-                err = huff_construct(distcode, lengths + nlen, ndist);
-                if (err < 0 || (err > 0 && ndist - distcode.count[0] != 1)) return -12;
-            }
-            // decode literals / length-distance pairs until end-of-block
-            for (;;) {
-                int sym = huff_decode(b, lencode);
-                if (sym < 0) return -13;
-                if (sym < 256) {
-                    if (n_out >= isize) return -14;
-                    out[n_out++] = (uint8_t)sym;
-                    crc = T->crc[(crc ^ (uint32_t)sym) & 0xFFu] ^ (crc >> 8);
-                } else if (sym == 256) {
-                    break;
-                } else {
-                    sym -= 257;
-                    if (sym >= 29) return -15;
-                    const uint32_t len = T->lbase[sym] + br_bits(b, T->lext[sym]);
-                    const int ds = huff_decode(b, distcode);
-                    if (ds < 0 || ds >= 30) return -16;
-                    const uint32_t dist = T->dbase[ds] + br_bits(b, T->dext[ds]);
-                    if (dist > n_out) return -17;
-                    if (n_out + len > isize) return -18;
-                    for (uint32_t i = 0; i < len; ++i) {
-                        const uint8_t c = out[n_out - dist];
-                        out[n_out++] = c;
-                        crc = T->crc[(crc ^ c) & 0xFFu] ^ (crc >> 8);
-                    }
-                }
-                if (b.over) return -19;
-            }
-        } else {
-            return -20;
-        }
-        if (b.over) return -19;
-    } while (!last);
-    if (n_out != isize) return -21;
-    if ((crc ^ 0xFFFFFFFFu) != want_crc) return -22;
-    return 0;
-}
-
-#define INF_THREADS 128
-
-__global__ void __launch_bounds__(INF_THREADS)
-k_inflate_members(const __grid_constant__ InflateArgs a)
-{
-    __shared__ InfTables T;
-    if (threadIdx.x == 0) {
-        const unsigned short lb[29] = {3, 4, 5, 6, 7, 8, 9, 10, 11, 13, 15, 17, 19, 23, 27, 31, 35, 43, 51, 59, 67, 83, 99, 115, 131, 163, 195, 227, 258};
-        const unsigned short le[29] = {0, 0, 0, 0, 0, 0, 0, 0, 1, 1, 1, 1, 2, 2, 2, 2, 3, 3, 3, 3, 4, 4, 4, 4, 5, 5, 5, 5, 0};
-        const unsigned short db[30] = {1, 2, 3, 4, 5, 7, 9, 13, 17, 25, 33, 49, 65, 97, 129, 193, 257, 385, 513, 769, 1025, 1537, 2049, 3073, 4097, 6145, 8193, 12289, 16385, 24577};
-        const unsigned short de[30] = {0, 0, 0, 0, 1, 1, 2, 2, 3, 3, 4, 4, 5, 5, 6, 6, 7, 7, 8, 8, 9, 9, 10, 10, 11, 11, 12, 12, 13, 13};
-        const unsigned char od[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
-        for (int i = 0; i < 29; ++i) { T.lbase[i] = lb[i]; T.lext[i] = le[i]; }
-        for (int i = 0; i < 30; ++i) { T.dbase[i] = db[i]; T.dext[i] = de[i]; }
-        for (int i = 0; i < 19; ++i) T.order[i] = od[i];
-    }
-    for (int i = threadIdx.x; i < 256; i += blockDim.x) {
-        uint32_t c = (uint32_t)i;
-        for (int k = 0; k < 8; ++k) c = (c & 1u) ? 0xEDB88320u ^ (c >> 1) : c >> 1;
-        T.crc[i] = c;
-    }
-    __syncthreads();
-    // Decoding is branchy and every stream takes its own path: lanes of a warp that decode
-    // different members serialise each other.  So only `lanes` lanes per warp decode (default 1:
-    // a warp is one independent decoder and the SM interleaves warps instead of lanes).
-    const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (lane >= a.lanes) return;
-    const uint32_t i = warp * a.lanes + lane;
-    if (i >= a.n_members) return;
-    const vfb_member m = a.members[i];
-    int rc = 0;
-    if (m.isize || m.z_len) rc = inflate_member(&T, a.z + m.z_off, m.z_len, a.out + m.out_off, m.isize);
-    if (rc != 0) atomicMin(a.first_bad, i);
-}
-
-// =====================================================================================
-// v2: one WARP per member, table-driven.
-//
-// All 32 lanes run the same decode (same bit buffer, same tables: no divergence, no broadcasts);
-// the lanes differ only where a warp helps: the compressed input arrives through a 512-byte
-// shared-memory ring that the lanes top up with coalesced 128-byte loads three lines ahead of
-// the bit reader, Huffman decode is one shared-memory lookup per symbol (10-bit table for
-// literal/length codes, 8-bit for distances, built by all lanes from the canonical code; longer
-// codes fall back to the bit-by-bit canonical decode), a match is copied by all lanes at once
-// (period `dist` when it overlaps itself), and the CRC-32 is computed after the decode, each
-// lane over 1/32 of the output, the partial CRCs combined with x^(8n) mod P multiplications.
 #define INFW_WARPS 4
 #define INFW_LBITS 9
 #define INFW_DBITS 8
@@ -721,8 +486,7 @@ __device__ int inflate_member_warp(const InfShared *S, InfWarp *W, const uint8_t
 // Occupancy: a member is one long serial chain (a launch of 2048 members takes 4.9 ms, one of 4096 members 5.5 ms), so
 // throughput is members in flight per SM: the tables are sized (9-bit literal/length look-up, 20 KB per block) and the
 // registers capped (40) for 11 blocks = 44 members per SM; at 6500 members per launch 55.6 GB/s of text (32 per SM: 48.3).
-template <int MINB>
-__global__ void __launch_bounds__(INFW_WARPS * 32, MINB)
+__global__ void __launch_bounds__(INFW_WARPS * 32, 11)
 k_inflate_warp(const __grid_constant__ InflateArgs a)
 {
     __shared__ InfShared S;
@@ -1413,39 +1177,18 @@ int launch_inflate(const uint8_t *d_z, const vfb_member *d_members, uint32_t n_m
                    uint32_t *d_first_bad, cudaStream_t st)
 {
     if (n_members == 0) return VFB_OK;
-    static int lanes = 0;
-    if (!lanes) {
-        const char *e = getenv("VFB_INFLATE_LANES");
-        lanes = e ? atoi(e) : 1;
-        if (lanes < 1 || lanes > 32) lanes = 1;
+    const InflateArgs a{d_z, d_members, n_members, d_out, d_first_bad};
+    static int bps = 0, sms = 0;
+    if (!bps) {
+        int dev = 0;
+        VFB_CUDA(cudaGetDevice(&dev));
+        VFB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+        VFB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_inflate_warp, INFW_WARPS * 32, 0));
+        if (bps < 1) bps = 1;
     }
-    InflateArgs a{d_z, d_members, n_members, d_out, d_first_bad, (uint32_t)lanes};
-    static int v1 = -1;
-    if (v1 < 0) v1 = getenv("VFB_INFLATE_V1") ? 1 : 0;
-    if (!v1) {
-        // blocks per SM the kernel is compiled for: 11 (40 registers) by default; VFB_INFLATE_BPS=9 / 10 for comparison
-        static int bps = 0, sms = 0, minb = 11;
-        if (!bps) {
-            int dev = 0;
-            VFB_CUDA(cudaGetDevice(&dev));
-            VFB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-            if (const char *e = getenv("VFB_INFLATE_BPS")) { const int v = atoi(e); if (v == 9 || v == 10) minb = v; }
-            if (minb == 9) VFB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_inflate_warp<9>, INFW_WARPS * 32, 0));
-            else if (minb == 10) VFB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_inflate_warp<10>, INFW_WARPS * 32, 0));
-            else VFB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_inflate_warp<11>, INFW_WARPS * 32, 0));
-            if (bps < 1) bps = 1;
-        }
-        uint32_t blocks = (n_members + INFW_WARPS - 1) / INFW_WARPS;
-        if (blocks > (uint32_t)(sms * bps)) blocks = (uint32_t)(sms * bps);
-        if (minb == 9) k_inflate_warp<9><<<blocks, INFW_WARPS * 32, 0, st>>>(a);
-        else if (minb == 10) k_inflate_warp<10><<<blocks, INFW_WARPS * 32, 0, st>>>(a);
-        else k_inflate_warp<11><<<blocks, INFW_WARPS * 32, 0, st>>>(a);
-        ++g_launches;
-        VFB_CUDA(cudaGetLastError());
-        return VFB_OK;
-    }
-    const uint32_t warps = (n_members + lanes - 1) / lanes;
-    k_inflate_members<<<(warps + INF_THREADS / 32 - 1) / (INF_THREADS / 32), INF_THREADS, 0, st>>>(a);
+    uint32_t blocks = (n_members + INFW_WARPS - 1) / INFW_WARPS;
+    if (blocks > (uint32_t)(sms * bps)) blocks = (uint32_t)(sms * bps);
+    k_inflate_warp<<<blocks, INFW_WARPS * 32, 0, st>>>(a);
     ++g_launches;
     VFB_CUDA(cudaGetLastError());
     return VFB_OK;

@@ -21,8 +21,6 @@
 //  * k1_scan_general (any adapter length, including 0 and > 64): one warp per read, byte-wise, ballot.
 #include "vfb_internal.cuh"
 
-#include <stdlib.h>
-
 namespace vfb {
 
 #define SCAN_THREADS 256
@@ -611,30 +609,30 @@ uint32_t vfb_tile_bytes_for(uint64_t text_bytes, uint32_t n_reads)
     uint64_t t = 32 * stride + stride + 64;
     t = (t + 127) & ~127ull;
     if (t < 2048) t = 2048;
-    if (t > 96 * 1024) t = 96 * 1024;
+    if (t > VFB_TILE_BYTES_MAX) t = VFB_TILE_BYTES_MAX;
     return (uint32_t)t;
 }
+
+// Shared memory of a tile block of `w` warps: their tiles (dynamic), the tables, worklist stages and barriers, and a
+// reserve.
+static constexpr size_t scan_tile_block_smem(size_t tile, int w)
+{
+    return (size_t)w * (tile + TILE_SLACK) + sizeof(TileTables) + TILE_WARPS_MAX * (2 * WL_BUF * 4 + 8) + 1024;
+}
+static_assert(scan_tile_block_smem(VFB_TILE_BYTES_MAX, 1) <= VFB_SMEM_BLOCK_MAX, "a block of one warp fits any tile");
 
 template <bool STRIDE16>
 static int launch_scan_tile(const ScanArgs &a, int sm_count, cudaStream_t st)
 {
     const uint32_t tile = vfb_tile_bytes_for(a.job.text_bytes, a.job.n_reads);
-    const size_t smem_cap = 227 * 1024;
-    int warps = TILE_WARPS_MAX;
-    auto smem_for = [&](int w) {
-        return (size_t)w * (tile + TILE_SLACK);
-    };
     // as many warps per SM as the tiles allow, in blocks of 8 / 4 / 2 / 1 warps
-    int best_w = 1, best_total = 0;
+    int warps = 1, best_total = 0;
     for (int w = TILE_WARPS_MAX; w >= 1; w >>= 1) {
-        const size_t per_block = smem_for(w) + sizeof(TileTables) + TILE_WARPS_MAX * (2 * WL_BUF * 4 + 8) + 1024;
-        int bps = (int)(smem_cap / per_block);
+        int bps = (int)(VFB_SMEM_BLOCK_MAX / scan_tile_block_smem(tile, w));
         if (bps * w > 32) bps = 32 / w;            // 1024 resident threads are plenty
-        if (bps * w > best_total) { best_total = bps * w; best_w = w; }
+        if (bps * w > best_total) { best_total = bps * w; warps = w; }
     }
-    warps = best_w;
-    const size_t smem = smem_for(warps);
-    if (best_total == 0) return -1;
+    const size_t smem = (size_t)warps * (tile + TILE_SLACK);
     const int bps = best_total / warps;
     VFB_CUDA(cudaFuncSetAttribute(k1_scan_tile<STRIDE16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const uint32_t units = (a.job.n_reads + 31) / 32;
@@ -732,24 +730,19 @@ int launch_scan(const ScanJob &job, const AdapterBytes &prefix, const AdapterByt
     uint32_t blocks = (units + SCAN_WARPS - 1) / SCAN_WARPS;
     const uint32_t cap = (uint32_t)sm_count * 8u;
     if (blocks > cap) blocks = cap;
-#define VFB_SCAN_LAUNCH(S, K8)                                                              \
+#define VFB_SCAN_LAUNCH(S)                                                                  \
     do {                                                                                    \
-        if (a.multi) k1_scan_fast<S, true, K8><<<blocks, SCAN_THREADS, 0, st>>>(a);         \
-        else k1_scan_fast<S, false, K8><<<blocks, SCAN_THREADS, 0, st>>>(a);                \
+        if (a.multi) k1_scan_fast<S, true, false><<<blocks, SCAN_THREADS, 0, st>>>(a);      \
+        else k1_scan_fast<S, false, false><<<blocks, SCAN_THREADS, 0, st>>>(a);             \
     } while (0)
-    static const bool old_scan = getenv("VFB_SCAN_TILE") && atoi(getenv("VFB_SCAN_TILE")) == 0;
-    bool tiled = false;
-    if (fast && key8 && !a.multi && !old_scan && job.text_bytes) {
+    if (!fast) k1_scan_general<<<blocks, SCAN_THREADS, 0, st>>>(a);
+    else if (key8 && !a.multi) {
         const int rc = stride_words == 4 ? launch_scan_tile<true>(a, sm_count, st) : launch_scan_tile<false>(a, sm_count, st);
-        if (rc > 0) return rc;
-        tiled = rc == VFB_OK;
-    }
-    if (tiled) {}
-    else if (!fast) k1_scan_general<<<blocks, SCAN_THREADS, 0, st>>>(a);
-    else if (key8 && stride_words == 4) VFB_SCAN_LAUNCH(4, true);
-    else if (key8) VFB_SCAN_LAUNCH(2, true);
-    else if (stride_words == 2) VFB_SCAN_LAUNCH(2, false);
-    else VFB_SCAN_LAUNCH(1, false);
+        if (rc) return rc;
+    } else if (key8 && stride_words == 4) k1_scan_fast<4, true, true><<<blocks, SCAN_THREADS, 0, st>>>(a);
+    else if (key8) k1_scan_fast<2, true, true><<<blocks, SCAN_THREADS, 0, st>>>(a);
+    else if (stride_words == 2) VFB_SCAN_LAUNCH(2);
+    else VFB_SCAN_LAUNCH(1);
 #undef VFB_SCAN_LAUNCH
     ++g_launches;
     VFB_CUDA(cudaGetLastError());

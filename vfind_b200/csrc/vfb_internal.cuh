@@ -132,7 +132,11 @@ struct ScanJob {
     int compute_all;              // 1: list every suffix miss (what the reference computes)
     int force_general;            // tests: use the byte-wise kernel
 };
-// Shared-memory tile for 32 reads that sit text_bytes / n_reads apart on average (scan and key kernels).
+// Shared-memory tile for 32 reads that sit text_bytes / n_reads apart on average (scan and key kernels), at most
+// VFB_TILE_BYTES_MAX.  The tile launchers static_assert that a block of one warp at that size fits
+// VFB_SMEM_BLOCK_MAX, the shared memory an sm_100 block may have, so they always launch.
+#define VFB_TILE_BYTES_MAX (96u * 1024u)
+#define VFB_SMEM_BLOCK_MAX (227u * 1024u)
 uint32_t vfb_tile_bytes_for(uint64_t text_bytes, uint32_t n_reads);
 int launch_scan(const ScanJob &job, const AdapterBytes &prefix, const AdapterBytes &suffix,
                 int sm_count, cudaStream_t st);
