@@ -338,6 +338,25 @@ int vfb_debug_translate12(const uint8_t *bases12, uint8_t *aa4, int *canonical);
 int vfb_debug_window_plan(int32_t match_score, int32_t mismatch_score, int32_t gap_open_penalty, int32_t gap_extend_penalty,
                           uint32_t adapter_len, double accept_alignment, int32_t *accept_bound, int32_t *max_edits);
 
+/* The packed DP word vfb_create picks for one adapter (csrc/kernels_dp.cu, DpLayout), so that a model of the DP
+ * kernels can run on the library's own constants. */
+typedef struct vfb_dp_layout_info {
+    int32_t packed;           /* 1 = a packed kernel runs (the fields below are set), 0 = the unpacked one */
+    int32_t max_edits;        /* K of the windowed path, -1 = the full-matrix kernel runs */
+    int32_t accept_bound;     /* T: accept iff score >= T */
+    uint32_t lcap;            /* longest read the packed kernels take; longer ones go to the unpacked kernel */
+    int32_t S0, LB, XB;       /* score << S0 | q << (LB+XB) | x << LB | len */
+    int32_t c_eopen, c_eext, c_fopen, c_fext;
+    int32_t hmask, lowmask, lenmask;
+    int32_t neg_e, neg_f;
+    int32_t w_match, w_mismatch, w_wild;
+} vfb_dp_layout_info;
+
+/* What vfb_create decides for one adapter of a context without diagnostics (or with dp_mode 2) when dp_mode != 1,
+ * and the full-matrix choice when dp_mode == 1.  Host code only, no GPU needed. */
+int vfb_debug_dp_layout(int32_t match_score, int32_t mismatch_score, int32_t gap_open_penalty, int32_t gap_extend_penalty,
+                        uint32_t adapter_len, double accept_alignment, int32_t dp_mode, vfb_dp_layout_info *out);
+
 /* Pinned host memory for callers without their own allocator. */
 int vfb_host_alloc(void **p, uint64_t bytes);
 int vfb_host_free(void *p);

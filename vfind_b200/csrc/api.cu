@@ -509,6 +509,19 @@ static int accept_bound(double thr, int32_t match, size_t len)
     return (int)f + 1;
 }
 
+// The packed DP of one adapter: the windowed path (K >= 0) when it is wanted, the filter applies and the window's
+// wider score range fits the packed word; else the full-matrix kernel (K = -1) when its range fits; else false (the
+// unpacked kernel runs).  The full kernel that takes the windowed path's fallback reads runs on the same layout.
+static bool plan_packed_dp(const DpScoring &sc, uint32_t A, int min_accept, bool want_window, DpLayout *lay,
+                           uint32_t *lcap, int *K)
+{
+    *K = want_window ? dpw_max_edits(sc, A, min_accept) : -1;
+    if (*K >= 0 && !make_dp_layout(sc, A, true, lay)) *K = -1;
+    if (*K < 0 && !make_dp_layout(sc, A, false, lay)) return false;
+    *lcap = dp_lcap(*lay, A, sc.extend);
+    return true;
+}
+
 // ------------------------------------------------------------------------------------ ABI
 extern "C" {
 
@@ -622,18 +635,16 @@ int vfb_create(const vfb_params *p, vfb_ctx **out)
 
     // DP setup: packed layout when the scores fit, else the fallback kernel
     const bool force_generic = p->force_generic_dp != 0;
-    auto setup_dp = [&](const std::string &ad, bool enabled, bool *packed, DpLayout *lay, uint32_t *lcap,
-                        DevBuf *codes) -> int {
+    const bool want_window = p->dp_mode != 1 && (!p->diagnostics || p->dp_mode == 2);
+    auto setup_dp = [&](const std::string &ad, bool enabled, int min_accept, bool *packed, DpLayout *lay, uint32_t *lcap,
+                        int *win_k, DevBuf *codes) -> int {
         *packed = false;
         if (!enabled) return VFB_OK;
         if (ad.size() > VFB_MAX_ADAPTER) { set_error("adapter too long for alignment"); return VFB_ERR_ARG; }
         long long worst = (long long)(std::abs((long long)c->sc.match) + std::abs((long long)c->sc.mismatch) +
                                       std::abs((long long)c->sc.open) + std::abs((long long)c->sc.extend));
         if (worst > (1 << 20)) { set_error("alignment scores beyond +-2^20 are not supported"); return VFB_ERR_ARG; }
-        if (!force_generic && make_dp_layout(c->sc, (uint32_t)ad.size(), 0, lay)) {
-            *packed = true;
-            *lcap = dp_lcap(*lay, (uint32_t)ad.size(), c->sc.extend);
-        }
+        if (!force_generic) *packed = plan_packed_dp(c->sc, (uint32_t)ad.size(), min_accept, want_window, lay, lcap, win_k);
         std::vector<uint8_t> code(ad.size());
         for (size_t i = 0; i < ad.size(); ++i) code[i] = (uint8_t)dp_code((uint8_t)ad[i]);
         int r = codes->ensure(code.size());
@@ -641,11 +652,12 @@ int vfb_create(const vfb_params *p, vfb_ctx **out)
         VFB_CUDA(cudaMemcpy(codes->p, code.data(), code.size(), cudaMemcpyHostToDevice));
         return VFB_OK;
     };
-    if ((rc = setup_dp(c->prefix, c->align_pre, &c->packed_pre, &c->lay_pre, &c->lcap_pre, &c->d_code_pre))) return fail(rc);
-    if ((rc = setup_dp(c->suffix, c->align_suf, &c->packed_suf, &c->lay_suf, &c->lcap_suf, &c->d_code_suf))) return fail(rc);
-    if (c->packed_pre) c->win_k_pre = dpw_max_edits(c->sc, (uint32_t)c->prefix.size(), c->min_accept_pre);
-    if (c->packed_suf) c->win_k_suf = dpw_max_edits(c->sc, (uint32_t)c->suffix.size(), c->min_accept_suf);
-    if (p->dp_mode == 1) c->win_k_pre = c->win_k_suf = -1;
+    if ((rc = setup_dp(c->prefix, c->align_pre, c->min_accept_pre, &c->packed_pre, &c->lay_pre, &c->lcap_pre, &c->win_k_pre,
+                       &c->d_code_pre)))
+        return fail(rc);
+    if ((rc = setup_dp(c->suffix, c->align_suf, c->min_accept_suf, &c->packed_suf, &c->lay_suf, &c->lcap_suf, &c->win_k_suf,
+                       &c->d_code_suf)))
+        return fail(rc);
     if (c->align_pre || c->align_suf) {
         c->generic_threads = dp_generic_threads(c->sm_count);
         size_t amax = c->prefix.size() > c->suffix.size() ? c->prefix.size() : c->suffix.size();
@@ -661,7 +673,7 @@ int vfb_create(const vfb_params *p, vfb_ctx **out)
     if ((rc = table_init(c))) return fail(rc);
     trace("vfb_create: table ready");
     c->stats.dp_kernel_kind = (c->packed_pre || c->packed_suf) ? 1 : ((c->align_pre || c->align_suf) ? 2 : 0);
-    if ((c->win_k_pre >= 0 || c->win_k_suf >= 0) && (!p->diagnostics || p->dp_mode == 2)) c->stats.dp_kernel_kind = 3;
+    if (c->win_k_pre >= 0 || c->win_k_suf >= 0) c->stats.dp_kernel_kind = 3;
     *out = c;
     return VFB_OK;
 }
@@ -1944,6 +1956,28 @@ int vfb_debug_window_plan(int32_t match_score, int32_t mismatch_score, int32_t g
     const DpScoring sc{match_score, mismatch_score, gap_open_penalty, gap_extend_penalty};
     *accept_bound_out = t;
     *max_edits_out = dpw_max_edits(sc, adapter_len, t);
+    return VFB_OK;
+}
+
+int vfb_debug_dp_layout(int32_t match_score, int32_t mismatch_score, int32_t gap_open_penalty, int32_t gap_extend_penalty,
+                        uint32_t adapter_len, double accept_alignment, int32_t dp_mode, vfb_dp_layout_info *out)
+{
+    if (!out || adapter_len == 0) { set_error("bad argument"); return VFB_ERR_ARG; }
+    memset(out, 0, sizeof *out);
+    const DpScoring sc{match_score, mismatch_score, gap_open_penalty, gap_extend_penalty};
+    out->accept_bound = accept_bound(accept_alignment, match_score, adapter_len);
+    DpLayout l;
+    uint32_t lcap = 0;
+    int K = -1;
+    out->packed = plan_packed_dp(sc, adapter_len, out->accept_bound, dp_mode != 1, &l, &lcap, &K) ? 1 : 0;
+    out->max_edits = out->packed ? K : -1;
+    if (!out->packed) return VFB_OK;
+    out->S0 = l.S0; out->LB = l.LB; out->XB = l.XB;
+    out->c_eopen = l.c_eopen; out->c_eext = l.c_eext; out->c_fopen = l.c_fopen; out->c_fext = l.c_fext;
+    out->hmask = l.hmask; out->lowmask = l.lowmask; out->lenmask = l.lenmask;
+    out->neg_e = l.neg_e; out->neg_f = l.neg_f;
+    out->w_match = l.w_match; out->w_mismatch = l.w_mismatch; out->w_wild = l.w_wild;
+    out->lcap = lcap;
     return VFB_OK;
 }
 

@@ -23,7 +23,19 @@ static inline int bits_for(uint64_t v)   // smallest b with 2^b > v
     return b;
 }
 
-bool make_dp_layout(const DpScoring &s, uint32_t A, uint32_t /*max_read_len*/, DpLayout *out)
+// The signed score field must hold every candidate any cell forms in rows 1..A, or an add wraps int32 and a low
+// candidate turns into a high score.  Upper end: H <= smax = A*wmax.  Lower end (wmin <= 0 the cheapest step):
+//   Full matrix: every H >= A*wmin (its diagonal runs back to row 0 or column 0, both 0), so H - o > neg; E and F
+//   are >= neg (their border), and the lowest candidate is an extension of that border: >= neg - e (the bound
+//   below takes neg - max(o, e)).
+//   Window from column j0 > 1 (kernels_dpw.cu): H = neg in every row of column j0 - 1.  A cell (i, j) with
+//   j - j0 + 1 < i has a diagonal that runs back into that border, so only H >= neg + (i-1)*wmin holds there; E and
+//   F are >= that H - o, and an extension of them loses e more:  lowest >= neg + (A-1)*wmin - o - e.
+//   Cells with j - j0 + 1 >= i reach row 0 on their diagonal and keep the full matrix's H >= i*wmin.
+// x (an E run of extensions, which beats an opening at equal score) needs no more room in a window: a run whose
+// last step is compared against an H past the triangle above (H >= i*wmin) loses at most smax - smin, as in the
+// full matrix, and a run that ends inside the triangle has at most i <= A columns.
+bool make_dp_layout(const DpScoring &s, uint32_t A, bool windowed, DpLayout *out)
 {
     if (A < 1 || A > VFB_MAX_PACKED_ADAPTER) return false;
     if (s.open < 0 || s.extend < 0) return false;
@@ -34,7 +46,8 @@ bool make_dp_layout(const DpScoring &s, uint32_t A, uint32_t /*max_read_len*/, D
     if (s.mismatch > wmax) wmax = s.mismatch;
     long long smax = (long long)A * wmax, smin = (long long)A * wmin;
     long long neg = smin - s.open - 1;           // border "-inf": below every real candidate
-    long long lowest = neg - (s.open > s.extend ? s.open : s.extend);   // the lowest value ever formed
+    long long lowest = neg - (s.open > s.extend ? s.open : s.extend);   // the lowest value ever formed (see above)
+    if (windowed) lowest = neg + ((long long)A - 1) * wmin - s.open - s.extend;
     long long need = smax + 1 > -lowest ? smax + 1 : -lowest;
     if (need > (1 << 20)) return false;
     int SB = bits_for((uint64_t)need) + 1;       // signed field holding [-need, need]

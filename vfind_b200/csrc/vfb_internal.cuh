@@ -72,8 +72,9 @@ struct DpScoring {
     int match, mismatch, open, extend;
 };
 
-// Returns false if the parameters do not fit the packed layout (then the fallback runs).
-bool make_dp_layout(const DpScoring &s, uint32_t adapter_len, uint32_t max_read_len, DpLayout *out);
+// Returns false if the parameters do not fit the packed layout (then the fallback runs).  `windowed`: sized for
+// the windowed DP too, whose windows start from a -inf border and so reach lower scores than the full matrix.
+bool make_dp_layout(const DpScoring &s, uint32_t adapter_len, bool windowed, DpLayout *out);
 
 struct DpJob {
     const uint8_t *text;
