@@ -74,6 +74,9 @@ typedef struct vfb_params {
                                          in diagnostics mode (scores of rejected alignments are then
                                          lower bounds or absent)                              */
     int32_t debug_win_cap;            /* tests only: > 0 caps the window list of the windowed DP   */
+    int32_t both_strands;             /* 1 = a read without a region (start, end located, start < end <= len) is
+                                         searched once more as its reverse complement; a region found there is
+                                         counted in the same table (at most one strand counts per read)       */
 } vfb_params;
 
 /* One read inside a text buffer: text[off .. off+len). */
@@ -145,6 +148,8 @@ typedef struct vfb_stats {
     double ms_dp_filter, ms_dp_window;   /* parts of ms_dp: k2_filter and k2_dp_window (profiling only) */
     uint64_t fused_batches;     /* batches whose key kernel probed the count table itself (k34_keys_count)   */
     uint64_t fused_hits;        /* counted reads whose key never left the key kernel (row already in the table) */
+    uint64_t reverse_reads;     /* both_strands: reads searched as their reverse complement                  */
+    uint64_t reverse_counted;   /* both_strands: reads counted from the reverse strand                       */
 } vfb_stats;
 
 typedef struct vfb_ctx vfb_ctx;
@@ -240,6 +245,10 @@ int vfb_get_stats(vfb_ctx *ctx, vfb_stats *out);
 /* Diagnostics of the most recent batch (requires params.diagnostics = 1 and that the
  * last submit was a single batch).  Parity tests compare these with the oracle. */
 int vfb_get_diag(vfb_ctx *ctx, vfb_read_diag *out, uint64_t n_reads);
+/* both_strands: the diagnostics of the reverse-complement pass over the same batch, in the batch's read order.  Reads
+ * that were not retried (they have a forward region, or are empty) carry the "absent" markers: positions and
+ * boundaries -1, scores INT32_MIN, lengths -1.  Positions refer to the reverse complement of the read. */
+int vfb_get_diag_reverse(vfb_ctx *ctx, vfb_read_diag *out, uint64_t n_reads);
 
 /* ---- multi-GPU (no reference equivalent; SURVEY §8(e)) ----
  * Reads shard across devices with no data-path collective; the only exchange is the final merge of the per-device
@@ -330,6 +339,10 @@ int vfb_debug_gpu_inflate(const uint8_t *z, uint64_t z_bytes, const uint32_t *me
  * the code the kernel uses (csrc/translate_fast.h) on twelve bases; aa receives four amino acids, *canonical is 1
  * when all twelve bytes are A/C/G/T/U of either case (only then does the kernel take this path). No GPU needed. */
 int vfb_debug_translate12(const uint8_t *bases12, uint8_t *aa4, int *canonical);
+
+/* Test hook for both_strands: the reverse complement the device gather writes (csrc/kernels_strand.cu, host build of
+ * the same base map): out[i] = complement(in[n-1-i]), A<->T, C<->G, a<->t, c<->g, U->A, u->a, other bytes unchanged. */
+int vfb_debug_revcomp(const uint8_t *in, uint64_t n, uint8_t *out);
 
 /* Test hook for the windowed alignment path (what vfb_create decides for one adapter; no GPU needed): *accept_bound
  * receives the integer T with score >= T <=> score as f64 > accept_alignment * match_score * adapter_len

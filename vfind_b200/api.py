@@ -42,7 +42,7 @@ class Params(C.Structure):
                 ("table_capacity_hint", C.c_uint64),
                 ("debug_hash_bits", C.c_int32), ("force_generic_dp", C.c_int32),
                 ("dp_compute_all", C.c_int32), ("force_general_scan", C.c_int32),
-                ("dp_mode", C.c_int32), ("debug_win_cap", C.c_int32)]
+                ("dp_mode", C.c_int32), ("debug_win_cap", C.c_int32), ("both_strands", C.c_int32)]
 
 
 class Table(C.Structure):
@@ -78,7 +78,8 @@ class Stats(C.Structure):
                 ("dp_kernel_launches", C.c_uint64), ("dp_kernel_kind", C.c_int32),
                 ("reserved", C.c_int32), ("dp_cells_computed", C.c_uint64), ("dp_windows", C.c_uint64),
                 ("ms_dp_filter", C.c_double), ("ms_dp_window", C.c_double),
-                ("fused_batches", C.c_uint64), ("fused_hits", C.c_uint64)]
+                ("fused_batches", C.c_uint64), ("fused_hits", C.c_uint64),
+                ("reverse_reads", C.c_uint64), ("reverse_counted", C.c_uint64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
@@ -126,6 +127,8 @@ def load_library():
     L.vfb_table_free.restype = None
     L.vfb_get_stats.argtypes = [vp, C.POINTER(Stats)]
     L.vfb_get_diag.argtypes = [vp, vp, u64]
+    L.vfb_get_diag_reverse.argtypes = [vp, vp, u64]
+    L.vfb_debug_revcomp.argtypes = [C.c_char_p, u64, vp]
     L.vfb_table_partition_sizes.argtypes = [vp, u32, C.POINTER(u64)]
     L.vfb_table_partition_fill.argtypes = [vp, u32, vp, C.POINTER(u64)]
     L.vfb_table_clear.argtypes = [vp]
@@ -202,7 +205,8 @@ def _as_bytes(s, what):
 def _make_params(L, adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                  accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
                  show_progress, device, diagnostics, batch_reads, batch_bytes, table_capacity_hint,
-                 debug_hash_bits, force_generic_dp, dp_compute_all, force_general_scan, dp_mode, debug_win_cap):
+                 debug_hash_bits, force_generic_dp, dp_compute_all, force_general_scan, dp_mode, debug_win_cap,
+                 both_strands=False):
     p = Params()
     L.vfb_default_params(C.byref(p))
     pre = _as_bytes(adapters[0], "adapters[0]")
@@ -226,6 +230,7 @@ def _make_params(L, adapters, match_score, mismatch_score, gap_open_penalty, gap
     p.force_general_scan = 1 if force_general_scan else 0
     p.dp_mode = int(dp_mode)
     p.debug_win_cap = int(debug_win_cap)
+    p.both_strands = 1 if both_strands else 0
     return p, pre, suf          # the byte strings must outlive the call that reads p
 
 
@@ -237,7 +242,9 @@ class Context:
                  n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
                  device=None, diagnostics=False, batch_reads=0, batch_bytes=0,
                  table_capacity_hint=0, debug_hash_bits=0, force_generic_dp=False,
-                 dp_compute_all=False, force_general_scan=False, dp_mode=0, debug_win_cap=0):
+                 dp_compute_all=False, force_general_scan=False, dp_mode=0, debug_win_cap=0, both_strands=False):
+        """both_strands: a read without a region is searched once more as its reverse complement, on the device, and
+        a region found there is counted in the same table (a read counts on at most one strand)."""
         L = load_library()
         self._lib = L
         self._h = C.c_void_p()
@@ -247,7 +254,7 @@ class Context:
                                                n_threads, queue_len, skip_translation, show_progress, device,
                                                diagnostics, batch_reads, batch_bytes, table_capacity_hint,
                                                debug_hash_bits, force_generic_dp, dp_compute_all, force_general_scan,
-                                               dp_mode, debug_win_cap)
+                                               dp_mode, debug_win_cap, both_strands)
         _check(L.vfb_create(C.byref(p), C.byref(self._h)))
 
     @classmethod
@@ -341,6 +348,13 @@ class Context:
         _check(self._lib.vfb_get_diag(self._h, out.ctypes.data, n))
         return out
 
+    def diag_reverse(self, n):
+        """both_strands: diagnostics of the reverse-complement pass over the last batch, in read order; rows of reads
+        that were not retried hold the absent markers (-1, INT32_MIN for scores)."""
+        out = np.zeros(n, dtype=DIAG_DTYPE)
+        _check(self._lib.vfb_get_diag_reverse(self._h, out.ctypes.data, n))
+        return out
+
     # -- results
     def finish_arrays(self, copy=True):
         """(offsets uint64[rows+1], data uint8[key_bytes], counts uint64[rows]) on the host.
@@ -409,7 +423,8 @@ class MultiContext:
     def __init__(self, adapters, match_score=3, mismatch_score=-2, gap_open_penalty=5,
                  gap_extend_penalty=2, accept_prefix_alignment=0.75, accept_suffix_alignment=0.75,
                  n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
-                 devices=None, batch_reads=0, batch_bytes=0, table_capacity_hint=0, debug_hash_bits=0, dp_mode=0):
+                 devices=None, batch_reads=0, batch_bytes=0, table_capacity_hint=0, debug_hash_bits=0, dp_mode=0,
+                 both_strands=False):
         L = load_library()
         self._lib = L
         self._h = C.c_void_p()
@@ -417,7 +432,7 @@ class MultiContext:
                                                gap_extend_penalty, accept_prefix_alignment, accept_suffix_alignment,
                                                n_threads, queue_len, skip_translation, show_progress, None, False,
                                                batch_reads, batch_bytes, table_capacity_hint, debug_hash_bits,
-                                               False, False, False, dp_mode, 0)
+                                               False, False, False, dp_mode, 0, both_strands)
         if devices is None:
             _check(L.vfb_multi_create(C.byref(p), None, 0, C.byref(self._h)))
         else:
@@ -570,7 +585,8 @@ def _bool_arg(v, name):
 def find_variants(fq_path, adapters, match_score=3, mismatch_score=-2, gap_open_penalty=5,
                   gap_extend_penalty=2, accept_prefix_alignment=0.75, accept_suffix_alignment=0.75,
                   n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
-                  device=None, devices=None, batch_reads=0, table_capacity_hint=0, progress=None, allow_text=False):
+                  device=None, devices=None, batch_reads=0, table_capacity_hint=0, progress=None, allow_text=False,
+                  both_strands=False):
     """Find variable regions flanked by adapters in a gzipped FASTQ dataset.
 
     Drop-in for `vfind.find_variants` (/root/reference/src/lib.rs:168-232): same positional
@@ -585,7 +601,9 @@ def find_variants(fq_path, adapters, match_score=3, mismatch_score=-2, gap_open_
     NVLink inside the library; default: every visible GPU that gets at least 64 MB of the compressed input —
     VFB_DEVICES=n caps it), batch_reads, table_capacity_hint,
     progress (callable(records, bytes_done, bytes_total), called about ten times per second),
-    allow_text (read a file without the gzip magic as uncompressed FASTQ; the reference panics on it).
+    allow_text (read a file without the gzip magic as uncompressed FASTQ; the reference panics on it),
+    both_strands (a read in which no region is found is searched once more as its reverse complement, on the GPU, and
+    counted in the same table: for libraries sequenced from both ends; a read counts on at most one strand).
     With show_progress (the default) and a terminal on stderr a one-line progress display is shown
     and cleared at the end, like the reference's spinner (src/lib.rs:265-269, :310).
     """
@@ -596,13 +614,15 @@ def find_variants(fq_path, adapters, match_score=3, mismatch_score=-2, gap_open_
                         % type(fq_path).__name__)
     return _find_variants([fq_path], adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                           accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
-                          show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text)
+                          show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text,
+                          both_strands)
 
 
 def find_variants_multi(fq_paths, adapters, match_score=3, mismatch_score=-2, gap_open_penalty=5,
                         gap_extend_penalty=2, accept_prefix_alignment=0.75, accept_suffix_alignment=0.75,
                         n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
-                        device=None, devices=None, batch_reads=0, table_capacity_hint=0, progress=None, allow_text=False):
+                        device=None, devices=None, batch_reads=0, table_capacity_hint=0, progress=None, allow_text=False,
+                        both_strands=False):
     """find_variants over several FASTQ files (lanes, split runs) counted into ONE table, on one context
     (SURVEY §8(f) next-4).  Same arguments as find_variants; fq_paths is a non-empty sequence of paths."""
     if isinstance(fq_paths, (str, bytes, os.PathLike)) or not hasattr(fq_paths, "__iter__"):
@@ -612,12 +632,13 @@ def find_variants_multi(fq_paths, adapters, match_score=3, mismatch_score=-2, ga
         raise TypeError("argument 'fq_paths': expected a non-empty sequence of str / os.PathLike")
     return _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                           accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
-                          show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text)
+                          show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text,
+                          both_strands)
 
 
 def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                    accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
-                   show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text):
+                   show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text, both_strands):
     if not isinstance(adapters, (tuple, list)):
         raise TypeError("argument 'adapters': '%s' object cannot be converted to 'PyTuple'"
                         % type(adapters).__name__)
@@ -639,6 +660,7 @@ def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalt
     queue_len = _int_arg(queue_len, "queue_len", 0, 2 ** 64 - 1)
     skip_translation = _bool_arg(skip_translation, "skip_translation")
     show_progress = _bool_arg(show_progress, "show_progress")
+    both_strands = _bool_arg(both_strands, "both_strands")
 
     # The reference opens the file before validating thresholds (src/lib.rs:233 vs :239).
     for p in paths:
@@ -657,12 +679,12 @@ def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalt
         ctx = Context(adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                       accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len,
                       skip_translation, show_progress, device=devs[0], batch_reads=batch_reads,
-                      table_capacity_hint=table_capacity_hint)
+                      table_capacity_hint=table_capacity_hint, both_strands=both_strands)
     else:
         ctx = MultiContext(adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                            accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len,
                            skip_translation, show_progress, devices=devs, batch_reads=batch_reads,
-                           table_capacity_hint=table_capacity_hint)
+                           table_capacity_hint=table_capacity_hint, both_strands=both_strands)
     with ctx:
         shown = show_progress and progress is None and sys.stderr.isatty()
         if progress is not None:
@@ -716,7 +738,7 @@ def _pick_devices(device, devices, paths):
 
 def read_diagnostics(reads, adapters, match_score=3, mismatch_score=-2, gap_open_penalty=5, gap_extend_penalty=2,
                      accept_prefix_alignment=0.75, accept_suffix_alignment=0.75, skip_translation=False, *,
-                     device=None):
+                     device=None, both_strands=False):
     """What find_variants decides for each read, as a pyarrow.Table with one row per read (SURVEY §8(f) next-3):
 
     exact_prefix / exact_suffix  leftmost exact adapter position, null when absent      (src/lib.rs:148)
@@ -725,6 +747,14 @@ def read_diagnostics(reads, adapters, match_score=3, mismatch_score=-2, gap_open
     accept_prefix / accept_suffix  the adapter was located (exactly or by an accepted alignment)
     start / end                  region boundaries, null when not located               (src/lib.rs:278-286)
     region                       the variable region (null unless both located and start < end, src/lib.rs:288)
+
+    With both_strands the columns above describe the forward pass, and these follow:
+
+    strand                       +1: the read has a region as given, -1: its reverse complement has one (the read was
+                                 retried), null: neither
+    rev_exact_prefix ... rev_end the columns above for the reverse complement of the read; null where no reverse pass
+                                 ran (the read has a forward region, or is empty)
+    region                       the bases that were counted: reverse-complemented for strand -1
 
     `reads` is a sequence of str / bytes.  Runs the full DP (exact scores also for rejected alignments)."""
     import pyarrow as pa
@@ -738,29 +768,56 @@ def read_diagnostics(reads, adapters, match_score=3, mismatch_score=-2, gap_open
     if n:
         spans["off"][1:] = np.cumsum(length[:-1])
     text = np.frombuffer(b"".join(seqs), dtype=np.uint8)
-    if n == 0:
-        d = np.zeros(0, dtype=DIAG_DTYPE)
-    else:
+    d = rd = np.zeros(0, dtype=DIAG_DTYPE)
+    if n:
         ad = tuple(a if isinstance(a, bytes) else a.encode() for a in adapters)
         with Context(ad, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty, accept_prefix_alignment,
                      accept_suffix_alignment, skip_translation=skip_translation, device=device, diagnostics=True,
-                     batch_reads=max(n, 1)) as ctx:
+                     batch_reads=max(n, 1), both_strands=both_strands) as ctx:
             ctx.submit_host(text, spans)
             d = ctx.diag(n)
-    cols = {}
-    for f in ("exact_prefix", "exact_suffix"):
-        cols[f] = pa.array(d[f], mask=d[f] < 0, type=pa.int32())
-    for side in ("prefix", "suffix"):
-        ran = d["len_" + side] >= 0
-        cols["score_" + side] = pa.array(d["score_" + side], mask=~ran, type=pa.int32())
-        cols["len_" + side] = pa.array(d["len_" + side], mask=~ran, type=pa.int32())
-    cols["accept_prefix"] = pa.array(d["start"] >= 0)
-    cols["accept_suffix"] = pa.array(d["end"] >= 0)
-    cols["start"] = pa.array(d["start"], mask=d["start"] < 0, type=pa.int32())
-    cols["end"] = pa.array(d["end"], mask=d["end"] < 0, type=pa.int32())
-    ok = (d["start"] >= 0) & (d["end"] >= 0) & (d["start"] < d["end"])
-    cols["region"] = pa.array([seqs[i][d["start"][i]:d["end"][i]] if ok[i] else None for i in range(n)], type=pa.binary())
+            if both_strands:
+                rd = ctx.diag_reverse(n)
+
+    def columns(d, prefix="", ran_pass=None):
+        cols = {}
+        absent = np.zeros(len(d), dtype=bool) if ran_pass is None else ~ran_pass
+        for f in ("exact_prefix", "exact_suffix"):
+            cols[prefix + f] = pa.array(d[f], mask=(d[f] < 0) | absent, type=pa.int32())
+        for side in ("prefix", "suffix"):
+            ran = d["len_" + side] >= 0
+            cols[prefix + "score_" + side] = pa.array(d["score_" + side], mask=~ran | absent, type=pa.int32())
+            cols[prefix + "len_" + side] = pa.array(d["len_" + side], mask=~ran | absent, type=pa.int32())
+        cols[prefix + "accept_prefix"] = pa.array(d["start"] >= 0, mask=absent)
+        cols[prefix + "accept_suffix"] = pa.array(d["end"] >= 0, mask=absent)
+        cols[prefix + "start"] = pa.array(d["start"], mask=(d["start"] < 0) | absent, type=pa.int32())
+        cols[prefix + "end"] = pa.array(d["end"], mask=(d["end"] < 0) | absent, type=pa.int32())
+        return cols
+
+    cols = columns(d)
+    if not both_strands:
+        ok = (d["start"] >= 0) & (d["end"] >= 0) & (d["start"] < d["end"])
+        cols["region"] = pa.array([seqs[i][d["start"][i]:d["end"][i]] if ok[i] else None for i in range(n)], type=pa.binary())
+        return pa.table(cols)
+    # the predicate that decides the retry (and that the key kernels use): both located, start < end <= len
+    fwd = (d["start"] >= 0) & (d["end"] >= 0) & (d["start"] < d["end"]) & (d["end"].astype(np.int64) <= length.astype(np.int64))
+    retried = ~fwd & (length > 0)
+    rev = retried & (rd["start"] >= 0) & (rd["end"] >= 0) & (rd["start"] < rd["end"]) & \
+        (rd["end"].astype(np.int64) <= length.astype(np.int64))
+    cols["strand"] = pa.array(np.where(fwd, 1, -1).astype(np.int8), mask=~(fwd | rev), type=pa.int8())
+    cols.update(columns(rd, "rev_", retried))
+    cols["region"] = pa.array([seqs[i][d["start"][i]:d["end"][i]] if fwd[i] else
+                               reverse_complement(seqs[i])[rd["start"][i]:rd["end"][i]] if rev[i] else None
+                               for i in range(n)], type=pa.binary())
     return pa.table(cols)
+
+
+_RC = bytes.maketrans(b"ACGTUacgtu", b"TGCAAtgcaa")
+
+
+def reverse_complement(seq: bytes) -> bytes:
+    """The reverse complement both_strands searches: A<->T, C<->G (either case), U->A, u->a, other bytes unchanged."""
+    return bytes(seq)[::-1].translate(_RC)
 
 
 # ---- synthetic reads (bench + tests) ----------------------------------------------------

@@ -701,7 +701,8 @@ int vfb_destroy(vfb_ctx *c)
     }
     for (auto &ln : c->lanes) {
         DevBuf *lb[] = {&ln.d_start, &ln.d_end, &ln.d_list_a, &ln.d_list_b, &ln.d_fb_a, &ln.d_fb_b, &ln.d_c32, &ln.d_t64, &ln.d_keys,
-                        &ln.d_koff, &ln.d_klen, &ln.d_khash, &ln.d_owner, &ln.d_wins, &ln.d_bestkey, &ln.d_cbval, &ln.d_fb2};
+                        &ln.d_koff, &ln.d_klen, &ln.d_khash, &ln.d_owner, &ln.d_wins, &ln.d_bestkey, &ln.d_cbval, &ln.d_fb2,
+                        &ln.d_rtext, &ln.d_rspans, &ln.d_rsrc, &ln.d_rstart, &ln.d_rend};
         for (auto *b : lb) b->release();
         if (ln.done) cudaEventDestroy(ln.done);
         if (ln.ev_scanned) cudaEventDestroy(ln.ev_scanned);
@@ -715,7 +716,8 @@ int vfb_destroy(vfb_ctx *c)
                       &c->d_diag_len_pre, &c->d_diag_score_suf, &c->d_diag_len_suf, &c->t_slots,
                       &c->t_row_hash, &c->t_row_off, &c->t_row_len, &c->t_row_slot, &c->t_arena, &c->t_counters, &c->t_row_count,
                       &c->m_part_rows, &c->m_part_keys, &c->m_cursors, &c->m_chunk_off, &c->m_send, &c->m_recv,
-                      &c->d_aligned_text, &c->d_span_sum,
+                      &c->d_rdiag_exact_pre, &c->d_rdiag_exact_suf, &c->d_rdiag_score_pre, &c->d_rdiag_len_pre,
+                      &c->d_rdiag_score_suf, &c->d_rdiag_len_suf, &c->d_aligned_text, &c->d_span_sum,
                       &c->x_block_bytes, &c->x_block_rows, &c->x_offsets, &c->x_counts, &c->x_data,
                       &c->p_tiles, &c->p_line_end, &c->p_err, &c->g_tail, &c->g_info};
     for (auto *b : bufs) b->release();
@@ -781,26 +783,35 @@ __global__ void k_accumulate(unsigned long long *t64, const uint32_t *c32, uint3
     t64[T_WINDOWS] += (c32[C_NWINPRE] < win_cap ? c32[C_NWINPRE] : win_cap) + (c32[C_NWINSUF] < win_cap ? c32[C_NWINSUF] : win_cap);
 }
 
-static int run_dp(vfb_ctx *c, Lane &ln, cudaStream_t st, const uint8_t *d_text, const vfb_span *d_spans, bool is_prefix,
-                  uint32_t n_batch, cudaEvent_t *pev)
+// What one pass over a batch reads and writes: the forward pass works on the batch's text and the lane's d_start /
+// d_end, the reverse pass (both_strands) on the gathered reverse complements and d_rstart / d_rend.  The diagnostics
+// buffers (exact_pre, exact_suf, score_pre, len_pre, score_suf, len_suf) are null without diagnostics.
+struct Pass {
+    const uint8_t *text;
+    const vfb_span *spans;
+    uint32_t *start, *end;
+    int32_t *diag[6];
+};
+
+static int run_dp(vfb_ctx *c, Lane &ln, cudaStream_t st, const Pass &ps, bool is_prefix, uint32_t n_batch, cudaEvent_t *pev)
 {
     int rc;
     DpJob job;
     memset(&job, 0, sizeof job);
-    job.text = d_text;
-    job.spans = d_spans;
+    job.text = ps.text;
+    job.spans = ps.spans;
     job.worklist = is_prefix ? ln.d_list_a.as<uint32_t>() : ln.d_list_b.as<uint32_t>();
     job.n_items = ln.d_c32.as<uint32_t>() + (is_prefix ? C_NPRE : C_NSUF);
-    job.bound = is_prefix ? ln.d_start.as<uint32_t>() : ln.d_end.as<uint32_t>();
+    job.bound = is_prefix ? ps.start : ps.end;
     if (c->prm.diagnostics) {
-        job.diag_score = is_prefix ? c->d_diag_score_pre.as<int32_t>() : c->d_diag_score_suf.as<int32_t>();
-        job.diag_len = is_prefix ? c->d_diag_len_pre.as<int32_t>() : c->d_diag_len_suf.as<int32_t>();
+        job.diag_score = ps.diag[is_prefix ? 2 : 4];
+        job.diag_len = ps.diag[is_prefix ? 3 : 5];
     }
     job.cells = ln.d_t64.as<unsigned long long>() + T_CELLS;
     if (is_prefix && c->align_suf && !(c->prm.dp_compute_all || c->prm.diagnostics)) {
         job.next_list = ln.d_list_b.as<uint32_t>();
         job.n_next = ln.d_c32.as<uint32_t>() + C_NSUF;
-        job.other_bound = ln.d_end.as<uint32_t>();
+        job.other_bound = ps.end;
     }
     job.is_prefix = is_prefix ? 1 : 0;
     job.min_accept = is_prefix ? c->min_accept_pre : c->min_accept_suf;
@@ -862,10 +873,107 @@ static int run_dp(vfb_ctx *c, Lane &ln, cudaStream_t st, const uint8_t *d_text, 
     return VFB_OK;
 }
 
+// Scan and alignments of one pass (see Pass), queued on `st` with the alignment kernels on `sd`.
+static int queue_scan_dp(vfb_ctx *c, Lane &ln, cudaStream_t st, cudaStream_t sd, const Pass &ps, uint32_t n,
+                         uint64_t text_bytes_hint, cudaEvent_t *pev)
+{
+    int rc;
+    const bool prof = pev != nullptr, diag = c->prm.diagnostics != 0, split = sd != st;
+    if (prof) VFB_CUDA(cudaEventRecord(pev[0], st));
+    VFB_CUDA(cudaMemsetAsync(ln.d_c32.p, 0, C_COUNT32 * 4, st));
+    VFB_CUDA(cudaMemsetAsync(ln.d_t64.as<unsigned long long>() + T_KEYBYTES, 0, 8, st));
+    ScanJob sj;
+    memset(&sj, 0, sizeof sj);
+    sj.text = ps.text; sj.spans = ps.spans; sj.n_reads = n; sj.text_bytes = text_bytes_hint;
+    sj.start = ps.start; sj.end = ps.end;
+    if (c->align_pre) { sj.list_pre = ln.d_list_a.as<uint32_t>(); sj.n_pre = ln.d_c32.as<uint32_t>() + C_NPRE; }
+    if (c->align_suf) { sj.list_suf = ln.d_list_b.as<uint32_t>(); sj.n_suf = ln.d_c32.as<uint32_t>() + C_NSUF; }
+    sj.compute_all = (c->prm.dp_compute_all || diag) ? 1 : 0;
+    sj.force_general = c->prm.force_general_scan;
+    if ((rc = launch_scan(sj, c->ad_pre, c->ad_suf, c->sm_count, st))) return rc;
+    if (prof) VFB_CUDA(cudaEventRecord(pev[1], st));
+    if (diag) {
+        VFB_CUDA(cudaMemcpyAsync(ps.diag[0], ps.start, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+        VFB_CUDA(cudaMemcpyAsync(ps.diag[1], ps.end, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+        // "no DP ran" markers: score = INT32_MIN (0x80000000), len = -1
+        VFB_CUDA(cudaMemsetAsync(ps.diag[3], 0xFF, (size_t)n * 4, st));
+        VFB_CUDA(cudaMemsetAsync(ps.diag[5], 0xFF, (size_t)n * 4, st));
+        VFB_CUDA(cudaMemsetAsync(ps.diag[2], 0, (size_t)n * 4, st));
+        VFB_CUDA(cudaMemsetAsync(ps.diag[4], 0, (size_t)n * 4, st));
+    }
+    // DP.  The prefix pass runs first: reads it rejects need no suffix alignment (no region
+    // either way, src/lib.rs:288), reads it accepts join the suffix worklist if they need one.
+    // split mode: the (ALU-bound) alignment kernels of the batch run on the lane's lower-priority stream, so that the
+    // other lane's memory-bound kernels get SM resources as soon as alignment blocks retire
+    if (split) {
+        VFB_CUDA(cudaEventRecord(ln.ev_scanned, st));
+        VFB_CUDA(cudaStreamWaitEvent(sd, ln.ev_scanned, 0));
+    }
+    if (prof) VFB_CUDA(cudaEventRecord(pev[2], st));
+    if (c->align_pre) if ((rc = run_dp(c, ln, sd, ps, true, n, pev))) return rc;
+    if (prof) VFB_CUDA(cudaEventRecord(pev[3], st));
+    if (prof) VFB_CUDA(cudaEventRecord(pev[4], st));
+    if (c->align_suf) if ((rc = run_dp(c, ln, sd, ps, false, n, pev))) return rc;
+    if (prof) VFB_CUDA(cudaEventRecord(pev[5], st));
+    k_accumulate<<<1, 1, 0, sd>>>(ln.d_t64.as<unsigned long long>(), ln.d_c32.as<uint32_t>(), ln.win_cap);
+    ++g_launches;
+    if (split) {
+        VFB_CUDA(cudaEventRecord(ln.ev_aligned, sd));
+        VFB_CUDA(cudaStreamWaitEvent(st, ln.ev_aligned, 0));
+    }
+    return VFB_OK;
+}
+
+// Keys and count of one pass.  `probe`: the fused key kernel may look the keys up in the table (it is not known to be
+// empty).  The caller has ordered the previous batch's inserts before this pass (ev_k4) unless `k4_wait` is set, in
+// which case this waits for them in front of the first kernel that touches the table.
+static int queue_keys_count(vfb_ctx *c, Lane &ln, cudaStream_t st, const Pass &ps, uint32_t n, uint64_t text_bytes_hint,
+                            bool probe, bool k4_wait, cudaEvent_t *pev)
+{
+    int rc;
+    KeyJob kj;
+    kj.text = ps.text; kj.spans = ps.spans;
+    kj.start = ps.start; kj.end = ps.end;
+    kj.n_reads = n; kj.text_bytes = text_bytes_hint; kj.skip_translation = c->prm.skip_translation;
+    kj.keys = ln.d_keys.as<uint8_t>(); kj.koff = ln.d_koff.as<uint64_t>();
+    kj.key_cursor = ln.d_t64.as<unsigned long long>() + T_KEYBYTES;
+    kj.klen = ln.d_klen.as<uint32_t>(); kj.khash = ln.d_khash.as<uint64_t>();
+    kj.hash_bits = c->prm.debug_hash_bits;
+    kj.flank_bytes = (uint32_t)(c->prefix.size() + c->suffix.size());
+    // the table work of a batch claims slots by batch-relative index, and the fused key kernel reads slots without
+    // fences: one batch at a time from here on
+    bool k4_waited = false;
+    InsertJob ij;
+    ij.keys = kj.keys; ij.klen = kj.klen; ij.khash = kj.khash; ij.kcount = nullptr; ij.koff = kj.koff;
+    ij.key_stride = 0; ij.n_keys = n; ij.owner_slot = ln.d_owner.as<uint32_t>();
+    int frc = -1;
+    if (c->fused_count && probe) {
+        if (k4_wait) { VFB_CUDA(cudaStreamWaitEvent(st, c->ev_k4, 0)); k4_waited = true; }
+        frc = launch_keys_count(kj, c->tab, ln.d_c32.as<uint32_t>() + C_NMISS, st);
+        if (frc > 0) return frc;
+        if (frc == VFB_OK) { ij.n_keys_dev = ln.d_c32.as<uint32_t>() + C_NMISS; ++c->stats.fused_batches; }
+    }
+    if (frc != VFB_OK && (rc = launch_keys(kj, st))) return rc;
+    if (pev) VFB_CUDA(cudaEventRecord(pev[6], st));
+
+    if (k4_wait && !k4_waited) VFB_CUDA(cudaStreamWaitEvent(st, c->ev_k4, 0));
+    if ((rc = launch_insert(c->tab, ij, st))) return rc;
+    return VFB_OK;
+}
+
+// both_strands needs every offset of the gathered text in 32 bits: a batch's span lengths may sum to at most this.
+#define VFB_STRAND_TEXT_MAX 0xFFFFFFFFull
+
 // The hot loop over one device-resident batch (all work queued on the compute stream).
 // span_len_ub bounds the SUM of the batch's span lengths (it sizes the key space: spans may overlap or repeat, so
 // the text range they address is not a bound); text_bytes_hint is the text this batch's reads are spread over (it
 // sizes the shared-memory tiles of the scan and key kernels; 0 = span_len_ub).
+//
+// both_strands: forward scan -> forward DP -> gather of the reads without a forward region (their reverse
+// complements, k_strand_gather) -> forward keys and count -> reverse scan -> reverse DP -> reverse keys and count, all
+// on the lane, the reverse pass reusing the lane's scratch.  The reverse pass runs over n reads: the span list is
+// zeroed first, so the entries past the gathered ones are empty reads, which no kernel does work for.  A read yields a
+// key on at most one strand, so the batch's bounds on new rows and key bytes are those of one pass.
 static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_spans, uint32_t n,
                          uint64_t span_len_ub, uint64_t text_bytes_hint = 0, unsigned *lanes_used = nullptr)
 {
@@ -873,6 +981,8 @@ static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_sp
     if (!text_bytes_hint) text_bytes_hint = span_bytes_upper;
     int rc;
     if (n == 0) return VFB_OK;
+    const bool both = c->prm.both_strands != 0;
+    if (both && span_len_ub > VFB_STRAND_TEXT_MAX) { set_error("both_strands: the reads of a batch exceed 4 GiB"); return VFB_ERR_ARG; }
     // the lane: with two lanes consecutive batches alternate, each on its own stream, forked from the compute stream
     // (whatever produced the batch's inputs was ordered into that stream by the caller)
     const int li = c->n_lanes > 1 ? (int)(c->lane_seq++ & 1u) : 0;
@@ -907,88 +1017,65 @@ static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_sp
                         &c->d_diag_score_suf, &c->d_diag_len_suf};
         for (auto *b : db) if ((rc = b->ensure((size_t)n * 4))) return rc;
     }
+    Pass fwd{d_text, d_spans, ln.d_start.as<uint32_t>(), ln.d_end.as<uint32_t>(),
+             {c->d_diag_exact_pre.as<int32_t>(), c->d_diag_exact_suf.as<int32_t>(), c->d_diag_score_pre.as<int32_t>(),
+              c->d_diag_len_pre.as<int32_t>(), c->d_diag_score_suf.as<int32_t>(), c->d_diag_len_suf.as<int32_t>()}};
+    Pass rev{};
+    if (both) {
+        // the gathered text sits 16 bytes into its buffer and is followed by 16 more: the kernels load aligned 16-byte
+        // chunks around each read
+        if ((rc = ln.d_rtext.ensure(span_len_ub + 32))) return rc;
+        if ((rc = ln.d_rspans.ensure((size_t)n * 8))) return rc;
+        if ((rc = ln.d_rsrc.ensure((size_t)n * 4))) return rc;
+        if ((rc = ln.d_rstart.ensure((size_t)n * 4))) return rc;
+        if ((rc = ln.d_rend.ensure((size_t)n * 4))) return rc;
+        if (diag) {
+            DevBuf *db[] = {&c->d_rdiag_exact_pre, &c->d_rdiag_exact_suf, &c->d_rdiag_score_pre, &c->d_rdiag_len_pre,
+                            &c->d_rdiag_score_suf, &c->d_rdiag_len_suf};
+            for (auto *b : db) if ((rc = b->ensure((size_t)n * 4))) return rc;
+        }
+        rev = Pass{ln.d_rtext.as<uint8_t>() + 16, ln.d_rspans.as<vfb_span>(), ln.d_rstart.as<uint32_t>(), ln.d_rend.as<uint32_t>(),
+                   {c->d_rdiag_exact_pre.as<int32_t>(), c->d_rdiag_exact_suf.as<int32_t>(), c->d_rdiag_score_pre.as<int32_t>(),
+                    c->d_rdiag_len_pre.as<int32_t>(), c->d_rdiag_score_suf.as<int32_t>(), c->d_rdiag_len_suf.as<int32_t>()}};
+    }
     if ((rc = table_reserve(c, n, key_bytes_ub, true))) return rc;
-    cudaEvent_t *pev = nullptr;
-    if (prof && (rc = prof_events(c, &pev))) return rc;
+    cudaEvent_t *pev = nullptr, *pev_rev = nullptr;
+    if (prof) {
+        // two consecutive groups of 12 events with both_strands (taken before either pointer is kept: the pool may grow)
+        const size_t first = c->ev_used;
+        if ((rc = prof_events(c, &pev))) return rc;
+        if (both && (rc = prof_events(c, &pev_rev))) return rc;
+        pev = &c->evpool[first];
+        if (both) pev_rev = pev + 12;
+    }
     if (c->n_lanes > 1) {
         VFB_CUDA(cudaEventRecord(c->ev_fork, c->st_compute));
         VFB_CUDA(cudaStreamWaitEvent(st, c->ev_fork, 0));
     }
-
-    if (prof) VFB_CUDA(cudaEventRecord(pev[0], st));
-    VFB_CUDA(cudaMemsetAsync(ln.d_c32.p, 0, C_COUNT32 * 4, st));
-    VFB_CUDA(cudaMemsetAsync(ln.d_t64.as<unsigned long long>() + T_KEYBYTES, 0, 8, st));
-    ScanJob sj;
-    memset(&sj, 0, sizeof sj);
-    sj.text = d_text; sj.spans = d_spans; sj.n_reads = n; sj.text_bytes = text_bytes_hint;
-    sj.start = ln.d_start.as<uint32_t>(); sj.end = ln.d_end.as<uint32_t>();
-    if (c->align_pre) { sj.list_pre = ln.d_list_a.as<uint32_t>(); sj.n_pre = ln.d_c32.as<uint32_t>() + C_NPRE; }
-    if (c->align_suf) { sj.list_suf = ln.d_list_b.as<uint32_t>(); sj.n_suf = ln.d_c32.as<uint32_t>() + C_NSUF; }
-    sj.compute_all = (c->prm.dp_compute_all || diag) ? 1 : 0;
-    sj.force_general = c->prm.force_general_scan;
-    if ((rc = launch_scan(sj, c->ad_pre, c->ad_suf, c->sm_count, st))) return rc;
-    if (prof) VFB_CUDA(cudaEventRecord(pev[1], st));
-    if (diag) {
-        VFB_CUDA(cudaMemcpyAsync(c->d_diag_exact_pre.p, ln.d_start.p, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
-        VFB_CUDA(cudaMemcpyAsync(c->d_diag_exact_suf.p, ln.d_end.p, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
-        // "no DP ran" markers: score = INT32_MIN (0x80000000), len = -1
-        VFB_CUDA(cudaMemsetAsync(c->d_diag_len_pre.p, 0xFF, (size_t)n * 4, st));
-        VFB_CUDA(cudaMemsetAsync(c->d_diag_len_suf.p, 0xFF, (size_t)n * 4, st));
-        VFB_CUDA(cudaMemsetAsync(c->d_diag_score_pre.p, 0, (size_t)n * 4, st));
-        VFB_CUDA(cudaMemsetAsync(c->d_diag_score_suf.p, 0, (size_t)n * 4, st));
-    }
-    // DP.  The prefix pass runs first: reads it rejects need no suffix alignment (no region
-    // either way, src/lib.rs:288), reads it accepts join the suffix worklist if they need one.
-    // split mode: the (ALU-bound) alignment kernels of the batch run on the lane's lower-priority stream, so that the
-    // other lane's memory-bound kernels get SM resources as soon as alignment blocks retire
     const bool split = c->n_lanes > 1 && !prof;
     cudaStream_t sd = split ? ln.st_dp : st;
-    if (split) {
-        VFB_CUDA(cudaEventRecord(ln.ev_scanned, st));
-        VFB_CUDA(cudaStreamWaitEvent(sd, ln.ev_scanned, 0));
+    if ((rc = queue_scan_dp(c, ln, st, sd, fwd, n, text_bytes_hint, pev))) return rc;
+    unsigned long long *t64 = ln.d_t64.as<unsigned long long>();
+    if (both) {
+        VFB_CUDA(cudaMemsetAsync(ln.d_rspans.p, 0, (size_t)n * 8, st));
+        VFB_CUDA(cudaMemsetAsync(t64 + T_GATHER, 0, 8, st));
+        StrandJob sj{d_spans, fwd.start, fwd.end, n, d_text, ln.d_rtext.as<uint8_t>() + 16, ln.d_rspans.as<vfb_span>(),
+                     ln.d_rsrc.as<uint32_t>(), t64 + T_GATHER, t64 + T_REVREADS};
+        if ((rc = launch_strand_gather(sj, c->sm_count, st))) return rc;
     }
-    if (prof) VFB_CUDA(cudaEventRecord(pev[2], st));
-    if (c->align_pre) if ((rc = run_dp(c, ln, sd, d_text, d_spans, true, n, prof ? pev : nullptr))) return rc;
-    if (prof) VFB_CUDA(cudaEventRecord(pev[3], st));
-    if (prof) VFB_CUDA(cudaEventRecord(pev[4], st));
-    if (c->align_suf) if ((rc = run_dp(c, ln, sd, d_text, d_spans, false, n, prof ? pev : nullptr))) return rc;
-    if (prof) VFB_CUDA(cudaEventRecord(pev[5], st));
-    k_accumulate<<<1, 1, 0, sd>>>(ln.d_t64.as<unsigned long long>(), ln.d_c32.as<uint32_t>(), ln.win_cap);
-    ++g_launches;
-    if (split) {
-        VFB_CUDA(cudaEventRecord(ln.ev_aligned, sd));
-        VFB_CUDA(cudaStreamWaitEvent(st, ln.ev_aligned, 0));
-    }
-
-    KeyJob kj;
-    kj.text = d_text; kj.spans = d_spans;
-    kj.start = ln.d_start.as<uint32_t>(); kj.end = ln.d_end.as<uint32_t>();
-    kj.n_reads = n; kj.text_bytes = text_bytes_hint; kj.skip_translation = c->prm.skip_translation;
-    kj.keys = ln.d_keys.as<uint8_t>(); kj.koff = ln.d_koff.as<uint64_t>();
-    kj.key_cursor = ln.d_t64.as<unsigned long long>() + T_KEYBYTES;
-    kj.klen = ln.d_klen.as<uint32_t>(); kj.khash = ln.d_khash.as<uint64_t>();
-    kj.hash_bits = c->prm.debug_hash_bits;
-    kj.flank_bytes = (uint32_t)(c->prefix.size() + c->suffix.size());
-    // the table work of a batch claims slots by batch-relative index, and the fused key kernel reads slots without
-    // fences: one batch at a time from here on
-    bool k4_waited = false;
-    InsertJob ij;
-    ij.keys = kj.keys; ij.klen = kj.klen; ij.khash = kj.khash; ij.kcount = nullptr; ij.koff = kj.koff;
-    ij.key_stride = 0; ij.n_keys = n; ij.owner_slot = ln.d_owner.as<uint32_t>();
-    int frc = -1;
     // (a table that is known to be empty — the first batch after a clear — has nothing to find: the probe would
     // only cost)
-    if (c->fused_count && c->ub_rows > 0) {
-        if (c->n_lanes > 1 && c->k4_pending) { VFB_CUDA(cudaStreamWaitEvent(st, c->ev_k4, 0)); k4_waited = true; }
-        frc = launch_keys_count(kj, c->tab, ln.d_c32.as<uint32_t>() + C_NMISS, st);
-        if (frc > 0) return frc;
-        if (frc == VFB_OK) { ij.n_keys_dev = ln.d_c32.as<uint32_t>() + C_NMISS; ++c->stats.fused_batches; }
+    const bool k4_wait = c->n_lanes > 1 && c->k4_pending;
+    if ((rc = queue_keys_count(c, ln, st, fwd, n, text_bytes_hint, c->ub_rows > 0, k4_wait, pev))) return rc;
+    if (both) {
+        if (prof) VFB_CUDA(cudaEventRecord(pev[7], st));
+        if ((rc = queue_scan_dp(c, ln, st, sd, rev, n, text_bytes_hint, pev_rev))) return rc;
+        // the forward pass may have added rows: the reverse keys always probe
+        if ((rc = launch_strand_tally(t64 + T_REVCOUNTED, c->tab.counters, false, st))) return rc;
+        if ((rc = queue_keys_count(c, ln, st, rev, n, text_bytes_hint, true, false, pev_rev))) return rc;
+        if ((rc = launch_strand_tally(t64 + T_REVCOUNTED, c->tab.counters, true, st))) return rc;
+        pev = pev_rev;
     }
-    if (frc != VFB_OK && (rc = launch_keys(kj, st))) return rc;
-    if (prof) VFB_CUDA(cudaEventRecord(pev[6], st));
-
-    if (c->n_lanes > 1 && c->k4_pending && !k4_waited) VFB_CUDA(cudaStreamWaitEvent(st, c->ev_k4, 0));
-    if ((rc = launch_insert(c->tab, ij, st))) return rc;
     if ((rc = snaps_push(c, n, key_bytes_ub, st))) return rc;
     if (c->n_lanes > 1) {
         VFB_CUDA(cudaEventRecord(c->ev_k4, st));
@@ -1052,8 +1139,9 @@ int vfb_submit_device(vfb_ctx *c, const uint8_t *d_text, uint64_t text_bytes, co
         d_text = dst;
     }
     if ((rc = c->d_span_sum.ensure(16))) return rc;
+    uint64_t n = 0;
     while (done < n_reads) {
-        const uint64_t n = n_reads - done < c->batch_reads ? n_reads - done : c->batch_reads;
+        if (!n) n = n_reads - done < c->batch_reads ? n_reads - done : c->batch_reads;
         // the spans are the caller's: every one must lie inside the buffer, and the key space of the batch is
         // bounded by the sum of their lengths (overlapping and repeated spans are legal)
         unsigned long long chk[2] = {0, 0};
@@ -1063,9 +1151,16 @@ int vfb_submit_device(vfb_ctx *c, const uint8_t *d_text, uint64_t text_bytes, co
         VFB_CUDA(cudaStreamSynchronize(c->st_compute));
         c->stats.d2h_bytes += 16;
         if (chk[1]) { set_error("span outside the text buffer"); rc = VFB_ERR_ARG; break; }
+        if (c->prm.both_strands && chk[0] > VFB_STRAND_TEXT_MAX) {
+            // the gathered reverse complements need 32-bit offsets: only overlapping spans get here; halve and measure again
+            if (n == 1) { set_error("both_strands: a read longer than 4 GiB"); rc = VFB_ERR_ARG; break; }
+            n /= 2;
+            continue;
+        }
         if ((rc = process_batch(c, d_text, d_spans + done, (uint32_t)n, chk[0],
                                 (uint64_t)((double)text_bytes * (double)n / (double)n_reads) + 1))) break;
         done += n;
+        n = 0;
     }
     bump_launches(c, before);
     return rc;
@@ -1120,7 +1215,8 @@ int vfb_submit_host(vfb_ctx *c, const uint8_t *text, uint64_t text_bytes, const 
                     all.sum += p.sum;
                     all.bad |= p.bad;
                 }
-                if (!all.bad && all.hi >= all.lo && all.hi - all.lo <= c->batch_bytes) {
+                if (!all.bad && all.hi >= all.lo && all.hi - all.lo <= c->batch_bytes &&
+                    !(c->prm.both_strands && all.sum > VFB_STRAND_TEXT_MAX)) {
                     n = cand; lo = all.lo; hi = all.hi; len_sum = all.sum;
                     cut = true;
                 }
@@ -1131,6 +1227,8 @@ int vfb_submit_host(vfb_ctx *c, const uint8_t *text, uint64_t text_bytes, const 
             if ((uint64_t)s.off + s.len > text_bytes) { set_error("span outside the text buffer"); rc = VFB_ERR_ARG; break; }
             const uint64_t nlo = s.off < lo ? s.off : lo, nhi = (uint64_t)s.off + s.len > hi ? (uint64_t)s.off + s.len : hi;
             if (n > 0 && nhi - nlo > c->batch_bytes) break;
+            // both_strands: the gathered reverse complements need 32-bit offsets (only overlapping spans get here)
+            if (n > 0 && c->prm.both_strands && len_sum + s.len > VFB_STRAND_TEXT_MAX) break;
             lo = nlo; hi = nhi; len_sum += s.len; ++n;
         }
         if (rc) break;
@@ -1489,9 +1587,19 @@ int vfb_get_stats(vfb_ctx *c, vfb_stats *out)
     c->stats.unique = ctr[0];
     c->stats.counted = ctr[2];
     c->stats.fused_hits = ctr[3];
+    c->stats.reverse_reads = t64[T_REVREADS];
+    c->stats.reverse_counted = t64[T_REVCOUNTED];
     *out = c->stats;
     return VFB_OK;
 }
+
+}  // extern "C"
+
+static int diag_rows(vfb_ctx *c, const std::vector<uint32_t> &ep, const std::vector<uint32_t> &es, const std::vector<int32_t> &sp,
+                     const std::vector<int32_t> &lp, const std::vector<int32_t> &ss, const std::vector<int32_t> &ls,
+                     const std::vector<uint32_t> &st, const std::vector<uint32_t> &en, vfb_read_diag *out, size_t n);
+
+extern "C" {
 
 int vfb_get_diag(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
 {
@@ -1512,6 +1620,53 @@ int vfb_get_diag(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
     VFB_CUDA(cudaMemcpy(ss.data(), c->d_diag_score_suf.p, n * 4, cudaMemcpyDeviceToHost));
     VFB_CUDA(cudaMemcpy(ls.data(), c->d_diag_len_suf.p, n * 4, cudaMemcpyDeviceToHost));
     c->stats.d2h_bytes += n * 32;
+    return diag_rows(c, ep, es, sp, lp, ss, ls, st, en, out, n);
+}
+
+int vfb_get_diag_reverse(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
+{
+    if (!c || !out) { set_error("null argument"); return VFB_ERR_ARG; }
+    if (!c->prm.diagnostics || !c->diag_valid) { set_error("diagnostics were not enabled for the last batch"); return VFB_ERR_ARG; }
+    if (!c->prm.both_strands) { set_error("the context was created without both_strands"); return VFB_ERR_ARG; }
+    if (n_reads != c->diag_n) { set_error("diagnostics cover exactly the last batch"); return VFB_ERR_ARG; }
+    int rc = vfb_sync(c);
+    if (rc) return rc;
+    const size_t n = (size_t)n_reads;
+    unsigned long long cursor = 0;
+    VFB_CUDA(cudaMemcpy(&cursor, c->lanes[0].d_t64.as<unsigned long long>() + T_GATHER, 8, cudaMemcpyDeviceToHost));
+    const size_t m = (size_t)(cursor >> 32);            // gathered reads, in compact order
+    std::vector<uint32_t> ep(m), es(m), st(m), en(m), src(m);
+    std::vector<int32_t> sp(m), lp(m), ss(m), ls(m);
+    if (m) {
+        VFB_CUDA(cudaMemcpy(ep.data(), c->d_rdiag_exact_pre.p, m * 4, cudaMemcpyDeviceToHost));
+        VFB_CUDA(cudaMemcpy(es.data(), c->d_rdiag_exact_suf.p, m * 4, cudaMemcpyDeviceToHost));
+        VFB_CUDA(cudaMemcpy(st.data(), c->lanes[0].d_rstart.p, m * 4, cudaMemcpyDeviceToHost));
+        VFB_CUDA(cudaMemcpy(en.data(), c->lanes[0].d_rend.p, m * 4, cudaMemcpyDeviceToHost));
+        VFB_CUDA(cudaMemcpy(sp.data(), c->d_rdiag_score_pre.p, m * 4, cudaMemcpyDeviceToHost));
+        VFB_CUDA(cudaMemcpy(lp.data(), c->d_rdiag_len_pre.p, m * 4, cudaMemcpyDeviceToHost));
+        VFB_CUDA(cudaMemcpy(ss.data(), c->d_rdiag_score_suf.p, m * 4, cudaMemcpyDeviceToHost));
+        VFB_CUDA(cudaMemcpy(ls.data(), c->d_rdiag_len_suf.p, m * 4, cudaMemcpyDeviceToHost));
+        VFB_CUDA(cudaMemcpy(src.data(), c->lanes[0].d_rsrc.p, m * 4, cudaMemcpyDeviceToHost));
+    }
+    c->stats.d2h_bytes += 8 + m * 36;
+    const vfb_read_diag absent = {-1, -1, INT32_MIN, -1, INT32_MIN, -1, -1, -1};
+    for (size_t i = 0; i < n; ++i) out[i] = absent;
+    std::vector<vfb_read_diag> rows(m);
+    diag_rows(c, ep, es, sp, lp, ss, ls, st, en, rows.data(), m);
+    for (size_t i = 0; i < m; ++i) {
+        if (src[i] >= n) { set_error("reverse diagnostics: read index out of range"); return VFB_ERR_CUDA; }
+        out[src[i]] = rows[i];
+    }
+    return VFB_OK;
+}
+
+}  // extern "C"
+
+// Device boundaries and diagnostics columns -> vfb_read_diag rows.
+static int diag_rows(vfb_ctx *c, const std::vector<uint32_t> &ep, const std::vector<uint32_t> &es, const std::vector<int32_t> &sp,
+                     const std::vector<int32_t> &lp, const std::vector<int32_t> &ss, const std::vector<int32_t> &ls,
+                     const std::vector<uint32_t> &st, const std::vector<uint32_t> &en, vfb_read_diag *out, size_t n)
+{
     const uint32_t A = (uint32_t)c->prefix.size();
     for (size_t i = 0; i < n; ++i) {
         vfb_read_diag d;
@@ -1527,8 +1682,6 @@ int vfb_get_diag(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
     }
     return VFB_OK;
 }
-
-}  // extern "C"
 
 // Export, pass 1: slot counts -> row counts, sizes of what will be exported (rows with a non-zero count).
 int vfb_internal_export_sizes(vfb_ctx *c, uint64_t *rows_out, uint64_t *bytes_out)

@@ -89,6 +89,9 @@ struct Lane {
     DevBuf d_start, d_end, d_list_a, d_list_b, d_fb_a, d_fb_b, d_c32, d_t64;
     DevBuf d_keys, d_koff, d_klen, d_khash, d_owner;
     DevBuf d_wins, d_bestkey, d_cbval, d_fb2;   // windowed DP: window items, per-item results, second fallback list
+    // both_strands: the reverse pass's text (reverse complements, padded), compact spans, original read indices and
+    // boundaries (the forward boundaries stay in d_start / d_end)
+    DevBuf d_rtext, d_rspans, d_rsrc, d_rstart, d_rend;
     uint32_t win_cap = 0;
 };
 
@@ -120,7 +123,8 @@ enum { C_NPRE = 0, C_NSUF, C_FBPRE, C_FBSUF, C_FB2PRE, C_FB2SUF, C_NWINPRE, C_NW
        C_NMISS = 160,        // fused key + count kernel: keys left for the insert kernels
        C_COUNT32 = 192 };
 // 64-bit device counters
-enum { T_CELLS = 0, T_DPPRE, T_DPSUF, T_KEYBYTES, T_CELLSCOMP, T_WINDOWS, T_COUNT64 };
+// (T_GATHER: the gather cursor of the batch; T_REVREADS / T_REVCOUNTED: both_strands statistics)
+enum { T_CELLS = 0, T_DPPRE, T_DPSUF, T_KEYBYTES, T_CELLSCOMP, T_WINDOWS, T_GATHER, T_REVREADS, T_REVCOUNTED, T_COUNT64 };
 
 }  // namespace vfb
 
@@ -158,6 +162,8 @@ struct vfb_ctx {
     vfb::DevBuf d_aligned_text;     // aligned copy of an unaligned caller buffer (vfb_submit_device)
     vfb::DevBuf d_span_sum;         // vfb_submit_device: sum of the span lengths of a batch
     vfb::DevBuf d_diag_exact_pre, d_diag_exact_suf, d_diag_score_pre, d_diag_len_pre, d_diag_score_suf, d_diag_len_suf;
+    // both_strands + diagnostics: the reverse pass's diagnostics, in compact (gathered) order
+    vfb::DevBuf d_rdiag_exact_pre, d_rdiag_exact_suf, d_rdiag_score_pre, d_rdiag_len_pre, d_rdiag_score_suf, d_rdiag_len_suf;
     uint64_t diag_n = 0;
     bool diag_valid = false;
 

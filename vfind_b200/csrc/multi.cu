@@ -358,6 +358,7 @@ int vfb_multi_get_stats(vfb_multi *m, vfb_stats *out)
         out->ms_count += s.ms_count; out->ms_total += s.ms_total; out->dp_kernel_launches += s.dp_kernel_launches;
         out->dp_kernel_kind = s.dp_kernel_kind; out->dp_cells_computed += s.dp_cells_computed; out->dp_windows += s.dp_windows;
         out->ms_dp_filter += s.ms_dp_filter; out->ms_dp_window += s.ms_dp_window;
+        out->reverse_reads += s.reverse_reads; out->reverse_counted += s.reverse_counted;
     }
     return VFB_OK;
 }

@@ -281,6 +281,25 @@ int launch_gz_resolve(const uint32_t *d_live, const unsigned long long *d_text_o
                       const uint16_t *d_out16, uint32_t cap, const uint8_t *d_win_store, uint8_t *d_text, uint32_t *d_piece_nl,
                       uint32_t *d_piece_crc, int first_window_known, uint32_t *d_flag_unknown, cudaStream_t st);
 
+// ---------------------------------------------------------------- both_strands (kernels_strand.cu)
+// Reverse complements of the reads that have no forward region, gathered back to back into `out` (16-byte aligned
+// base; the caller keeps 16 readable bytes before it and after the gathered text, which is at most 2^32 - 1 bytes).
+// out_spans / src are compact: entry i is the i-th gathered read and its index in the batch.  `cursor` (zeroed before
+// the launch) ends as gathered reads << 32 | gathered bytes; *n_gathered is incremented by the gathered reads.
+struct StrandJob {
+    const vfb_span *spans;
+    const uint32_t *start, *end;      // the forward pass's final boundaries
+    uint32_t n;
+    const uint8_t *text;
+    uint8_t *out;
+    vfb_span *out_spans;
+    uint32_t *src;
+    unsigned long long *cursor, *n_gathered;
+};
+int launch_strand_gather(const StrandJob &job, int sm_count, cudaStream_t st);
+// *t64 -= counters[2] (after = false) or += counters[2] (after = true): brackets the reverse pass's counting.
+int launch_strand_tally(unsigned long long *t64, const unsigned long long *counters, bool after, cudaStream_t st);
+
 // ---------------------------------------------------------------- misc
 int launch_synth(const vfb_synth_cfg &cfg, uint64_t first, uint64_t n, uint8_t *d_text,
                  vfb_span *d_spans, cudaStream_t st);
