@@ -279,17 +279,12 @@ static int prof_resolve(vfb_ctx *c)
         VFB_CUDA(cudaEventElapsedTime(&ms, ev[5], ev[6])); c->stats.ms_translate += ms;
         VFB_CUDA(cudaEventElapsedTime(&ms, ev[6], ev[7])); c->stats.ms_count += ms;
         VFB_CUDA(cudaEventElapsedTime(&ms, ev[0], ev[7])); c->stats.ms_total += ms;
-        if (c->stats.dp_kernel_kind == 3) {
-            // windowed DP: [2] filter [8] windows [9] resolve + fallbacks [3], same for the suffix pass
-            if (c->win_k_pre >= 0 && c->align_pre) {
-                VFB_CUDA(cudaEventElapsedTime(&ms, ev[2], ev[8])); c->stats.ms_dp_filter += ms;
-                VFB_CUDA(cudaEventElapsedTime(&ms, ev[8], ev[9])); c->stats.ms_dp_window += ms;
+        // windowed DP: [2] filter [8] windows [9] resolve + fallbacks [3] for the prefix, [4] [10] [11] [5] for the suffix
+        for (int s = 0; s < 2; ++s)
+            if (c->side[s].win_k >= 0) {
+                VFB_CUDA(cudaEventElapsedTime(&ms, ev[2 + 2 * s], ev[8 + 2 * s])); c->stats.ms_dp_filter += ms;
+                VFB_CUDA(cudaEventElapsedTime(&ms, ev[8 + 2 * s], ev[9 + 2 * s])); c->stats.ms_dp_window += ms;
             }
-            if (c->win_k_suf >= 0 && c->align_suf) {
-                VFB_CUDA(cudaEventElapsedTime(&ms, ev[4], ev[10])); c->stats.ms_dp_filter += ms;
-                VFB_CUDA(cudaEventElapsedTime(&ms, ev[10], ev[11])); c->stats.ms_dp_window += ms;
-            }
-        }
     }
     c->ev_used = 0;
     return VFB_OK;
@@ -560,15 +555,18 @@ int vfb_create(const vfb_params *p, vfb_ctx **out)
     if (!p || !out) { set_error("null argument"); return VFB_ERR_ARG; }
     if (p->struct_size != sizeof(vfb_params)) { set_error("vfb_params size mismatch"); return VFB_ERR_ARG; }
     if ((p->prefix_len && !p->prefix) || (p->suffix_len && !p->suffix)) { set_error("null adapter"); return VFB_ERR_ARG; }
-    bool skip_pre, skip_suf;
+    const uint8_t *const seq[2] = {p->prefix, p->suffix};
+    const uint64_t len[2] = {p->prefix_len, p->suffix_len};
+    const double thr[2] = {p->accept_prefix_alignment, p->accept_suffix_alignment};
+    bool skip[2];
     int rc;
-    if ((rc = preflight(p->accept_prefix_alignment, &skip_pre))) return rc;   // :239
-    if ((rc = preflight(p->accept_suffix_alignment, &skip_suf))) return rc;   // :249
-    if (p->prefix_len > VFB_MAX_SCAN_ADAPTER || p->suffix_len > VFB_MAX_SCAN_ADAPTER) {
+    for (int s = 0; s < 2; ++s)
+        if ((rc = preflight(thr[s], &skip[s]))) return rc;   // :239, :249
+    if (len[PRE] > VFB_MAX_SCAN_ADAPTER || len[SUF] > VFB_MAX_SCAN_ADAPTER) {
         set_error("adapters longer than 256 bases are not supported");
         return VFB_ERR_ARG;
     }
-    if ((!skip_pre && p->prefix_len == 0) || (!skip_suf && p->suffix_len == 0)) {
+    if ((!skip[PRE] && len[PRE] == 0) || (!skip[SUF] && len[SUF] == 0)) {
         // Profile::new on an empty adapter fails and the reference unwraps it (src/lib.rs:124-126)
         set_error("Error creating profile for adapter: empty adapter");
         return VFB_ERR_VALUE;
@@ -582,17 +580,16 @@ int vfb_create(const vfb_params *p, vfb_ctx **out)
     }
     vfb_ctx *c = new vfb_ctx();
     c->prm = *p;
-    c->prefix.assign((const char *)p->prefix, p->prefix_len);
-    c->suffix.assign((const char *)p->suffix, p->suffix_len);
-    c->prm.prefix = (const uint8_t *)c->prefix.data();
-    c->prm.suffix = (const uint8_t *)c->suffix.data();
-    fill_adapter(&c->ad_pre, c->prefix);
-    fill_adapter(&c->ad_suf, c->suffix);
+    for (int s = 0; s < 2; ++s) {
+        AdapterSide &side = c->side[s];
+        side.seq.assign((const char *)seq[s], len[s]);
+        fill_adapter(&side.ad, side.seq);
+        side.align = !skip[s];
+        side.min_accept = accept_bound(thr[s], p->match_score, len[s]);
+    }
+    c->prm.prefix = (const uint8_t *)c->side[PRE].seq.data();
+    c->prm.suffix = (const uint8_t *)c->side[SUF].seq.data();
     c->sc = DpScoring{p->match_score, p->mismatch_score, p->gap_open_penalty, p->gap_extend_penalty};
-    c->align_pre = !skip_pre;
-    c->align_suf = !skip_suf;
-    c->min_accept_pre = accept_bound(p->accept_prefix_alignment, p->match_score, p->prefix_len);
-    c->min_accept_suf = accept_bound(p->accept_suffix_alignment, p->match_score, p->suffix_len);
     c->batch_reads = p->batch_reads ? p->batch_reads : (8ull << 20);
     c->batch_bytes = p->batch_bytes ? p->batch_bytes : (2ull << 30);
     if (c->batch_reads > 0x7FFFFFFFull) c->batch_reads = 0x7FFFFFFFull;
@@ -634,33 +631,26 @@ int vfb_create(const vfb_params *p, vfb_ctx **out)
     if (p->diagnostics) c->n_lanes = 1;
 
     // DP setup: packed layout when the scores fit, else the fallback kernel
-    const bool force_generic = p->force_generic_dp != 0;
     const bool want_window = p->dp_mode != 1 && (!p->diagnostics || p->dp_mode == 2);
-    auto setup_dp = [&](const std::string &ad, bool enabled, int min_accept, bool *packed, DpLayout *lay, uint32_t *lcap,
-                        int *win_k, DevBuf *codes) -> int {
-        *packed = false;
-        if (!enabled) return VFB_OK;
-        if (ad.size() > VFB_MAX_ADAPTER) { set_error("adapter too long for alignment"); return VFB_ERR_ARG; }
+    for (AdapterSide &side : c->side) {
+        if (!side.align) continue;
+        const std::string &ad = side.seq;
+        if (ad.size() > VFB_MAX_ADAPTER) { set_error("adapter too long for alignment"); return fail(VFB_ERR_ARG); }
         long long worst = (long long)(std::abs((long long)c->sc.match) + std::abs((long long)c->sc.mismatch) +
                                       std::abs((long long)c->sc.open) + std::abs((long long)c->sc.extend));
-        if (worst > (1 << 20)) { set_error("alignment scores beyond +-2^20 are not supported"); return VFB_ERR_ARG; }
-        if (!force_generic) *packed = plan_packed_dp(c->sc, (uint32_t)ad.size(), min_accept, want_window, lay, lcap, win_k);
+        if (worst > (1 << 20)) { set_error("alignment scores beyond +-2^20 are not supported"); return fail(VFB_ERR_ARG); }
+        if (!p->force_generic_dp)
+            side.packed = plan_packed_dp(c->sc, (uint32_t)ad.size(), side.min_accept, want_window, &side.lay, &side.lcap, &side.win_k);
         std::vector<uint8_t> code(ad.size());
         for (size_t i = 0; i < ad.size(); ++i) code[i] = (uint8_t)dp_code((uint8_t)ad[i]);
-        int r = codes->ensure(code.size());
-        if (r) return r;
-        VFB_CUDA(cudaMemcpy(codes->p, code.data(), code.size(), cudaMemcpyHostToDevice));
-        return VFB_OK;
-    };
-    if ((rc = setup_dp(c->prefix, c->align_pre, c->min_accept_pre, &c->packed_pre, &c->lay_pre, &c->lcap_pre, &c->win_k_pre,
-                       &c->d_code_pre)))
-        return fail(rc);
-    if ((rc = setup_dp(c->suffix, c->align_suf, c->min_accept_suf, &c->packed_suf, &c->lay_suf, &c->lcap_suf, &c->win_k_suf,
-                       &c->d_code_suf)))
-        return fail(rc);
-    if (c->align_pre || c->align_suf) {
+        if ((rc = side.d_code.ensure(code.size()))) return fail(rc);
+        if ((e = cudaMemcpy(side.d_code.p, code.data(), code.size(), cudaMemcpyHostToDevice)) != cudaSuccess)
+            return fail(cuda_fail(e, "cudaMemcpy", __FILE__, __LINE__));
+    }
+    const AdapterSide &pre = c->side[PRE], &suf = c->side[SUF];
+    if (pre.align || suf.align) {
         c->generic_threads = dp_generic_threads(c->sm_count);
-        size_t amax = c->prefix.size() > c->suffix.size() ? c->prefix.size() : c->suffix.size();
+        size_t amax = pre.seq.size() > suf.seq.size() ? pre.seq.size() : suf.seq.size();
         if ((rc = c->d_generic_scratch.ensure(4 * amax * (size_t)c->generic_threads * sizeof(int32_t)))) return fail(rc);
     }
     for (auto &ln : c->lanes) {
@@ -672,8 +662,7 @@ int vfb_create(const vfb_params *p, vfb_ctx **out)
     trace("vfb_create: streams, events, DP setup done");
     if ((rc = table_init(c))) return fail(rc);
     trace("vfb_create: table ready");
-    c->stats.dp_kernel_kind = (c->packed_pre || c->packed_suf) ? 1 : ((c->align_pre || c->align_suf) ? 2 : 0);
-    if (c->win_k_pre >= 0 || c->win_k_suf >= 0) c->stats.dp_kernel_kind = 3;
+    c->stats.dp_kernel_kind = (pre.win_k >= 0 || suf.win_k >= 0) ? 3 : (pre.packed || suf.packed) ? 1 : (pre.align || suf.align) ? 2 : 0;
     *out = c;
     return VFB_OK;
 }
@@ -700,7 +689,7 @@ int vfb_destroy(vfb_ctx *c)
         for (auto &ev : g.computed) if (ev) cudaEventDestroy(ev);
     }
     for (auto &ln : c->lanes) {
-        DevBuf *lb[] = {&ln.d_start, &ln.d_end, &ln.d_list_a, &ln.d_list_b, &ln.d_fb_a, &ln.d_fb_b, &ln.d_c32, &ln.d_t64, &ln.d_keys,
+        DevBuf *lb[] = {&ln.d_start, &ln.d_end, &ln.d_list[PRE], &ln.d_list[SUF], &ln.d_fb[PRE], &ln.d_fb[SUF], &ln.d_c32, &ln.d_t64, &ln.d_keys,
                         &ln.d_koff, &ln.d_klen, &ln.d_khash, &ln.d_owner, &ln.d_wins, &ln.d_bestkey, &ln.d_cbval, &ln.d_fb2,
                         &ln.d_rtext, &ln.d_rspans, &ln.d_rsrc, &ln.d_rstart, &ln.d_rend};
         for (auto *b : lb) b->release();
@@ -712,12 +701,12 @@ int vfb_destroy(vfb_ctx *c)
     }
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev_k4) cudaEventDestroy(c->ev_k4);
-    DevBuf *bufs[] = {&c->d_code_pre, &c->d_code_suf, &c->d_generic_scratch, &c->d_diag_exact_pre, &c->d_diag_exact_suf, &c->d_diag_score_pre,
-                      &c->d_diag_len_pre, &c->d_diag_score_suf, &c->d_diag_len_suf, &c->t_slots,
+    for (auto &side : c->side) side.d_code.release();
+    c->diag_fwd.release(); c->diag_rev.release();
+    DevBuf *bufs[] = {&c->d_generic_scratch, &c->t_slots,
                       &c->t_row_hash, &c->t_row_off, &c->t_row_len, &c->t_row_slot, &c->t_arena, &c->t_counters, &c->t_row_count,
                       &c->m_part_rows, &c->m_part_keys, &c->m_cursors, &c->m_chunk_off, &c->m_send, &c->m_recv,
-                      &c->d_rdiag_exact_pre, &c->d_rdiag_exact_suf, &c->d_rdiag_score_pre, &c->d_rdiag_len_pre,
-                      &c->d_rdiag_score_suf, &c->d_rdiag_len_suf, &c->d_aligned_text, &c->d_span_sum,
+                      &c->d_aligned_text, &c->d_span_sum,
                       &c->x_block_bytes, &c->x_block_rows, &c->x_offsets, &c->x_counts, &c->x_data,
                       &c->p_tiles, &c->p_line_end, &c->p_err, &c->g_tail, &c->g_info};
     for (auto *b : bufs) b->release();
@@ -784,92 +773,74 @@ __global__ void k_accumulate(unsigned long long *t64, const uint32_t *c32, uint3
 }
 
 // What one pass over a batch reads and writes: the forward pass works on the batch's text and the lane's d_start /
-// d_end, the reverse pass (both_strands) on the gathered reverse complements and d_rstart / d_rend.  The diagnostics
-// buffers (exact_pre, exact_suf, score_pre, len_pre, score_suf, len_suf) are null without diagnostics.
+// d_end, the reverse pass (both_strands) on the gathered reverse complements and d_rstart / d_rend.  `bound` holds
+// them by side (start: prefix, end: suffix); `diag` is null without diagnostics.
 struct Pass {
     const uint8_t *text;
     const vfb_span *spans;
-    uint32_t *start, *end;
-    int32_t *diag[6];
+    uint32_t *bound[2];
+    const DiagBufs *diag;
 };
 
-static int run_dp(vfb_ctx *c, Lane &ln, cudaStream_t st, const Pass &ps, bool is_prefix, uint32_t n_batch, cudaEvent_t *pev)
+// The alignments of adapter side `s`, as a fallback chain: the windowed DP (filter -> DP on the flagged windows ->
+// resolve) passes the reads it cannot take to the packed full-matrix kernel, which passes the reads too long for the
+// packed word (normally none) to the unpacked one.  Each stage runs only where vfb_create planned it.
+static int run_dp(vfb_ctx *c, Lane &ln, cudaStream_t st, const Pass &ps, int s, uint32_t n_batch, cudaEvent_t *pev)
 {
     int rc;
+    const AdapterSide &side = c->side[s];
+    uint32_t *c32 = ln.d_c32.as<uint32_t>();
     DpJob job;
     memset(&job, 0, sizeof job);
     job.text = ps.text;
     job.spans = ps.spans;
-    job.worklist = is_prefix ? ln.d_list_a.as<uint32_t>() : ln.d_list_b.as<uint32_t>();
-    job.n_items = ln.d_c32.as<uint32_t>() + (is_prefix ? C_NPRE : C_NSUF);
-    job.bound = is_prefix ? ps.start : ps.end;
-    if (c->prm.diagnostics) {
-        job.diag_score = ps.diag[is_prefix ? 2 : 4];
-        job.diag_len = ps.diag[is_prefix ? 3 : 5];
+    job.worklist = ln.d_list[s].as<uint32_t>();
+    job.n_items = c32 + C_NPRE + s;
+    job.bound = ps.bound[s];
+    if (ps.diag) {
+        job.diag_score = ps.diag->score[s].as<int32_t>();
+        job.diag_len = ps.diag->len[s].as<int32_t>();
     }
     job.cells = ln.d_t64.as<unsigned long long>() + T_CELLS;
-    if (is_prefix && c->align_suf && !(c->prm.dp_compute_all || c->prm.diagnostics)) {
-        job.next_list = ln.d_list_b.as<uint32_t>();
-        job.n_next = ln.d_c32.as<uint32_t>() + C_NSUF;
-        job.other_bound = ps.end;
+    if (s == PRE && c->side[SUF].align && !(c->prm.dp_compute_all || c->prm.diagnostics)) {
+        job.next_list = ln.d_list[SUF].as<uint32_t>();
+        job.n_next = c32 + C_NSUF;
+        job.other_bound = ps.bound[SUF];
     }
-    job.is_prefix = is_prefix ? 1 : 0;
-    job.min_accept = is_prefix ? c->min_accept_pre : c->min_accept_suf;
-    const std::string &ad = is_prefix ? c->prefix : c->suffix;
-    job.adapter_len = (uint32_t)ad.size();
-    const bool packed = is_prefix ? c->packed_pre : c->packed_suf;
-    DpGenericJob gj;
-    gj.sc = c->sc;
-    gj.d_adapter_code = is_prefix ? c->d_code_pre.as<uint8_t>() : c->d_code_suf.as<uint8_t>();
-    gj.scratch = c->d_generic_scratch.as<int32_t>();
-    gj.n_threads = c->generic_threads;
-    const int K = is_prefix ? c->win_k_pre : c->win_k_suf;
-    const bool windowed = packed && K >= 0 && c->prm.dp_mode != 1 && (!c->prm.diagnostics || c->prm.dp_mode == 2);
-    if (windowed) {
-        // filter -> DP on the flagged windows -> resolve; reads the windowed path cannot take go
-        // to the full kernel, and from there (too long for the packed word) to the unpacked one
-        for (size_t i = 0; i < ad.size(); ++i) job.adapter_code[i] = (uint8_t)dp_code((uint8_t)ad[i]);
-        uint32_t *c32 = ln.d_c32.as<uint32_t>();
-        uint32_t *fb = is_prefix ? ln.d_fb_a.as<uint32_t>() : ln.d_fb_b.as<uint32_t>();
-        uint32_t *nfb = c32 + (is_prefix ? C_FBPRE : C_FBSUF);
-        uint32_t *fb2 = ln.d_fb2.as<uint32_t>();
-        uint32_t *nfb2 = c32 + (is_prefix ? C_FB2PRE : C_FB2SUF);
-        const DpLayout &lay = is_prefix ? c->lay_pre : c->lay_suf;
-        const uint32_t lcap = is_prefix ? c->lcap_pre : c->lcap_suf;
-        if ((rc = launch_dp_windowed(job, lay, K, lcap, n_batch, ln.d_wins.p, c32 + (is_prefix ? C_NWINPRE : C_NWINSUF),
+    job.is_prefix = s == PRE;
+    job.min_accept = side.min_accept;
+    job.adapter_len = (uint32_t)side.seq.size();
+    if (side.packed)
+        for (size_t i = 0; i < side.seq.size(); ++i) job.adapter_code[i] = (uint8_t)dp_code((uint8_t)side.seq[i]);
+    DpJob rest = job;                   // the reads the next stage of the chain takes
+    uint32_t *fb = ln.d_fb[s].as<uint32_t>(), *nfb = c32 + C_FBPRE + s;
+    if (side.win_k >= 0) {
+        if ((rc = launch_dp_windowed(job, side.lay, side.win_k, side.lcap, n_batch, ln.d_wins.p, c32 + C_NWINPRE + s,
                                      ln.win_cap, ln.d_bestkey.as<unsigned long long>(), ln.d_cbval.as<unsigned long long>(),
-                                     fb, nfb, ln.d_t64.as<unsigned long long>() + T_CELLSCOMP, c32 + (is_prefix ? C_WORKPRE : C_WORKSUF) /* the window cursor sits 32 words on */,
-                                     c->sm_count, st,
-                                     pev ? pev[is_prefix ? 8 : 10] : nullptr, pev ? pev[is_prefix ? 9 : 11] : nullptr)))
+                                     fb, nfb, ln.d_t64.as<unsigned long long>() + T_CELLSCOMP,
+                                     c32 + C_WORKPRE + 64 * s /* the window cursor sits 32 words on */, c->sm_count, st,
+                                     pev ? pev[8 + 2 * s] : nullptr, pev ? pev[9 + 2 * s] : nullptr)))
             return rc;
-        DpJob fj = job;
-        fj.worklist = fb;
-        fj.n_items = nfb;
-        if ((rc = launch_dp_packed_ex(fj, lay, lcap, fb2, nfb2, c->sm_count, st))) return rc;
-        gj.base = fj;
-        gj.base.worklist = fb2;
-        gj.base.n_items = nfb2;
-        if ((rc = launch_dp_generic(gj, c->sm_count, st))) return rc;
-        c->stats.dp_kernel_launches += 5;
-    } else if (packed) {
-        for (size_t i = 0; i < ad.size(); ++i) job.adapter_code[i] = (uint8_t)dp_code((uint8_t)ad[i]);
-        uint32_t *fb = is_prefix ? ln.d_fb_a.as<uint32_t>() : ln.d_fb_b.as<uint32_t>();
-        uint32_t *nfb = ln.d_c32.as<uint32_t>() + (is_prefix ? C_FBPRE : C_FBSUF);
-        if ((rc = launch_dp_packed_ex(job, is_prefix ? c->lay_pre : c->lay_suf,
-                                      is_prefix ? c->lcap_pre : c->lcap_suf, fb, nfb, c->sm_count, st)))
-            return rc;
-        // reads too long for the packed word (normally none): same rule set, unpacked
-        gj.base = job;
-        gj.base.worklist = fb;
-        gj.base.n_items = nfb;
-        gj.base.cells = job.cells;
-        if ((rc = launch_dp_generic(gj, c->sm_count, st))) return rc;
-        c->stats.dp_kernel_launches += 2;
-    } else {
-        gj.base = job;
-        if ((rc = launch_dp_generic(gj, c->sm_count, st))) return rc;
+        rest.worklist = fb;
+        rest.n_items = nfb;
+        fb = ln.d_fb2.as<uint32_t>();
+        nfb = c32 + C_FB2PRE + s;
+        c->stats.dp_kernel_launches += 3;
+    }
+    if (side.packed) {
+        if ((rc = launch_dp_packed_ex(rest, side.lay, side.lcap, fb, nfb, c->sm_count, st))) return rc;
+        rest.worklist = fb;
+        rest.n_items = nfb;
         c->stats.dp_kernel_launches += 1;
     }
+    DpGenericJob gj;
+    gj.base = rest;
+    gj.d_adapter_code = side.d_code.as<uint8_t>();
+    gj.sc = c->sc;
+    gj.scratch = c->d_generic_scratch.as<int32_t>();
+    gj.n_threads = c->generic_threads;
+    if ((rc = launch_dp_generic(gj, c->sm_count, st))) return rc;
+    c->stats.dp_kernel_launches += 1;
     return VFB_OK;
 }
 
@@ -885,21 +856,19 @@ static int queue_scan_dp(vfb_ctx *c, Lane &ln, cudaStream_t st, cudaStream_t sd,
     ScanJob sj;
     memset(&sj, 0, sizeof sj);
     sj.text = ps.text; sj.spans = ps.spans; sj.n_reads = n; sj.text_bytes = text_bytes_hint;
-    sj.start = ps.start; sj.end = ps.end;
-    if (c->align_pre) { sj.list_pre = ln.d_list_a.as<uint32_t>(); sj.n_pre = ln.d_c32.as<uint32_t>() + C_NPRE; }
-    if (c->align_suf) { sj.list_suf = ln.d_list_b.as<uint32_t>(); sj.n_suf = ln.d_c32.as<uint32_t>() + C_NSUF; }
+    sj.start = ps.bound[PRE]; sj.end = ps.bound[SUF];
+    if (c->side[PRE].align) { sj.list_pre = ln.d_list[PRE].as<uint32_t>(); sj.n_pre = ln.d_c32.as<uint32_t>() + C_NPRE; }
+    if (c->side[SUF].align) { sj.list_suf = ln.d_list[SUF].as<uint32_t>(); sj.n_suf = ln.d_c32.as<uint32_t>() + C_NSUF; }
     sj.compute_all = (c->prm.dp_compute_all || diag) ? 1 : 0;
     sj.force_general = c->prm.force_general_scan;
-    if ((rc = launch_scan(sj, c->ad_pre, c->ad_suf, c->sm_count, st))) return rc;
+    if ((rc = launch_scan(sj, c->side[PRE].ad, c->side[SUF].ad, c->sm_count, st))) return rc;
     if (prof) VFB_CUDA(cudaEventRecord(pev[1], st));
     if (diag) {
-        VFB_CUDA(cudaMemcpyAsync(ps.diag[0], ps.start, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
-        VFB_CUDA(cudaMemcpyAsync(ps.diag[1], ps.end, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+        for (int s = 0; s < 2; ++s)
+            VFB_CUDA(cudaMemcpyAsync(ps.diag->exact[s].p, ps.bound[s], (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
         // "no DP ran" markers: score = INT32_MIN (0x80000000), len = -1
-        VFB_CUDA(cudaMemsetAsync(ps.diag[3], 0xFF, (size_t)n * 4, st));
-        VFB_CUDA(cudaMemsetAsync(ps.diag[5], 0xFF, (size_t)n * 4, st));
-        VFB_CUDA(cudaMemsetAsync(ps.diag[2], 0, (size_t)n * 4, st));
-        VFB_CUDA(cudaMemsetAsync(ps.diag[4], 0, (size_t)n * 4, st));
+        for (int s = 0; s < 2; ++s) VFB_CUDA(cudaMemsetAsync(ps.diag->len[s].p, 0xFF, (size_t)n * 4, st));
+        for (int s = 0; s < 2; ++s) VFB_CUDA(cudaMemsetAsync(ps.diag->score[s].p, 0, (size_t)n * 4, st));
     }
     // DP.  The prefix pass runs first: reads it rejects need no suffix alignment (no region
     // either way, src/lib.rs:288), reads it accepts join the suffix worklist if they need one.
@@ -909,12 +878,11 @@ static int queue_scan_dp(vfb_ctx *c, Lane &ln, cudaStream_t st, cudaStream_t sd,
         VFB_CUDA(cudaEventRecord(ln.ev_scanned, st));
         VFB_CUDA(cudaStreamWaitEvent(sd, ln.ev_scanned, 0));
     }
-    if (prof) VFB_CUDA(cudaEventRecord(pev[2], st));
-    if (c->align_pre) if ((rc = run_dp(c, ln, sd, ps, true, n, pev))) return rc;
-    if (prof) VFB_CUDA(cudaEventRecord(pev[3], st));
-    if (prof) VFB_CUDA(cudaEventRecord(pev[4], st));
-    if (c->align_suf) if ((rc = run_dp(c, ln, sd, ps, false, n, pev))) return rc;
-    if (prof) VFB_CUDA(cudaEventRecord(pev[5], st));
+    for (int s = 0; s < 2; ++s) {
+        if (prof) VFB_CUDA(cudaEventRecord(pev[2 + 2 * s], st));
+        if (c->side[s].align) if ((rc = run_dp(c, ln, sd, ps, s, n, pev))) return rc;
+        if (prof) VFB_CUDA(cudaEventRecord(pev[3 + 2 * s], st));
+    }
     k_accumulate<<<1, 1, 0, sd>>>(ln.d_t64.as<unsigned long long>(), ln.d_c32.as<uint32_t>(), ln.win_cap);
     ++g_launches;
     if (split) {
@@ -933,13 +901,13 @@ static int queue_keys_count(vfb_ctx *c, Lane &ln, cudaStream_t st, const Pass &p
     int rc;
     KeyJob kj;
     kj.text = ps.text; kj.spans = ps.spans;
-    kj.start = ps.start; kj.end = ps.end;
+    kj.start = ps.bound[PRE]; kj.end = ps.bound[SUF];
     kj.n_reads = n; kj.text_bytes = text_bytes_hint; kj.skip_translation = c->prm.skip_translation;
     kj.keys = ln.d_keys.as<uint8_t>(); kj.koff = ln.d_koff.as<uint64_t>();
     kj.key_cursor = ln.d_t64.as<unsigned long long>() + T_KEYBYTES;
     kj.klen = ln.d_klen.as<uint32_t>(); kj.khash = ln.d_khash.as<uint64_t>();
     kj.hash_bits = c->prm.debug_hash_bits;
-    kj.flank_bytes = (uint32_t)(c->prefix.size() + c->suffix.size());
+    kj.flank_bytes = (uint32_t)(c->side[PRE].seq.size() + c->side[SUF].seq.size());
     // the table work of a batch claims slots by batch-relative index, and the fused key kernel reads slots without
     // fences: one batch at a time from here on
     bool k4_waited = false;
@@ -993,8 +961,8 @@ static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_sp
     // scratch
     if ((rc = ln.d_start.ensure((size_t)n * 4))) return rc;
     if ((rc = ln.d_end.ensure((size_t)n * 4))) return rc;
-    if (c->align_pre) { if ((rc = ln.d_list_a.ensure((size_t)n * 4))) return rc; if ((rc = ln.d_fb_a.ensure((size_t)n * 4))) return rc; }
-    if (c->align_suf) { if ((rc = ln.d_list_b.ensure((size_t)n * 4))) return rc; if ((rc = ln.d_fb_b.ensure((size_t)n * 4))) return rc; }
+    for (int s = 0; s < 2; ++s)
+        if (c->side[s].align) { if ((rc = ln.d_list[s].ensure((size_t)n * 4))) return rc; if ((rc = ln.d_fb[s].ensure((size_t)n * 4))) return rc; }
     // keys: sum of padded key lengths <= bytes/(3|1) + 16 per read
     const uint64_t key_bytes_ub = (c->prm.skip_translation ? span_bytes_upper : span_bytes_upper / 3) + 16ull * n;
     if ((rc = ln.d_keys.ensure(key_bytes_ub))) return rc;
@@ -1002,7 +970,7 @@ static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_sp
     if ((rc = ln.d_klen.ensure((size_t)n * 4))) return rc;
     if ((rc = ln.d_khash.ensure((size_t)n * 8))) return rc;
     if ((rc = ln.d_owner.ensure((size_t)n * 4))) return rc;
-    if (c->win_k_pre >= 0 || c->win_k_suf >= 0) {
+    if (c->side[PRE].win_k >= 0 || c->side[SUF].win_k >= 0) {
         const uint32_t cap = n < 0x3FFFFFFFu ? n * 2u + 1024u : 0x7FFFFFFFu;
         if ((rc = ln.d_wins.ensure((size_t)cap * dpw_item_bytes()))) return rc;
         ln.win_cap = (uint32_t)(ln.d_wins.cap / dpw_item_bytes());
@@ -1012,14 +980,8 @@ static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_sp
         if ((rc = ln.d_fb2.ensure((size_t)n * 4))) return rc;
     }
     const bool diag = c->prm.diagnostics != 0;
-    if (diag) {
-        DevBuf *db[] = {&c->d_diag_exact_pre, &c->d_diag_exact_suf, &c->d_diag_score_pre, &c->d_diag_len_pre,
-                        &c->d_diag_score_suf, &c->d_diag_len_suf};
-        for (auto *b : db) if ((rc = b->ensure((size_t)n * 4))) return rc;
-    }
-    Pass fwd{d_text, d_spans, ln.d_start.as<uint32_t>(), ln.d_end.as<uint32_t>(),
-             {c->d_diag_exact_pre.as<int32_t>(), c->d_diag_exact_suf.as<int32_t>(), c->d_diag_score_pre.as<int32_t>(),
-              c->d_diag_len_pre.as<int32_t>(), c->d_diag_score_suf.as<int32_t>(), c->d_diag_len_suf.as<int32_t>()}};
+    if (diag && (rc = c->diag_fwd.ensure((size_t)n * 4))) return rc;
+    Pass fwd{d_text, d_spans, {ln.d_start.as<uint32_t>(), ln.d_end.as<uint32_t>()}, diag ? &c->diag_fwd : nullptr};
     Pass rev{};
     if (both) {
         // the gathered text sits 16 bytes into its buffer and is followed by 16 more: the kernels load aligned 16-byte
@@ -1029,14 +991,9 @@ static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_sp
         if ((rc = ln.d_rsrc.ensure((size_t)n * 4))) return rc;
         if ((rc = ln.d_rstart.ensure((size_t)n * 4))) return rc;
         if ((rc = ln.d_rend.ensure((size_t)n * 4))) return rc;
-        if (diag) {
-            DevBuf *db[] = {&c->d_rdiag_exact_pre, &c->d_rdiag_exact_suf, &c->d_rdiag_score_pre, &c->d_rdiag_len_pre,
-                            &c->d_rdiag_score_suf, &c->d_rdiag_len_suf};
-            for (auto *b : db) if ((rc = b->ensure((size_t)n * 4))) return rc;
-        }
-        rev = Pass{ln.d_rtext.as<uint8_t>() + 16, ln.d_rspans.as<vfb_span>(), ln.d_rstart.as<uint32_t>(), ln.d_rend.as<uint32_t>(),
-                   {c->d_rdiag_exact_pre.as<int32_t>(), c->d_rdiag_exact_suf.as<int32_t>(), c->d_rdiag_score_pre.as<int32_t>(),
-                    c->d_rdiag_len_pre.as<int32_t>(), c->d_rdiag_score_suf.as<int32_t>(), c->d_rdiag_len_suf.as<int32_t>()}};
+        if (diag && (rc = c->diag_rev.ensure((size_t)n * 4))) return rc;
+        rev = Pass{ln.d_rtext.as<uint8_t>() + 16, ln.d_rspans.as<vfb_span>(), {ln.d_rstart.as<uint32_t>(), ln.d_rend.as<uint32_t>()},
+                   diag ? &c->diag_rev : nullptr};
     }
     if ((rc = table_reserve(c, n, key_bytes_ub, true))) return rc;
     cudaEvent_t *pev = nullptr, *pev_rev = nullptr;
@@ -1059,7 +1016,7 @@ static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_sp
     if (both) {
         VFB_CUDA(cudaMemsetAsync(ln.d_rspans.p, 0, (size_t)n * 8, st));
         VFB_CUDA(cudaMemsetAsync(t64 + T_GATHER, 0, 8, st));
-        StrandJob sj{d_spans, fwd.start, fwd.end, n, d_text, ln.d_rtext.as<uint8_t>() + 16, ln.d_rspans.as<vfb_span>(),
+        StrandJob sj{d_spans, fwd.bound[PRE], fwd.bound[SUF], n, d_text, ln.d_rtext.as<uint8_t>() + 16, ln.d_rspans.as<vfb_span>(),
                      ln.d_rsrc.as<uint32_t>(), t64 + T_GATHER, t64 + T_REVREADS};
         if ((rc = launch_strand_gather(sj, c->sm_count, st))) return rc;
     }
@@ -1595,9 +1552,35 @@ int vfb_get_stats(vfb_ctx *c, vfb_stats *out)
 
 }  // extern "C"
 
-static int diag_rows(vfb_ctx *c, const std::vector<uint32_t> &ep, const std::vector<uint32_t> &es, const std::vector<int32_t> &sp,
-                     const std::vector<int32_t> &lp, const std::vector<int32_t> &ss, const std::vector<int32_t> &ls,
-                     const std::vector<uint32_t> &st, const std::vector<uint32_t> &en, vfb_read_diag *out, size_t n);
+// The first n rows of a pass's diagnostics columns and boundaries (device) -> vfb_read_diag rows (host).
+static int diag_fetch(vfb_ctx *c, const DiagBufs &d, const DevBuf &start, const DevBuf &end, size_t n, vfb_read_diag *out)
+{
+    if (!n) return VFB_OK;
+    std::vector<uint32_t> ep(n), es(n), st(n), en(n);
+    std::vector<int32_t> sp(n), lp(n), ss(n), ls(n);
+    VFB_CUDA(cudaMemcpy(ep.data(), d.exact[PRE].p, n * 4, cudaMemcpyDeviceToHost));
+    VFB_CUDA(cudaMemcpy(es.data(), d.exact[SUF].p, n * 4, cudaMemcpyDeviceToHost));
+    VFB_CUDA(cudaMemcpy(st.data(), start.p, n * 4, cudaMemcpyDeviceToHost));
+    VFB_CUDA(cudaMemcpy(en.data(), end.p, n * 4, cudaMemcpyDeviceToHost));
+    VFB_CUDA(cudaMemcpy(sp.data(), d.score[PRE].p, n * 4, cudaMemcpyDeviceToHost));
+    VFB_CUDA(cudaMemcpy(lp.data(), d.len[PRE].p, n * 4, cudaMemcpyDeviceToHost));
+    VFB_CUDA(cudaMemcpy(ss.data(), d.score[SUF].p, n * 4, cudaMemcpyDeviceToHost));
+    VFB_CUDA(cudaMemcpy(ls.data(), d.len[SUF].p, n * 4, cudaMemcpyDeviceToHost));
+    const uint32_t A = (uint32_t)c->side[PRE].seq.size();
+    for (size_t i = 0; i < n; ++i) {
+        vfb_read_diag r;
+        r.exact_prefix = ep[i] == VFB_NONE ? -1 : (int32_t)(ep[i] - A);
+        r.exact_suffix = es[i] == VFB_NONE ? -1 : (int32_t)es[i];
+        r.score_prefix = lp[i] < 0 ? INT32_MIN : sp[i];
+        r.len_prefix = lp[i];
+        r.score_suffix = ls[i] < 0 ? INT32_MIN : ss[i];
+        r.len_suffix = ls[i];
+        r.start = st[i] == VFB_NONE ? -1 : (int32_t)st[i];
+        r.end = en[i] == VFB_NONE ? -1 : (int32_t)en[i];
+        out[i] = r;
+    }
+    return VFB_OK;
+}
 
 extern "C" {
 
@@ -1609,18 +1592,9 @@ int vfb_get_diag(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
     int rc = vfb_sync(c);
     if (rc) return rc;
     const size_t n = (size_t)n_reads;
-    std::vector<uint32_t> ep(n), es(n), st(n), en(n);
-    std::vector<int32_t> sp(n), lp(n), ss(n), ls(n);
-    VFB_CUDA(cudaMemcpy(ep.data(), c->d_diag_exact_pre.p, n * 4, cudaMemcpyDeviceToHost));
-    VFB_CUDA(cudaMemcpy(es.data(), c->d_diag_exact_suf.p, n * 4, cudaMemcpyDeviceToHost));
-    VFB_CUDA(cudaMemcpy(st.data(), c->lanes[0].d_start.p, n * 4, cudaMemcpyDeviceToHost));
-    VFB_CUDA(cudaMemcpy(en.data(), c->lanes[0].d_end.p, n * 4, cudaMemcpyDeviceToHost));
-    VFB_CUDA(cudaMemcpy(sp.data(), c->d_diag_score_pre.p, n * 4, cudaMemcpyDeviceToHost));
-    VFB_CUDA(cudaMemcpy(lp.data(), c->d_diag_len_pre.p, n * 4, cudaMemcpyDeviceToHost));
-    VFB_CUDA(cudaMemcpy(ss.data(), c->d_diag_score_suf.p, n * 4, cudaMemcpyDeviceToHost));
-    VFB_CUDA(cudaMemcpy(ls.data(), c->d_diag_len_suf.p, n * 4, cudaMemcpyDeviceToHost));
+    if ((rc = diag_fetch(c, c->diag_fwd, c->lanes[0].d_start, c->lanes[0].d_end, n, out))) return rc;
     c->stats.d2h_bytes += n * 32;
-    return diag_rows(c, ep, es, sp, lp, ss, ls, st, en, out, n);
+    return VFB_OK;
 }
 
 int vfb_get_diag_reverse(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
@@ -1635,24 +1609,13 @@ int vfb_get_diag_reverse(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
     unsigned long long cursor = 0;
     VFB_CUDA(cudaMemcpy(&cursor, c->lanes[0].d_t64.as<unsigned long long>() + T_GATHER, 8, cudaMemcpyDeviceToHost));
     const size_t m = (size_t)(cursor >> 32);            // gathered reads, in compact order
-    std::vector<uint32_t> ep(m), es(m), st(m), en(m), src(m);
-    std::vector<int32_t> sp(m), lp(m), ss(m), ls(m);
-    if (m) {
-        VFB_CUDA(cudaMemcpy(ep.data(), c->d_rdiag_exact_pre.p, m * 4, cudaMemcpyDeviceToHost));
-        VFB_CUDA(cudaMemcpy(es.data(), c->d_rdiag_exact_suf.p, m * 4, cudaMemcpyDeviceToHost));
-        VFB_CUDA(cudaMemcpy(st.data(), c->lanes[0].d_rstart.p, m * 4, cudaMemcpyDeviceToHost));
-        VFB_CUDA(cudaMemcpy(en.data(), c->lanes[0].d_rend.p, m * 4, cudaMemcpyDeviceToHost));
-        VFB_CUDA(cudaMemcpy(sp.data(), c->d_rdiag_score_pre.p, m * 4, cudaMemcpyDeviceToHost));
-        VFB_CUDA(cudaMemcpy(lp.data(), c->d_rdiag_len_pre.p, m * 4, cudaMemcpyDeviceToHost));
-        VFB_CUDA(cudaMemcpy(ss.data(), c->d_rdiag_score_suf.p, m * 4, cudaMemcpyDeviceToHost));
-        VFB_CUDA(cudaMemcpy(ls.data(), c->d_rdiag_len_suf.p, m * 4, cudaMemcpyDeviceToHost));
-        VFB_CUDA(cudaMemcpy(src.data(), c->lanes[0].d_rsrc.p, m * 4, cudaMemcpyDeviceToHost));
-    }
+    std::vector<vfb_read_diag> rows(m);
+    std::vector<uint32_t> src(m);
+    if ((rc = diag_fetch(c, c->diag_rev, c->lanes[0].d_rstart, c->lanes[0].d_rend, m, rows.data()))) return rc;
+    if (m) VFB_CUDA(cudaMemcpy(src.data(), c->lanes[0].d_rsrc.p, m * 4, cudaMemcpyDeviceToHost));
     c->stats.d2h_bytes += 8 + m * 36;
     const vfb_read_diag absent = {-1, -1, INT32_MIN, -1, INT32_MIN, -1, -1, -1};
     for (size_t i = 0; i < n; ++i) out[i] = absent;
-    std::vector<vfb_read_diag> rows(m);
-    diag_rows(c, ep, es, sp, lp, ss, ls, st, en, rows.data(), m);
     for (size_t i = 0; i < m; ++i) {
         if (src[i] >= n) { set_error("reverse diagnostics: read index out of range"); return VFB_ERR_CUDA; }
         out[src[i]] = rows[i];
@@ -1661,27 +1624,6 @@ int vfb_get_diag_reverse(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
 }
 
 }  // extern "C"
-
-// Device boundaries and diagnostics columns -> vfb_read_diag rows.
-static int diag_rows(vfb_ctx *c, const std::vector<uint32_t> &ep, const std::vector<uint32_t> &es, const std::vector<int32_t> &sp,
-                     const std::vector<int32_t> &lp, const std::vector<int32_t> &ss, const std::vector<int32_t> &ls,
-                     const std::vector<uint32_t> &st, const std::vector<uint32_t> &en, vfb_read_diag *out, size_t n)
-{
-    const uint32_t A = (uint32_t)c->prefix.size();
-    for (size_t i = 0; i < n; ++i) {
-        vfb_read_diag d;
-        d.exact_prefix = ep[i] == VFB_NONE ? -1 : (int32_t)(ep[i] - A);
-        d.exact_suffix = es[i] == VFB_NONE ? -1 : (int32_t)es[i];
-        d.score_prefix = lp[i] < 0 ? INT32_MIN : sp[i];
-        d.len_prefix = lp[i];
-        d.score_suffix = ls[i] < 0 ? INT32_MIN : ss[i];
-        d.len_suffix = ls[i];
-        d.start = st[i] == VFB_NONE ? -1 : (int32_t)st[i];
-        d.end = en[i] == VFB_NONE ? -1 : (int32_t)en[i];
-        out[i] = d;
-    }
-    return VFB_OK;
-}
 
 // Export, pass 1: slot counts -> row counts, sizes of what will be exported (rows with a non-zero count).
 int vfb_internal_export_sizes(vfb_ctx *c, uint64_t *rows_out, uint64_t *bytes_out)

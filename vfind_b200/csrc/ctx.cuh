@@ -53,6 +53,39 @@ struct DevBuf {
     template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
 
+// The adapter sides, indexes of vfb_ctx::side and of the per-side arrays below.
+enum { PRE = 0, SUF = 1 };
+
+// What vfb_create decides for one adapter.  win_k >= 0 <=> this side runs the windowed DP (filter -> windows ->
+// resolve), and then `packed` is set too; plan_packed_dp is the one place that decides it.
+struct AdapterSide {
+    std::string seq;
+    AdapterBytes ad;
+    bool align = false;                 // the threshold is below 1: reads without an exact match are aligned
+    int min_accept = 0;
+    bool packed = false;                // the packed kernels run on `lay` (else only the unpacked one)
+    DpLayout lay;
+    uint32_t lcap = 0;
+    int win_k = -1;                     // Myers threshold of the windowed DP
+    DevBuf d_code;                      // adapter codes for the unpacked kernel
+};
+
+// The per-read diagnostics columns of one pass, by adapter side.
+struct DiagBufs {
+    DevBuf exact[2], score[2], len[2];
+    int ensure(size_t bytes)
+    {
+        for (int s = 0; s < 2; ++s)
+            for (DevBuf *b : {&exact[s], &score[s], &len[s]})
+                if (int rc = b->ensure(bytes)) return rc;
+        return VFB_OK;
+    }
+    void release()
+    {
+        for (int s = 0; s < 2; ++s) { exact[s].release(); score[s].release(); len[s].release(); }
+    }
+};
+
 struct PinBuf {
     void *p = nullptr;
     size_t cap = 0;
@@ -86,7 +119,8 @@ struct Lane {
     cudaEvent_t ev_scanned = nullptr, ev_aligned = nullptr;
     cudaEvent_t done = nullptr;         // the lane's last batch has finished
     bool pending = false;               // `done` has not been joined into the compute stream yet
-    DevBuf d_start, d_end, d_list_a, d_list_b, d_fb_a, d_fb_b, d_c32, d_t64;
+    DevBuf d_start, d_end, d_c32, d_t64;
+    DevBuf d_list[2], d_fb[2];          // per side: DP worklist, reads for the next kernel of the fallback chain
     DevBuf d_keys, d_koff, d_klen, d_khash, d_owner;
     DevBuf d_wins, d_bestkey, d_cbval, d_fb2;   // windowed DP: window items, per-item results, second fallback list
     // both_strands: the reverse pass's text (reverse complements, padded), compact spans, original read indices and
@@ -129,16 +163,9 @@ enum { T_CELLS = 0, T_DPPRE, T_DPSUF, T_KEYBYTES, T_CELLSCOMP, T_WINDOWS, T_GATH
 }  // namespace vfb
 
 struct vfb_ctx {
-    vfb_params prm;
-    std::string prefix, suffix;
-    vfb::AdapterBytes ad_pre, ad_suf;
+    vfb_params prm;                       // prm.prefix / prm.suffix point into side[].seq
+    vfb::AdapterSide side[2];
     vfb::DpScoring sc;
-    bool align_pre = false, align_suf = false;
-    int min_accept_pre = 0, min_accept_suf = 0;
-    bool packed_pre = false, packed_suf = false;
-    vfb::DpLayout lay_pre, lay_suf;
-    uint32_t lcap_pre = 0, lcap_suf = 0;
-    vfb::DevBuf d_code_pre, d_code_suf;   // adapter codes for the fallback kernel
     vfb::DevBuf d_generic_scratch;
     uint32_t generic_threads = 0;
 
@@ -158,12 +185,10 @@ struct vfb_ctx {
     uint64_t lane_seq = 0;
     cudaEvent_t ev_fork = nullptr, ev_k4 = nullptr;   // compute stream -> lane; the previous batch's insert is done
     bool k4_pending = false;
-    int win_k_pre = -1, win_k_suf = -1;         // Myers thresholds (-1: the windowed DP does not apply)
     vfb::DevBuf d_aligned_text;     // aligned copy of an unaligned caller buffer (vfb_submit_device)
     vfb::DevBuf d_span_sum;         // vfb_submit_device: sum of the span lengths of a batch
-    vfb::DevBuf d_diag_exact_pre, d_diag_exact_suf, d_diag_score_pre, d_diag_len_pre, d_diag_score_suf, d_diag_len_suf;
-    // both_strands + diagnostics: the reverse pass's diagnostics, in compact (gathered) order
-    vfb::DevBuf d_rdiag_exact_pre, d_rdiag_exact_suf, d_rdiag_score_pre, d_rdiag_len_pre, d_rdiag_score_suf, d_rdiag_len_suf;
+    // diagnostics of the forward pass and (both_strands) of the reverse pass, the latter in compact (gathered) order
+    vfb::DiagBufs diag_fwd, diag_rev;
     uint64_t diag_n = 0;
     bool diag_valid = false;
 
