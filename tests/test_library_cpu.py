@@ -120,8 +120,8 @@ def test_synth_host_is_deterministic_and_shaped(lib):
 
 
 def test_hash_reference_properties(lib):
-    # the device hash is order sensitive and length sensitive (host twin in hash.h is
-    # exercised through the chunk tests on the GPU); here: chunk header rejects garbage
+    # the host twin of the device hash (hash.h) is restated in test_keys_cpu.py and compared with
+    # every hash the device stores in test_gpu_keys.py; here: chunk header rejects garbage
     from vfind_b200 import api
     rows = ctypes.c_uint64(0)
     buf = np.zeros(64, dtype=np.uint8)

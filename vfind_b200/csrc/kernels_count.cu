@@ -1348,7 +1348,9 @@ int launch_partition_count(const DevTable &t, uint64_t rows, uint32_t n_parts,
     return VFB_OK;
 }
 
-// Chunk headers are written by the kernel too (block 0), from the part sizes the count pass left on the device.
+// Chunk headers are written by the kernel too (block 0), from the part sizes the count pass left on the device.  An
+// export of the whole table (self >= n_parts, vfb_table_partition_fill) gives every part a chunk, an empty one a
+// header of zero rows; a keep-own merge sends no chunk for an empty part, and its offset is the next part's.
 __global__ void __launch_bounds__(256)
 k5_partition_fill(const DevTable t, uint64_t rows, uint32_t n_parts, uint32_t self, bool release,
                   uint8_t *buf, const uint64_t *chunk_off,
@@ -1357,7 +1359,7 @@ k5_partition_fill(const DevTable t, uint64_t rows, uint32_t n_parts, uint32_t se
 {
     if (blockIdx.x == 0)
         for (uint32_t p = threadIdx.x; p < n_parts; p += blockDim.x)
-            if (p != self && part_rows[p]) {
+            if (p != self && (part_rows[p] || self >= n_parts)) {
                 ChunkHeader *hd = reinterpret_cast<ChunkHeader *>(buf + chunk_off[p]);
                 hd->magic = VFB_CHUNK_MAGIC; hd->rows = part_rows[p]; hd->key_bytes = part_keybytes[p]; hd->reserved = 0;
             }
