@@ -2,8 +2,8 @@
 // Kernels and the scheme: kernels_inflate.cu ("Single-stream gzip on the device").  Replaces flate2's MultiGzDecoder
 // (/root/reference/src/lib.rs:233) for the FIRST member of a plain gzip file; whatever the device cannot take — further
 // members, a chunk that runs out of room, a stream without usable block starts — is inflated by zlib from the exact bit
-// where the device stopped (raw inflate primed with the bits of the first byte and the 32 KiB window as dictionary), so
-// every valid gzip file decodes to the same bytes either way.  CRC-32 and ISIZE are checked as flate2 does.
+// where the device stopped (raw inflate primed with the bits of the first byte and the text before it, up to 32 KiB, as
+// dictionary), so every valid gzip file decodes to the same bytes either way.  CRC-32 and ISIZE are checked as flate2 does.
 #include "gunzip_gpu.h"
 
 #include <unistd.h>
@@ -46,8 +46,8 @@ struct GpuGunzip::Impl {
     // where the deflate stream continues: file byte offset and bit inside that byte
     uint64_t byte_pos = 0;
     uint32_t bit_in_byte = 0;
-    bool window_known = false;               // false only before the stream's first byte
-    std::vector<uint8_t> window;             // the 32 KiB of text before byte_pos/bit_in_byte
+    uint32_t hist = 0;                       // bytes of text before byte_pos/bit_in_byte, at most VFB_GZ_WIN
+    std::vector<uint8_t> window;             // the 32 KiB before byte_pos/bit_in_byte: the last `hist` bytes are text
     uint32_t crc = 0;                        // of the member's text so far
     uint64_t text_total = 0;
     // parameters
@@ -317,7 +317,7 @@ struct GpuGunzip::Impl {
             if (slot.d_text.ensure(total + 64) || d_nl.ensure(np * 4) || d_crc.ensure(nc * 4)) { *err = "out of device memory for the gzip decoder"; return false; }
             if (launch_gz_resolve(d_live.as<uint32_t>(), d_text_off.as<unsigned long long>(), co.n_live, total, d_out16.as<uint16_t>(),
                                   cap_syms, d_win_store.as<uint8_t>(), slot.d_text.as<uint8_t>(), d_nl.as<uint32_t>(), d_crc.as<uint32_t>(),
-                                  window_known ? 1 : 0, d_flags.as<uint32_t>(), st)) { *err = vfb_last_error(); return false; }
+                                  hist, d_flags.as<uint32_t>(), st)) { *err = vfb_last_error(); return false; }
             slot.nl.resize(np);
             piece_crc.resize(nc);
             uint32_t flag = 0;
@@ -335,7 +335,7 @@ struct GpuGunzip::Impl {
             }
             text_total += total;
             window.assign(h_win, h_win + VFB_GZ_WIN);
-            window_known = true;
+            hist = (uint32_t)std::min<uint64_t>((uint64_t)hist + total, VFB_GZ_WIN);
         }
         slot.text = total;
         t_resolve = ms();
@@ -380,13 +380,14 @@ struct GpuGunzip::Impl {
         return true;
     }
 
-    // zlib from (byte_pos, bit_in_byte) with `window` as dictionary
+    // zlib from (byte_pos, bit_in_byte) with the text in `window` as dictionary (so that zlib, too, rejects a distance
+    // that reaches before the stream's first byte)
     bool start_host(std::string *err)
     {
         memset(&zs, 0, sizeof zs);
         if (inflateInit2(&zs, -15) != Z_OK) { *err = "zlib init failed"; mode = FAILED; return false; }
         zs_open = true;
-        if (window_known && inflateSetDictionary(&zs, window.data(), VFB_GZ_WIN) != Z_OK) { *err = "zlib dictionary failed"; mode = FAILED; return false; }
+        if (hist && inflateSetDictionary(&zs, window.data() + (VFB_GZ_WIN - hist), hist) != Z_OK) { *err = "zlib dictionary failed"; mode = FAILED; return false; }
         zin.resize(1 << 20);
         uint64_t off = byte_pos;
         if (bit_in_byte) {
@@ -445,7 +446,7 @@ struct GpuGunzip::Impl {
                 if (inflateGetDictionary(&zs, dict.data(), &dl) != Z_OK) continue;
                 window.assign(VFB_GZ_WIN, 0);
                 memcpy(window.data() + (VFB_GZ_WIN - dl), dict.data(), dl);
-                window_known = true;
+                hist = dl;
                 if (unused) { byte_pos = next - 1; bit_in_byte = 8 - unused; }
                 else { byte_pos = next; bit_in_byte = 0; }
                 inflateEnd(&zs);

@@ -193,10 +193,11 @@ __device__ int infw_build(const InfTables *T, InfWarp *W, int nlen, int ndist, i
 {
     int e1 = 0, e2 = 0;
     if (lane == 0) {
+        // an incomplete code is accepted only as a single code of length 1 (zlib's inflate_table)
         e1 = canon_construct(W->lcount, W->lsym, W->lens, nlen);
-        if (!(e1 < 0 || (e1 > 0 && nlen - W->lcount[0] != 1))) e1 = 0; else e1 = 1;
+        if (!(e1 < 0 || (e1 > 0 && !(nlen - W->lcount[0] == 1 && W->lcount[1] == 1)))) e1 = 0; else e1 = 1;
         e2 = canon_construct(W->dcount, W->dsym, W->lens + nlen, ndist);
-        if (!(e2 < 0 || (e2 > 0 && ndist - W->dcount[0] != 1))) e2 = 0; else e2 = 1;
+        if (!(e2 < 0 || (e2 > 0 && !(ndist - W->dcount[0] == 1 && W->dcount[1] == 1)))) e2 = 0; else e2 = 1;
         if (fixed) e1 = e2 = 0;            // the fixed distance code leaves two codes unused (RFC 1951 3.2.6)
     }
     e1 = __shfl_sync(0xffffffffu, e1, 0);
@@ -1040,10 +1041,12 @@ k_gz_chain(const GzChunkRes *res, const uint32_t *starts, uint32_t n_chunks, con
 }
 
 // Pieces of GZ_PIECE bytes of text: symbols -> bytes (place holders through the chunk's window), newlines per piece.
+// hist0 = bytes of real text in front of the segment (at most GZ_WIN): a place holder p of visited chunk k stands for the
+// byte GZ_WIN - p before the chunk, which exists only when GZ_WIN - p <= hist0 + text_off[k].
 #define GZ_PIECE 65536u
 __global__ void __launch_bounds__(256)
 k_gz_resolve(const uint32_t *live, const unsigned long long *text_off, uint32_t n_live, const uint16_t *out16, uint32_t cap,
-             const uint8_t *win_store, uint8_t *text, uint32_t *piece_nl, int first_window_known, uint32_t *flag_unknown)
+             const uint8_t *win_store, uint8_t *text, uint32_t *piece_nl, uint32_t hist0, uint32_t *flag_unknown)
 {
     __shared__ uint32_t s_nl;
     const unsigned long long lo = (unsigned long long)blockIdx.x * GZ_PIECE;
@@ -1063,13 +1066,15 @@ k_gz_resolve(const uint32_t *live, const unsigned long long *text_off, uint32_t 
         const unsigned long long from = c_lo > lo ? c_lo : lo, to = c_hi < hi ? c_hi : hi;
         const uint16_t *sym = out16 + (size_t)live[k] * (GZ_WIN + (size_t)cap) + GZ_WIN;
         const uint8_t *win = win_store + (size_t)k * GZ_WIN;
+        const unsigned long long hist = hist0 + c_lo;
+        const uint32_t n_invalid = hist >= GZ_WIN ? 0u : GZ_WIN - (uint32_t)hist;    // place holders below this point before the stream
         for (unsigned long long q = from + threadIdx.x; q < to; q += blockDim.x) {
             const uint32_t s = sym[q - c_lo];
             uint8_t v;
             if (s < 256u) v = (uint8_t)s;
             else {
                 v = __ldg(win + ((s - 256u) & (GZ_WIN - 1u)));
-                if (k == 0 && !first_window_known) unknown = 1;    // the stream's first bytes refer to nothing
+                if (s - 256u < n_invalid) unknown = 1;
             }
             text[q] = v;
             nl += v == (uint8_t)'\n';
@@ -1160,12 +1165,12 @@ int launch_gz_chain(const void *d_res, const uint32_t *d_starts, uint32_t n_chun
 
 int launch_gz_resolve(const uint32_t *d_live, const unsigned long long *d_text_off, uint32_t n_live, unsigned long long total_text,
                       const uint16_t *d_out16, uint32_t cap, const uint8_t *d_win_store, uint8_t *d_text, uint32_t *d_piece_nl,
-                      uint32_t *d_piece_crc, int first_window_known, uint32_t *d_flag_unknown, cudaStream_t st)
+                      uint32_t *d_piece_crc, uint32_t hist, uint32_t *d_flag_unknown, cudaStream_t st)
 {
     if (total_text == 0) return VFB_OK;
     const uint32_t pieces = (uint32_t)((total_text + GZ_PIECE - 1) / GZ_PIECE);
     k_gz_resolve<<<pieces, 256, 0, st>>>(d_live, d_text_off, n_live, d_out16, cap, d_win_store, d_text, d_piece_nl,
-                                         first_window_known, d_flag_unknown);
+                                         hist, d_flag_unknown);
     const uint32_t cp = (uint32_t)((total_text + GZ_CRC_PIECE - 1) / GZ_CRC_PIECE);
     k_gz_crc<<<(cp + 127) / 128, 128, 0, st>>>(d_text, total_text, d_piece_crc);
     g_launches += 2;

@@ -205,10 +205,11 @@ bool read_dynamic(Bits &b, Tables &T)
         if (b.past_end()) return false;
     }
     if (lens[256] == 0) return false;
+    // an incomplete code is accepted only as a single code of length 1 (zlib's inflate_table)
     int e = construct(T.lh, lens, nlen);
-    if (e < 0 || (e > 0 && nlen - T.lh.count[0] != 1)) return false;
+    if (e < 0 || (e > 0 && !(nlen - T.lh.count[0] == 1 && T.lh.count[1] == 1))) return false;
     e = construct(T.dh, lens + nlen, ndist);
-    if (e < 0 || (e > 0 && ndist - T.dh.count[0] != 1)) return false;
+    if (e < 0 || (e > 0 && !(ndist - T.dh.count[0] == 1 && T.dh.count[1] == 1))) return false;
     T.build();
     return true;
 }

@@ -279,7 +279,7 @@ int launch_gz_chain(const void *d_res, const uint32_t *d_starts, uint32_t n_chun
                     uint8_t *d_win_store, uint8_t *d_out_window, void *d_out, cudaStream_t st);
 int launch_gz_resolve(const uint32_t *d_live, const unsigned long long *d_text_off, uint32_t n_live, unsigned long long total_text,
                       const uint16_t *d_out16, uint32_t cap, const uint8_t *d_win_store, uint8_t *d_text, uint32_t *d_piece_nl,
-                      uint32_t *d_piece_crc, int first_window_known, uint32_t *d_flag_unknown, cudaStream_t st);
+                      uint32_t *d_piece_crc, uint32_t hist, uint32_t *d_flag_unknown, cudaStream_t st);
 
 // ---------------------------------------------------------------- both_strands (kernels_strand.cu)
 // Reverse complements of the reads that have no forward region, gathered back to back into `out` (16-byte aligned
