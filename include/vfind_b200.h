@@ -77,6 +77,9 @@ typedef struct vfb_params {
     int32_t both_strands;             /* 1 = a read without a region (start, end located, start < end <= len) is
                                          searched once more as its reverse complement; a region found there is
                                          counted in the same table (at most one strand counts per read)       */
+    double collapse_ratio;            /* 0 = off; else (finite, >= 1) vfb_finish folds every key into a more abundant key of
+                                         the same length one byte substitution away, as vfb_collapse does, before the
+                                         table leaves the device (the count table itself keeps every key)               */
 } vfb_params;
 
 /* One read inside a text buffer: text[off .. off+len). */
@@ -242,6 +245,31 @@ int vfb_finish_arrow(vfb_ctx *ctx, vfb_arrow_array *out_array, vfb_arrow_schema 
 
 int vfb_get_stats(vfb_ctx *ctx, vfb_stats *out);
 
+/* collapse_ratio (directional clustering of sequencing errors).  Rows are ordered by count descending, then key bytes
+ * ascending (unsigned).  Key a may be the parent of key b when both have the same length and differ in exactly one byte,
+ * a comes first in the order and (double)count(a) >= ratio * (double)count(b) (one IEEE multiply, no FMA).  parent(b)
+ * is the first such a; every row's count goes to the end of its parent chain, and only those roots are returned.
+ * Rows with count 0 take no part and are not returned.  Wrong for libraries whose true members are one substitution
+ * apart (single-mutant scans): the most abundant member absorbs its neighbours.
+ *
+ * What the last collapsing finish did: rows with a non-zero count before, roots after, and ms = elapsed time on the
+ * device stream from the first collapse kernel to the last (the host waits between some launches for a 4-byte flag, and
+ * that wait is included).  All zero until a finish has collapsed.  A collapse takes at most 2^29 rows with a count
+ * (VFB_ERR_ARG beyond). */
+typedef struct vfb_collapse_info {
+    uint64_t rows_in;
+    uint64_t rows_out;
+    double ms;
+} vfb_collapse_info;
+int vfb_get_collapse_info(vfb_ctx *ctx, vfb_collapse_info *out);
+
+/* The same collapse over host columns (in->data holds in->key_bytes bytes, offsets[0] <= ... <= offsets[rows] <=
+ * key_bytes; owner ignored): uploaded to `device` (-1 = current), collapsed and compacted there, downloaded into malloc'd
+ * columns (out->owner = NULL; vfb_table_free frees them).  Counts must be below 2^56.  VFB_ERR_VALUE for a ratio that is
+ * not a finite number >= 1 and for a key that appears twice.  debug_hash_bits: tests only, as in vfb_params.  `info`
+ * may be NULL. */
+int vfb_collapse(const vfb_table *in, double ratio, int device, int debug_hash_bits, vfb_table *out, vfb_collapse_info *info);
+
 /* Diagnostics of the most recent batch (requires params.diagnostics = 1 and that the
  * last submit was a single batch).  Parity tests compare these with the oracle. */
 int vfb_get_diag(vfb_ctx *ctx, vfb_read_diag *out, uint64_t n_reads);
@@ -274,6 +302,9 @@ int vfb_multi_merge(vfb_multi *m);      /* afterwards context i holds exactly th
 int vfb_multi_finish(vfb_multi *m, vfb_table *out);          /* merge + export; columns owned by m            */
 int vfb_multi_finish_arrow(vfb_multi *m, vfb_arrow_array *out_array, vfb_arrow_schema *out_schema);
 int vfb_multi_get_stats(vfb_multi *m, vfb_stats *out);       /* summed over the devices                       */
+/* With collapse_ratio set, vfb_multi_finish* collapse the merged table on the first device (the merge partitions keys by
+ * hash, so neighbours sit on different devices); this reports that collapse. */
+int vfb_multi_get_collapse_info(vfb_multi *m, vfb_collapse_info *out);
 
 /* (2) One process per device (torchrun, MPI): the same keep-your-own-keys merge over NCCL send/recv, queued on the
  * context's compute stream, one host synchronisation.  libnccl.so.2 is loaded at run time (VFB_NCCL_LIB names
@@ -284,6 +315,7 @@ int vfb_nccl_unique_id(uint8_t *id128);
 int vfb_nccl_comm_init(const uint8_t *id128, uint32_t n_ranks, uint32_t rank, int device, void **comm_out);
 int vfb_nccl_comm_destroy(void *comm);
 int vfb_merge_nccl(vfb_ctx *ctx, void *comm, uint32_t rank, uint32_t n_ranks);
+/* (NCCL ranks collapse nothing themselves: the gathered result goes through vfb_collapse.) */
 
 /* (3) Any other transport: export the local table as n_parts self-describing chunks in device memory (every row,
  * the rank's own included), exchange them, clear, absorb the received chunks (the round-1 interface; the gloo

@@ -42,7 +42,8 @@ class Params(C.Structure):
                 ("table_capacity_hint", C.c_uint64),
                 ("debug_hash_bits", C.c_int32), ("force_generic_dp", C.c_int32),
                 ("dp_compute_all", C.c_int32), ("force_general_scan", C.c_int32),
-                ("dp_mode", C.c_int32), ("debug_win_cap", C.c_int32), ("both_strands", C.c_int32)]
+                ("dp_mode", C.c_int32), ("debug_win_cap", C.c_int32), ("both_strands", C.c_int32),
+                ("collapse_ratio", C.c_double)]
 
 
 class Table(C.Structure):
@@ -83,6 +84,13 @@ class Stats(C.Structure):
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
+
+
+class CollapseInfo(C.Structure):
+    _fields_ = [("rows_in", C.c_uint64), ("rows_out", C.c_uint64), ("ms", C.c_double)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
 
 
 class SynthCfg(C.Structure):
@@ -163,6 +171,9 @@ def load_library():
     L.vfb_multi_finish.argtypes = [vp, C.POINTER(Table)]
     L.vfb_multi_finish_arrow.argtypes = [vp, vp, vp]
     L.vfb_multi_get_stats.argtypes = [vp, C.POINTER(Stats)]
+    L.vfb_get_collapse_info.argtypes = [vp, C.POINTER(CollapseInfo)]
+    L.vfb_multi_get_collapse_info.argtypes = [vp, C.POINTER(CollapseInfo)]
+    L.vfb_collapse.argtypes = [C.POINTER(Table), C.c_double, i32, i32, C.POINTER(Table), C.POINTER(CollapseInfo)]
     L.vfb_nccl_available.restype = i32
     L.vfb_nccl_unique_id.argtypes = [vp]
     L.vfb_nccl_comm_init.argtypes = [vp, u32, u32, i32, C.POINTER(vp)]
@@ -206,7 +217,7 @@ def _make_params(L, adapters, match_score, mismatch_score, gap_open_penalty, gap
                  accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
                  show_progress, device, diagnostics, batch_reads, batch_bytes, table_capacity_hint,
                  debug_hash_bits, force_generic_dp, dp_compute_all, force_general_scan, dp_mode, debug_win_cap,
-                 both_strands=False):
+                 both_strands=False, collapse_ratio=None):
     p = Params()
     L.vfb_default_params(C.byref(p))
     pre = _as_bytes(adapters[0], "adapters[0]")
@@ -231,6 +242,7 @@ def _make_params(L, adapters, match_score, mismatch_score, gap_open_penalty, gap
     p.dp_mode = int(dp_mode)
     p.debug_win_cap = int(debug_win_cap)
     p.both_strands = 1 if both_strands else 0
+    p.collapse_ratio = collapse_ratio or 0.0          # validated by the callers
     return p, pre, suf          # the byte strings must outlive the call that reads p
 
 
@@ -242,9 +254,13 @@ class Context:
                  n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
                  device=None, diagnostics=False, batch_reads=0, batch_bytes=0,
                  table_capacity_hint=0, debug_hash_bits=0, force_generic_dp=False,
-                 dp_compute_all=False, force_general_scan=False, dp_mode=0, debug_win_cap=0, both_strands=False):
+                 dp_compute_all=False, force_general_scan=False, dp_mode=0, debug_win_cap=0, both_strands=False,
+                 collapse_ratio=None):
         """both_strands: a read without a region is searched once more as its reverse complement, on the device, and
-        a region found there is counted in the same table (a read counts on at most one strand)."""
+        a region found there is counted in the same table (a read counts on at most one strand).
+        collapse_ratio: every finish folds sequencing-error keys into their more abundant neighbours first (see
+        collapse_variants); the count table keeps every key, so further reads and another finish collapse them all."""
+        collapse_ratio = _ratio_arg(collapse_ratio, "collapse_ratio", True) or None
         L = load_library()
         self._lib = L
         self._h = C.c_void_p()
@@ -254,7 +270,7 @@ class Context:
                                                n_threads, queue_len, skip_translation, show_progress, device,
                                                diagnostics, batch_reads, batch_bytes, table_capacity_hint,
                                                debug_hash_bits, force_generic_dp, dp_compute_all, force_general_scan,
-                                               dp_mode, debug_win_cap, both_strands)
+                                               dp_mode, debug_win_cap, both_strands, collapse_ratio)
         _check(L.vfb_create(C.byref(p), C.byref(self._h)))
 
     @classmethod
@@ -343,6 +359,13 @@ class Context:
         _check(self._lib.vfb_get_stats(self._h, C.byref(s)))
         return s.as_dict()
 
+    def collapse_info(self) -> dict:
+        """What the last collapsing finish did: rows_in (keys with a count), rows_out (roots), ms (elapsed time of
+        the collapse on the device stream)."""
+        s = CollapseInfo()
+        _check(self._lib.vfb_get_collapse_info(self._h, C.byref(s)))
+        return s.as_dict()
+
     def diag(self, n):
         out = np.zeros(n, dtype=DIAG_DTYPE)
         _check(self._lib.vfb_get_diag(self._h, out.ctypes.data, n))
@@ -424,7 +447,8 @@ class MultiContext:
                  gap_extend_penalty=2, accept_prefix_alignment=0.75, accept_suffix_alignment=0.75,
                  n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
                  devices=None, batch_reads=0, batch_bytes=0, table_capacity_hint=0, debug_hash_bits=0, dp_mode=0,
-                 both_strands=False):
+                 both_strands=False, collapse_ratio=None):
+        collapse_ratio = _ratio_arg(collapse_ratio, "collapse_ratio", True) or None
         L = load_library()
         self._lib = L
         self._h = C.c_void_p()
@@ -432,7 +456,7 @@ class MultiContext:
                                                gap_extend_penalty, accept_prefix_alignment, accept_suffix_alignment,
                                                n_threads, queue_len, skip_translation, show_progress, None, False,
                                                batch_reads, batch_bytes, table_capacity_hint, debug_hash_bits,
-                                               False, False, False, dp_mode, 0, both_strands)
+                                               False, False, False, dp_mode, 0, both_strands, collapse_ratio)
         if devices is None:
             _check(L.vfb_multi_create(C.byref(p), None, 0, C.byref(self._h)))
         else:
@@ -488,6 +512,12 @@ class MultiContext:
     def stats(self) -> dict:
         s = Stats()
         _check(self._lib.vfb_multi_get_stats(self._h, C.byref(s)))
+        return s.as_dict()
+
+    def collapse_info(self) -> dict:
+        """The collapse of the merged table by the last finish (collapse_ratio)."""
+        s = CollapseInfo()
+        _check(self._lib.vfb_multi_get_collapse_info(self._h, C.byref(s)))
         return s.as_dict()
 
     def finish_arrays(self, copy=True):
@@ -576,6 +606,18 @@ def _float_arg(v, name):
     raise TypeError("argument '%s': must be real number, not %s" % (name, type(v).__name__))
 
 
+def _ratio_arg(v, name, optional):
+    """collapse_ratio: None (off, where optional) -> 0.0; else a finite real >= 1."""
+    if v is None and optional:
+        return 0.0
+    if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.floating, np.integer)):
+        raise TypeError("argument '%s': must be real number, not %s" % (name, type(v).__name__))
+    r = float(v)
+    if not (r >= 1.0 and r != float("inf")):
+        raise ValueError("argument '%s': must be a finite number >= 1, got %r" % (name, v))
+    return r
+
+
 def _bool_arg(v, name):
     if isinstance(v, (bool, np.bool_)):
         return bool(v)
@@ -586,7 +628,7 @@ def find_variants(fq_path, adapters, match_score=3, mismatch_score=-2, gap_open_
                   gap_extend_penalty=2, accept_prefix_alignment=0.75, accept_suffix_alignment=0.75,
                   n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
                   device=None, devices=None, batch_reads=0, table_capacity_hint=0, progress=None, allow_text=False,
-                  both_strands=False):
+                  both_strands=False, collapse_ratio=None):
     """Find variable regions flanked by adapters in a gzipped FASTQ dataset.
 
     Drop-in for `vfind.find_variants` (/root/reference/src/lib.rs:168-232): same positional
@@ -603,7 +645,10 @@ def find_variants(fq_path, adapters, match_score=3, mismatch_score=-2, gap_open_
     progress (callable(records, bytes_done, bytes_total), called about ten times per second),
     allow_text (read a file without the gzip magic as uncompressed FASTQ; the reference panics on it),
     both_strands (a read in which no region is found is searched once more as its reverse complement, on the GPU, and
-    counted in the same table: for libraries sequenced from both ends; a read counts on at most one strand).
+    counted in the same table: for libraries sequenced from both ends; a read counts on at most one strand),
+    collapse_ratio (a real >= 1: fold sequencing-error variants into a more abundant variant of the same length one
+    substitution away, on the GPU before the table leaves it; see collapse_variants — not for libraries whose members
+    are themselves one substitution apart).
     With show_progress (the default) and a terminal on stderr a one-line progress display is shown
     and cleared at the end, like the reference's spinner (src/lib.rs:265-269, :310).
     """
@@ -615,14 +660,14 @@ def find_variants(fq_path, adapters, match_score=3, mismatch_score=-2, gap_open_
     return _find_variants([fq_path], adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                           accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
                           show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text,
-                          both_strands)
+                          both_strands, collapse_ratio)
 
 
 def find_variants_multi(fq_paths, adapters, match_score=3, mismatch_score=-2, gap_open_penalty=5,
                         gap_extend_penalty=2, accept_prefix_alignment=0.75, accept_suffix_alignment=0.75,
                         n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
                         device=None, devices=None, batch_reads=0, table_capacity_hint=0, progress=None, allow_text=False,
-                        both_strands=False):
+                        both_strands=False, collapse_ratio=None):
     """find_variants over several FASTQ files (lanes, split runs) counted into ONE table, on one context
     (SURVEY §8(f) next-4).  Same arguments as find_variants; fq_paths is a non-empty sequence of paths."""
     if isinstance(fq_paths, (str, bytes, os.PathLike)) or not hasattr(fq_paths, "__iter__"):
@@ -633,12 +678,13 @@ def find_variants_multi(fq_paths, adapters, match_score=3, mismatch_score=-2, ga
     return _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                           accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
                           show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text,
-                          both_strands)
+                          both_strands, collapse_ratio)
 
 
 def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                    accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
-                   show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text, both_strands):
+                   show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text, both_strands,
+                   collapse_ratio):
     if not isinstance(adapters, (tuple, list)):
         raise TypeError("argument 'adapters': '%s' object cannot be converted to 'PyTuple'"
                         % type(adapters).__name__)
@@ -661,6 +707,7 @@ def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalt
     skip_translation = _bool_arg(skip_translation, "skip_translation")
     show_progress = _bool_arg(show_progress, "show_progress")
     both_strands = _bool_arg(both_strands, "both_strands")
+    collapse_ratio = _ratio_arg(collapse_ratio, "collapse_ratio", True) or None
 
     # The reference opens the file before validating thresholds (src/lib.rs:233 vs :239).
     for p in paths:
@@ -679,12 +726,14 @@ def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalt
         ctx = Context(adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                       accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len,
                       skip_translation, show_progress, device=devs[0], batch_reads=batch_reads,
-                      table_capacity_hint=table_capacity_hint, both_strands=both_strands)
+                      table_capacity_hint=table_capacity_hint, both_strands=both_strands,
+                      collapse_ratio=collapse_ratio)
     else:
         ctx = MultiContext(adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                            accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len,
                            skip_translation, show_progress, devices=devs, batch_reads=batch_reads,
-                           table_capacity_hint=table_capacity_hint, both_strands=both_strands)
+                           table_capacity_hint=table_capacity_hint, both_strands=both_strands,
+                           collapse_ratio=collapse_ratio)
     with ctx:
         shown = show_progress and progress is None and sys.stderr.isatty()
         if progress is not None:
@@ -704,6 +753,67 @@ def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalt
                 sys.stderr.write("\r" + " " * 60 + "\r")       # finish_and_clear
                 sys.stderr.flush()
         return batch_to_frame(ctx.finish_arrow())
+
+
+def collapse_variants(table, ratio, *, device=None, debug_hash_bits=0):
+    """Fold sequencing-error variants into their parents, on the GPU (directional clustering, as UMI-tools does).
+
+    `table` has columns `sequence` (string or binary) and `count` (unsigned): a pyarrow Table / RecordBatch or a
+    polars DataFrame, such as find_variants returns.  Rows are ordered by count descending, then sequence bytes
+    ascending.  Sequence a may be the parent of b when both have the same length and differ in exactly one byte
+    (Hamming distance 1: no indels), a comes first in the order and count(a) >= ratio * count(b) in float64.  parent(b)
+    is the first such a; each row's count goes to the end of its parent chain, so a sequence two substitutions from its
+    root can be folded in through an intermediate one.  One row per root comes back (rows with count 0 are dropped), in
+    the frame type find_variants returns, the sequence column as a string column if it was one, else binary.
+
+    ratio: a finite real >= 1 (ValueError otherwise; TypeError for a non-number).  A sequence that appears twice is a
+    ValueError.  Not for libraries whose true members are one substitution apart (single-mutant deep mutational
+    scanning): the wild type would absorb the mutants.  debug_hash_bits: tests only."""
+    import pyarrow as pa
+    ratio = _ratio_arg(ratio, "ratio", False)
+    if not isinstance(table, (pa.Table, pa.RecordBatch)) and hasattr(table, "to_arrow"):
+        table = table.to_arrow()                                       # polars.DataFrame
+    if isinstance(table, pa.RecordBatch):
+        table = pa.Table.from_batches([table])
+    if not isinstance(table, pa.Table):
+        raise TypeError("collapse_variants: expected a pyarrow Table / RecordBatch or a polars DataFrame, not %s"
+                        % type(table).__name__)
+    seq, cnt = table.column("sequence").combine_chunks(), table.column("count").combine_chunks()
+    # (polars exports its strings as string_view on recent versions)
+    is_type = lambda name: getattr(pa.types, "is_" + name, lambda t: False)(seq.type)
+    text = is_type("string") or is_type("large_string") or is_type("string_view")
+    if not (text or is_type("binary") or is_type("large_binary") or is_type("binary_view")):
+        raise TypeError("collapse_variants: column 'sequence' must be string or binary, not %s" % seq.type)
+    if seq.null_count or cnt.null_count:
+        raise ValueError("collapse_variants: null sequence or count")
+    try:
+        cnt = cnt.cast(pa.uint64())
+    except (pa.ArrowInvalid, pa.ArrowNotImplementedError) as e:
+        raise ValueError("collapse_variants: column 'count' must hold non-negative integers (%s)" % e) from None
+    seq = seq.cast(pa.large_binary())
+    n = len(seq)
+    offsets = np.zeros(n + 1, dtype=np.uint64)
+    data = np.zeros(0, dtype=np.uint8)
+    if n:
+        offsets = np.frombuffer(seq.buffers()[1], dtype=np.int64)[seq.offset:seq.offset + n + 1].astype(np.uint64)
+        if seq.buffers()[2] is not None:
+            data = np.frombuffer(seq.buffers()[2], dtype=np.uint8)
+    counts = np.ascontiguousarray(cnt.to_numpy(zero_copy_only=False), dtype=np.uint64)
+    L = load_library()
+    t_in = Table(n, data.size, offsets.ctypes.data_as(C.POINTER(C.c_uint64)), data.ctypes.data_as(C.POINTER(C.c_uint8)),
+                 counts.ctypes.data_as(C.POINTER(C.c_uint64)), None)
+    t_out = Table()
+    _check(L.vfb_collapse(C.byref(t_in), ratio, -1 if device is None else int(device), int(debug_hash_bits),
+                          C.byref(t_out), None))
+    o, d, c = _table_views(L, t_out, True)
+    typ = pa.large_string() if text else pa.large_binary()
+    tbl = pa.table({"sequence": pa.Array.from_buffers(typ, len(c), [None, pa.py_buffer(o.astype(np.int64)), pa.py_buffer(d)]),
+                    "count": pa.array(c, type=pa.uint64())})
+    try:
+        import polars as pl
+    except ImportError:
+        return tbl
+    return pl.from_arrow(tbl)
 
 
 def _visible_devices() -> int:

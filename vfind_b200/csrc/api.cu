@@ -562,6 +562,10 @@ int vfb_create(const vfb_params *p, vfb_ctx **out)
     int rc;
     for (int s = 0; s < 2; ++s)
         if ((rc = preflight(thr[s], &skip[s]))) return rc;   // :239, :249
+    if (p->collapse_ratio != 0. && !collapse_ratio_ok(p->collapse_ratio)) {
+        set_error("collapse_ratio must be 0 (off) or a finite number >= 1");
+        return VFB_ERR_VALUE;
+    }
     if (len[PRE] > VFB_MAX_SCAN_ADAPTER || len[SUF] > VFB_MAX_SCAN_ADAPTER) {
         set_error("adapters longer than 256 bases are not supported");
         return VFB_ERR_ARG;
@@ -1584,6 +1588,13 @@ static int diag_fetch(vfb_ctx *c, const DiagBufs &d, const DevBuf &start, const 
 
 extern "C" {
 
+int vfb_get_collapse_info(vfb_ctx *c, vfb_collapse_info *out)
+{
+    if (!c || !out) { set_error("null argument"); return VFB_ERR_ARG; }
+    *out = c->collapse_info;
+    return VFB_OK;
+}
+
 int vfb_get_diag(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
 {
     if (!c || !out) { set_error("null argument"); return VFB_ERR_ARG; }
@@ -1626,7 +1637,7 @@ int vfb_get_diag_reverse(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
 }  // extern "C"
 
 // Export, pass 1: slot counts -> row counts, sizes of what will be exported (rows with a non-zero count).
-int vfb_internal_export_sizes(vfb_ctx *c, uint64_t *rows_out, uint64_t *bytes_out)
+int vfb_internal_export_sizes(vfb_ctx *c, uint64_t *rows_out, uint64_t *bytes_out, bool collapse)
 {
     *rows_out = 0; *bytes_out = 0;
     int rc = vfb_sync(c);
@@ -1643,6 +1654,14 @@ int vfb_internal_export_sizes(vfb_ctx *c, uint64_t *rows_out, uint64_t *bytes_ou
     if ((rc = c->x_block_rows.ensure(nb * 8))) return rc;
     unsigned long long *d_totals = c->x_block_bytes.as<unsigned long long>() + nb;
     if ((rc = launch_export_counts(c->tab, rows, c->t_row_count.as<unsigned long long>(), c->st_compute))) return rc;
+    if (collapse) {
+        float ms = 0.f;
+        if ((rc = collapse_rows(c->tab.arena, c->tab.row_off, c->tab.row_len, c->t_row_count.as<unsigned long long>(), rows,
+                                c->prm.collapse_ratio, c->prm.debug_hash_bits, c->st_compute, &c->collapse_info.rows_in,
+                                &c->collapse_info.rows_out, &ms)))
+            return rc;
+        c->collapse_info.ms = ms;
+    }
     if ((rc = launch_export_sizes(c->tab, rows, c->t_row_count.as<unsigned long long>(), c->x_block_bytes.as<unsigned long long>(),
                                   c->x_block_rows.as<unsigned long long>(), d_totals, c->st_compute))) return rc;
     unsigned long long totals[2] = {0, 0};
@@ -1685,7 +1704,9 @@ int vfb_finish(vfb_ctx *c, vfb_table *out)
     if (!c || !out) { set_error("null argument"); return VFB_ERR_ARG; }
     memset(out, 0, sizeof *out);
     uint64_t rows = 0, bytes = 0;
-    int rc = vfb_internal_export_sizes(c, &rows, &bytes);
+    const bool collapse = c->prm.collapse_ratio != 0.;
+    if (collapse) c->collapse_info = vfb_collapse_info{};
+    int rc = vfb_internal_export_sizes(c, &rows, &bytes, collapse);
     if (rc) return rc;
     // The columns are compacted on the device and land in pinned host buffers owned by the
     // context (valid until the next vfb_finish / vfb_destroy on it).

@@ -236,13 +236,15 @@ struct vfb_ctx {
     std::vector<cudaEvent_t> evpool;   // 12 events per profiled batch, resolved at sync time
     size_t ev_used = 0;
     vfb_stats stats{};
+    vfb_collapse_info collapse_info{};   // the last finish that collapsed (collapse_ratio)
 };
 
 // ---- internal hooks between api.cu, ingest.cu and multi.cu (not part of the C ABI)
 // Export in two passes, so that several contexts can write consecutive pieces of ONE set of host columns:
 // sizes (synchronous: rows with a non-zero count and their key bytes), then offsets (+ byte_base) / counts / keys
-// copied to the given PINNED host pointers on the compute stream (asynchronous; vfb_sync waits).
-int vfb_internal_export_sizes(vfb_ctx *ctx, uint64_t *rows, uint64_t *key_bytes);
+// copied to the given PINNED host pointers on the compute stream (asynchronous; vfb_sync waits).  `collapse`: the
+// exported counts are collapsed first (prm.collapse_ratio; the count table keeps its rows and counts).
+int vfb_internal_export_sizes(vfb_ctx *ctx, uint64_t *rows, uint64_t *key_bytes, bool collapse);
 int vfb_internal_export_write(vfb_ctx *ctx, uint64_t byte_base, uint64_t *h_offsets, uint64_t *h_counts, uint8_t *h_data);
 // Merge building blocks.  export: partition the rows (all of them, or with self < n_parts only the rows other
 // parts own) into one chunk per part in the context's send buffer; sizes land in chunk_bytes / chunk_offsets

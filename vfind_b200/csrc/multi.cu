@@ -207,6 +207,7 @@ struct vfb_multi {
     std::vector<vfb_ctx *> ctx;
     bool peers_enabled = false;
     PinBuf h_offsets, h_counts, h_data;     // the merged result columns
+    vfb_collapse_info collapse_info{};      // the last finish that collapsed (collapse_ratio)
 };
 
 extern "C" {
@@ -372,7 +373,7 @@ static int multi_export(vfb_multi *m, uint64_t *rows_out, uint64_t *bytes_out)
     std::vector<uint64_t> rows(n), bytes(n);
     uint64_t tr = 0, tb = 0;
     for (size_t i = 0; i < n; ++i) {
-        if ((rc = vfb_internal_export_sizes(m->ctx[i], &rows[i], &bytes[i]))) return rc;
+        if ((rc = vfb_internal_export_sizes(m->ctx[i], &rows[i], &bytes[i], false))) return rc;
         tr += rows[i]; tb += bytes[i];
     }
     if ((rc = m->h_offsets.ensure((tr + 1) * 8))) return rc;
@@ -387,6 +388,26 @@ static int multi_export(vfb_multi *m, uint64_t *rows_out, uint64_t *bytes_out)
     if ((rc = vfb_multi_sync(m))) return rc;
     ((uint64_t *)m->h_offsets.p)[tr] = tb;
     *rows_out = tr; *bytes_out = tb;
+    const vfb_ctx *c0 = m->ctx[0];
+    if (c0->prm.collapse_ratio == 0.) return VFB_OK;
+    // keys are partitioned by hash, so neighbours sit on different devices: the merged columns go back to the first
+    // device and are collapsed there, the result overwriting them (it is never larger)
+    m->collapse_info = vfb_collapse_info{};
+    vfb_table in{tr, tb, (uint64_t *)m->h_offsets.p, (uint8_t *)m->h_data.p, (uint64_t *)m->h_counts.p, nullptr}, out;
+    auto alloc = [&](uint64_t, uint64_t, vfb_table *t) {
+        t->offsets = in.offsets; t->data = in.data; t->counts = in.counts;
+        return (int)VFB_OK;
+    };
+    rc = collapse_columns(in, c0->prm.collapse_ratio, c0->device, c0->prm.debug_hash_bits, alloc, &out, &m->collapse_info);
+    if (rc) return rc;
+    *rows_out = out.rows; *bytes_out = out.key_bytes;
+    return VFB_OK;
+}
+
+int vfb_multi_get_collapse_info(vfb_multi *m, vfb_collapse_info *out)
+{
+    if (!m || !out) { set_error("null argument"); return VFB_ERR_ARG; }
+    *out = m->collapse_info;
     return VFB_OK;
 }
 

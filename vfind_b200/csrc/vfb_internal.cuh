@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <functional>
 #include <string>
 
 #include "../../include/vfind_b200.h"
@@ -212,6 +213,24 @@ int launch_export_gather(const DevTable &t, uint64_t rows, const unsigned long l
                          const unsigned long long *block_bytes, const unsigned long long *block_rows,
                          unsigned long long byte_base, unsigned long long *offsets, unsigned long long *counts,
                          uint8_t *data, cudaStream_t st);
+
+// ---------------------------------------------------------------- collapse_ratio (kernels_collapse.cu)
+// Folds the rows of a row view (row r: keys[off[r] .. off[r] + len[r]), count[r]) into their roots, in place on `st`:
+// children end with count 0, each root with its group's sum (vfb_collapse_info in the header has the rule).  Synchronous.
+// *rows_in = rows with a non-zero count, *rows_out = roots, *ms = elapsed time on `st` from the first collapse kernel to
+// the last (it includes the host's waits between launches).  A key that appears twice is VFB_ERR_VALUE; more than
+// VFB_COLLAPSE_MAX_ROWS rows is VFB_ERR_ARG.
+int collapse_rows(const uint8_t *keys, const uint64_t *off, const uint32_t *len, unsigned long long *count, uint64_t rows,
+                  double ratio, int hash_bits, cudaStream_t st, uint64_t *rows_in, uint64_t *rows_out, float *ms);
+// ratio is finite and >= 1
+bool collapse_ratio_ok(double ratio);
+// most rows a collapse takes (a pass holds every row at one position at least)
+#define VFB_COLLAPSE_MAX_ROWS (1ull << 29)
+// collapse_rows over host columns on `device`: the result lands in the columns `alloc` gives it for its size (the
+// input's own buffers are fine: they have been uploaded by then, and the result is never larger).
+int collapse_columns(const vfb_table &in, double ratio, int device, int hash_bits,
+                     const std::function<int(uint64_t rows, uint64_t bytes, vfb_table *out)> &alloc, vfb_table *out,
+                     vfb_collapse_info *info);
 
 // ---------------------------------------------------------------- merge chunks
 // Chunk layout (all sections 16-byte aligned):
