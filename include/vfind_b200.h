@@ -270,6 +270,35 @@ int vfb_get_collapse_info(vfb_ctx *ctx, vfb_collapse_info *out);
  * may be NULL. */
 int vfb_collapse(const vfb_table *in, double ratio, int device, int debug_hash_bits, vfb_table *out, vfb_collapse_info *info);
 
+/* umi_length: count distinct molecules per variant from a UMI inside the read.  The UMI of a counted read is bytes
+ * [umi_offset, umi_offset + umi_length) of the read in the orientation its region was found in (the read as submitted,
+ * or its reverse complement for a read counted by the both_strands reverse pass), compared as raw bytes.  The key
+ * kernels append it to the key, so the table counts (variant, UMI) pairs; vfb_finish groups them by variant on the
+ * device and returns one row per variant with count = reads and molecules = distinct UMIs ("unique" method: no error
+ * correction, a UMI with a sequencing error is one more molecule).  A read with a key that is shorter than
+ * umi_offset + umi_length is not counted (vfb_umi_info.reads_short).
+ *
+ * vfb_set_umi: umi_length 0 = off (the default), at most 64; umi_offset + umi_length <= 65536; an offset needs a length.
+ * Only while the table is empty (after vfb_create, vfb_reset or vfb_table_clear): VFB_ERR_ARG otherwise.  VFB_ERR_VALUE
+ * for bad values and with collapse_ratio set (not supported together).  Validated before any device use.  Every context
+ * of a merge must use the same setting: with UMIs on, a row's owner is owner(hash(variant bytes)), so all rows of one
+ * variant land on one part. */
+int vfb_set_umi(vfb_ctx *ctx, uint32_t umi_offset, uint32_t umi_length);
+/* pairs: distinct (variant, UMI) rows grouped by the last finish; rows_out: variant rows it returned; reads_short:
+ * reads dropped for a short UMI since create or reset; ms: device time of the group-by, measured as
+ * vfb_collapse_info.ms is. */
+typedef struct vfb_umi_info {
+    uint64_t pairs;
+    uint64_t rows_out;
+    uint64_t reads_short;
+    double ms;
+} vfb_umi_info;
+int vfb_get_umi_info(vfb_ctx *ctx, vfb_umi_info *out);
+/* The molecules column of the last vfb_finish (pinned, rows entries aligned with its rows), owned and invalidated as the
+ * table's columns are.  VFB_ERR_ARG when UMIs are off.  vfb_finish_arrow returns it as a third child
+ * `molecules: uint64`. */
+int vfb_get_molecules(vfb_ctx *ctx, const uint64_t **col);
+
 /* Diagnostics of the most recent batch (requires params.diagnostics = 1 and that the
  * last submit was a single batch).  Parity tests compare these with the oracle. */
 int vfb_get_diag(vfb_ctx *ctx, vfb_read_diag *out, uint64_t n_reads);
@@ -305,6 +334,11 @@ int vfb_multi_get_stats(vfb_multi *m, vfb_stats *out);       /* summed over the 
 /* With collapse_ratio set, vfb_multi_finish* collapse the merged table on the first device (the merge partitions keys by
  * hash, so neighbours sit on different devices); this reports that collapse. */
 int vfb_multi_get_collapse_info(vfb_multi *m, vfb_collapse_info *out);
+/* umi_length on every device (vfb_set_umi).  Each device groups the variants it owns after the merge and writes its
+ * piece of the columns, molecules included; the info is summed over the devices (ms: the largest). */
+int vfb_multi_set_umi(vfb_multi *m, uint32_t umi_offset, uint32_t umi_length);
+int vfb_multi_get_umi_info(vfb_multi *m, vfb_umi_info *out);
+int vfb_multi_get_molecules(vfb_multi *m, const uint64_t **col);
 
 /* (2) One process per device (torchrun, MPI): the same keep-your-own-keys merge over NCCL send/recv, queued on the
  * context's compute stream, one host synchronisation.  libnccl.so.2 is loaded at run time (VFB_NCCL_LIB names

@@ -93,6 +93,13 @@ class CollapseInfo(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class UmiInfo(C.Structure):
+    _fields_ = [("pairs", C.c_uint64), ("rows_out", C.c_uint64), ("reads_short", C.c_uint64), ("ms", C.c_double)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 class SynthCfg(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("read_len", C.c_uint32), ("adapter_len", C.c_uint32),
                 ("region_len", C.c_uint32), ("n_variants", C.c_uint32), ("zipf", C.c_uint32),
@@ -174,6 +181,12 @@ def load_library():
     L.vfb_get_collapse_info.argtypes = [vp, C.POINTER(CollapseInfo)]
     L.vfb_multi_get_collapse_info.argtypes = [vp, C.POINTER(CollapseInfo)]
     L.vfb_collapse.argtypes = [C.POINTER(Table), C.c_double, i32, i32, C.POINTER(Table), C.POINTER(CollapseInfo)]
+    L.vfb_set_umi.argtypes = [vp, u32, u32]
+    L.vfb_multi_set_umi.argtypes = [vp, u32, u32]
+    L.vfb_get_umi_info.argtypes = [vp, C.POINTER(UmiInfo)]
+    L.vfb_multi_get_umi_info.argtypes = [vp, C.POINTER(UmiInfo)]
+    L.vfb_get_molecules.argtypes = [vp, C.POINTER(C.POINTER(C.c_uint64))]
+    L.vfb_multi_get_molecules.argtypes = [vp, C.POINTER(C.POINTER(C.c_uint64))]
     L.vfb_nccl_available.restype = i32
     L.vfb_nccl_unique_id.argtypes = [vp]
     L.vfb_nccl_comm_init.argtypes = [vp, u32, u32, i32, C.POINTER(vp)]
@@ -255,12 +268,15 @@ class Context:
                  device=None, diagnostics=False, batch_reads=0, batch_bytes=0,
                  table_capacity_hint=0, debug_hash_bits=0, force_generic_dp=False,
                  dp_compute_all=False, force_general_scan=False, dp_mode=0, debug_win_cap=0, both_strands=False,
-                 collapse_ratio=None):
+                 collapse_ratio=None, umi_length=None, umi_offset=0):
         """both_strands: a read without a region is searched once more as its reverse complement, on the device, and
         a region found there is counted in the same table (a read counts on at most one strand).
         collapse_ratio: every finish folds sequencing-error keys into their more abundant neighbours first (see
-        collapse_variants); the count table keeps every key, so further reads and another finish collapse them all."""
+        collapse_variants); the count table keeps every key, so further reads and another finish collapse them all.
+        umi_length / umi_offset: count distinct UMIs per variant (see find_variants); molecules() gives the column of
+        the last finish, finish_arrow() returns it as a third column."""
         collapse_ratio = _ratio_arg(collapse_ratio, "collapse_ratio", True) or None
+        umi = _umi_args(umi_length, umi_offset, collapse_ratio)
         L = load_library()
         self._lib = L
         self._h = C.c_void_p()
@@ -272,6 +288,8 @@ class Context:
                                                debug_hash_bits, force_generic_dp, dp_compute_all, force_general_scan,
                                                dp_mode, debug_win_cap, both_strands, collapse_ratio)
         _check(L.vfb_create(C.byref(p), C.byref(self._h)))
+        if umi[1]:
+            _check(L.vfb_set_umi(self._h, umi[0], umi[1]))
 
     @classmethod
     def _borrowed(cls, lib, handle):
@@ -366,6 +384,18 @@ class Context:
         _check(self._lib.vfb_get_collapse_info(self._h, C.byref(s)))
         return s.as_dict()
 
+    def umi_info(self) -> dict:
+        """umi_length: pairs ((variant, UMI) rows grouped by the last finish), rows_out (variant rows it returned),
+        reads_short (reads not counted because they are shorter than umi_offset + umi_length, since creation or reset)
+        and ms (device time of the group-by)."""
+        s = UmiInfo()
+        _check(self._lib.vfb_get_umi_info(self._h, C.byref(s)))
+        return s.as_dict()
+
+    def molecules(self):
+        """umi_length: the molecules column (uint64) of the last finish_arrays / finish_dict, aligned with its rows."""
+        return _molecules(self._lib.vfb_get_molecules, self._h, getattr(self, "_rows", 0))
+
     def diag(self, n):
         out = np.zeros(n, dtype=DIAG_DTYPE)
         _check(self._lib.vfb_get_diag(self._h, out.ctypes.data, n))
@@ -386,6 +416,7 @@ class Context:
         finish on this context or its close()."""
         t = Table()
         _check(self._lib.vfb_finish(self._h, C.byref(t)))
+        self._rows = int(t.rows)
         return _table_views(self._lib, t, copy)
 
     def finish_arrow(self):
@@ -425,6 +456,12 @@ class Context:
         _check(self._lib.vfb_merge_nccl(self._h, comm, rank, n_ranks))
 
 
+def _molecules(getter, h, rows):
+    col = C.POINTER(C.c_uint64)()
+    _check(getter(h, C.byref(col)))
+    return np.ctypeslib.as_array(col, shape=(rows,)).copy() if rows else np.zeros(0, np.uint64)
+
+
 def _table_views(lib, t, copy):
     try:
         rows, kb = int(t.rows), int(t.key_bytes)
@@ -447,8 +484,9 @@ class MultiContext:
                  gap_extend_penalty=2, accept_prefix_alignment=0.75, accept_suffix_alignment=0.75,
                  n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
                  devices=None, batch_reads=0, batch_bytes=0, table_capacity_hint=0, debug_hash_bits=0, dp_mode=0,
-                 both_strands=False, collapse_ratio=None):
+                 both_strands=False, collapse_ratio=None, umi_length=None, umi_offset=0):
         collapse_ratio = _ratio_arg(collapse_ratio, "collapse_ratio", True) or None
+        umi = _umi_args(umi_length, umi_offset, collapse_ratio)
         L = load_library()
         self._lib = L
         self._h = C.c_void_p()
@@ -465,6 +503,8 @@ class MultiContext:
             if not devs:
                 raise ValueError("devices must not be empty")
             _check(L.vfb_multi_create(C.byref(p), arr, len(devs), C.byref(self._h)))
+        if umi[1]:
+            _check(L.vfb_multi_set_umi(self._h, umi[0], umi[1]))
         self.n_devices = int(L.vfb_multi_devices(self._h))
         self.contexts = [Context._borrowed(L, L.vfb_multi_ctx(self._h, i)) for i in range(self.n_devices)]
 
@@ -520,9 +560,19 @@ class MultiContext:
         _check(self._lib.vfb_multi_get_collapse_info(self._h, C.byref(s)))
         return s.as_dict()
 
+    def umi_info(self) -> dict:
+        """Context.umi_info summed over the devices (ms: the slowest device's group-by)."""
+        s = UmiInfo()
+        _check(self._lib.vfb_multi_get_umi_info(self._h, C.byref(s)))
+        return s.as_dict()
+
+    def molecules(self):
+        return _molecules(self._lib.vfb_multi_get_molecules, self._h, getattr(self, "_rows", 0))
+
     def finish_arrays(self, copy=True):
         t = Table()
         _check(self._lib.vfb_multi_finish(self._h, C.byref(t)))
+        self._rows = int(t.rows)
         return _table_views(self._lib, t, copy)
 
     def finish_dict(self) -> dict:
@@ -618,6 +668,23 @@ def _ratio_arg(v, name, optional):
     return r
 
 
+def _umi_args(umi_length, umi_offset, collapse_ratio):
+    """(offset, length) for vfb_set_umi; (0, 0) = off.  Checked before any file is opened or device is used."""
+    if umi_length is None:
+        if umi_offset is not None and _int_arg(umi_offset, "umi_offset", 0, 2 ** 32 - 1):
+            raise ValueError("argument 'umi_offset': needs umi_length")
+        return 0, 0
+    k = _int_arg(umi_length, "umi_length", -(2 ** 63), 2 ** 63 - 1)
+    o = _int_arg(umi_offset, "umi_offset", -(2 ** 63), 2 ** 63 - 1)
+    if not 1 <= k <= 64:
+        raise ValueError("argument 'umi_length': must be between 1 and 64, got %d" % k)
+    if o < 0 or o + k > 65536:
+        raise ValueError("argument 'umi_offset': must be >= 0 with umi_offset + umi_length <= 65536, got %d" % o)
+    if collapse_ratio:
+        raise ValueError("umi_length cannot be combined with collapse_ratio")
+    return o, k
+
+
 def _bool_arg(v, name):
     if isinstance(v, (bool, np.bool_)):
         return bool(v)
@@ -628,7 +695,7 @@ def find_variants(fq_path, adapters, match_score=3, mismatch_score=-2, gap_open_
                   gap_extend_penalty=2, accept_prefix_alignment=0.75, accept_suffix_alignment=0.75,
                   n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
                   device=None, devices=None, batch_reads=0, table_capacity_hint=0, progress=None, allow_text=False,
-                  both_strands=False, collapse_ratio=None):
+                  both_strands=False, collapse_ratio=None, umi_length=None, umi_offset=0):
     """Find variable regions flanked by adapters in a gzipped FASTQ dataset.
 
     Drop-in for `vfind.find_variants` (/root/reference/src/lib.rs:168-232): same positional
@@ -648,7 +715,12 @@ def find_variants(fq_path, adapters, match_score=3, mismatch_score=-2, gap_open_
     counted in the same table: for libraries sequenced from both ends; a read counts on at most one strand),
     collapse_ratio (a real >= 1: fold sequencing-error variants into a more abundant variant of the same length one
     substitution away, on the GPU before the table leaves it; see collapse_variants — not for libraries whose members
-    are themselves one substitution apart).
+    are themselves one substitution apart),
+    umi_length / umi_offset (an integer 1..64 and an offset >= 0: bytes [umi_offset, umi_offset + umi_length) of each
+    counted read, in the orientation its region was found in, are its UMI; the result gains a column `molecules` = the
+    number of distinct UMIs among the variant's reads.  UMIs are compared as raw bytes with no error correction, so a
+    UMI with a sequencing error counts as one more molecule.  A read shorter than umi_offset + umi_length is not
+    counted.  Cannot be combined with collapse_ratio).
     With show_progress (the default) and a terminal on stderr a one-line progress display is shown
     and cleared at the end, like the reference's spinner (src/lib.rs:265-269, :310).
     """
@@ -660,14 +732,14 @@ def find_variants(fq_path, adapters, match_score=3, mismatch_score=-2, gap_open_
     return _find_variants([fq_path], adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                           accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
                           show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text,
-                          both_strands, collapse_ratio)
+                          both_strands, collapse_ratio, umi_length, umi_offset)
 
 
 def find_variants_multi(fq_paths, adapters, match_score=3, mismatch_score=-2, gap_open_penalty=5,
                         gap_extend_penalty=2, accept_prefix_alignment=0.75, accept_suffix_alignment=0.75,
                         n_threads=3, queue_len=2, skip_translation=False, show_progress=True, *,
                         device=None, devices=None, batch_reads=0, table_capacity_hint=0, progress=None, allow_text=False,
-                        both_strands=False, collapse_ratio=None):
+                        both_strands=False, collapse_ratio=None, umi_length=None, umi_offset=0):
     """find_variants over several FASTQ files (lanes, split runs) counted into ONE table, on one context
     (SURVEY §8(f) next-4).  Same arguments as find_variants; fq_paths is a non-empty sequence of paths."""
     if isinstance(fq_paths, (str, bytes, os.PathLike)) or not hasattr(fq_paths, "__iter__"):
@@ -678,13 +750,13 @@ def find_variants_multi(fq_paths, adapters, match_score=3, mismatch_score=-2, ga
     return _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                           accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
                           show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text,
-                          both_strands, collapse_ratio)
+                          both_strands, collapse_ratio, umi_length, umi_offset)
 
 
 def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                    accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len, skip_translation,
                    show_progress, device, devices, batch_reads, table_capacity_hint, progress, allow_text, both_strands,
-                   collapse_ratio):
+                   collapse_ratio, umi_length=None, umi_offset=0):
     if not isinstance(adapters, (tuple, list)):
         raise TypeError("argument 'adapters': '%s' object cannot be converted to 'PyTuple'"
                         % type(adapters).__name__)
@@ -708,6 +780,8 @@ def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalt
     show_progress = _bool_arg(show_progress, "show_progress")
     both_strands = _bool_arg(both_strands, "both_strands")
     collapse_ratio = _ratio_arg(collapse_ratio, "collapse_ratio", True) or None
+    umi_offset, umi_length = _umi_args(umi_length, umi_offset, collapse_ratio)
+    umi_length = umi_length or None
 
     # The reference opens the file before validating thresholds (src/lib.rs:233 vs :239).
     for p in paths:
@@ -727,13 +801,13 @@ def _find_variants(paths, adapters, match_score, mismatch_score, gap_open_penalt
                       accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len,
                       skip_translation, show_progress, device=devs[0], batch_reads=batch_reads,
                       table_capacity_hint=table_capacity_hint, both_strands=both_strands,
-                      collapse_ratio=collapse_ratio)
+                      collapse_ratio=collapse_ratio, umi_length=umi_length, umi_offset=umi_offset)
     else:
         ctx = MultiContext(adapters, match_score, mismatch_score, gap_open_penalty, gap_extend_penalty,
                            accept_prefix_alignment, accept_suffix_alignment, n_threads, queue_len,
                            skip_translation, show_progress, devices=devs, batch_reads=batch_reads,
                            table_capacity_hint=table_capacity_hint, both_strands=both_strands,
-                           collapse_ratio=collapse_ratio)
+                           collapse_ratio=collapse_ratio, umi_length=umi_length, umi_offset=umi_offset)
     with ctx:
         shown = show_progress and progress is None and sys.stderr.isatty()
         if progress is not None:
@@ -848,7 +922,7 @@ def _pick_devices(device, devices, paths):
 
 def read_diagnostics(reads, adapters, match_score=3, mismatch_score=-2, gap_open_penalty=5, gap_extend_penalty=2,
                      accept_prefix_alignment=0.75, accept_suffix_alignment=0.75, skip_translation=False, *,
-                     device=None, both_strands=False):
+                     device=None, both_strands=False, umi_length=None, umi_offset=0):
     """What find_variants decides for each read, as a pyarrow.Table with one row per read (SURVEY §8(f) next-3):
 
     exact_prefix / exact_suffix  leftmost exact adapter position, null when absent      (src/lib.rs:148)
@@ -866,8 +940,23 @@ def read_diagnostics(reads, adapters, match_score=3, mismatch_score=-2, gap_open
                                  ran (the read has a forward region, or is empty)
     region                       the bases that were counted: reverse-complemented for strand -1
 
+    With umi_length:
+
+    umi                          bytes [umi_offset, umi_offset + umi_length) of the read in the orientation its region
+                                 was found in (the reverse complement for strand -1); null where there is no region or
+                                 the read is too short
+
     `reads` is a sequence of str / bytes.  Runs the full DP (exact scores also for rejected alignments)."""
     import pyarrow as pa
+    umi_offset, umi_length = _umi_args(umi_length, umi_offset, None)
+
+    def with_umi(cols, oriented):
+        """oriented[i]: read i in its counted orientation, or None without a region"""
+        if umi_length:
+            cols["umi"] = pa.array([r[umi_offset:umi_offset + umi_length] if r is not None and len(r) >= umi_offset + umi_length
+                                    else None for r in oriented], type=pa.binary())
+        return pa.table(cols)
+
     seqs = [r if isinstance(r, bytes) else r.encode() for r in reads]
     n = len(seqs)
     length = np.array([len(s) for s in seqs], dtype=np.uint64)
@@ -908,7 +997,7 @@ def read_diagnostics(reads, adapters, match_score=3, mismatch_score=-2, gap_open
     if not both_strands:
         ok = (d["start"] >= 0) & (d["end"] >= 0) & (d["start"] < d["end"])
         cols["region"] = pa.array([seqs[i][d["start"][i]:d["end"][i]] if ok[i] else None for i in range(n)], type=pa.binary())
-        return pa.table(cols)
+        return with_umi(cols, [seqs[i] if ok[i] else None for i in range(n)])
     # the predicate that decides the retry (and that the key kernels use): both located, start < end <= len
     fwd = (d["start"] >= 0) & (d["end"] >= 0) & (d["start"] < d["end"]) & (d["end"].astype(np.int64) <= length.astype(np.int64))
     retried = ~fwd & (length > 0)
@@ -919,7 +1008,7 @@ def read_diagnostics(reads, adapters, match_score=3, mismatch_score=-2, gap_open
     cols["region"] = pa.array([seqs[i][d["start"][i]:d["end"][i]] if fwd[i] else
                                reverse_complement(seqs[i])[rd["start"][i]:rd["end"][i]] if rev[i] else None
                                for i in range(n)], type=pa.binary())
-    return pa.table(cols)
+    return with_umi(cols, [seqs[i] if fwd[i] else reverse_complement(seqs[i]) if rev[i] else None for i in range(n)])
 
 
 _RC = bytes.maketrans(b"ACGTUacgtu", b"TGCAAtgcaa")

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libvfind_b200.so")
 OBJ = os.path.join(HERE, "_obj")
-SOURCES = ["api.cu", "multi.cu", "ingest.cu", "pgunzip.cu", "gunzip_gpu.cu", "kernels_parse.cu", "kernels_inflate.cu", "kernels_scan.cu", "kernels_dp.cu", "kernels_dpw.cu", "kernels_count.cu", "kernels_misc.cu", "kernels_strand.cu", "kernels_collapse.cu"]
+SOURCES = ["api.cu", "multi.cu", "ingest.cu", "pgunzip.cu", "gunzip_gpu.cu", "kernels_parse.cu", "kernels_inflate.cu", "kernels_scan.cu", "kernels_dp.cu", "kernels_dpw.cu", "kernels_count.cu", "kernels_misc.cu", "kernels_strand.cu", "kernels_collapse.cu", "kernels_umi.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "-Xptxas", "-v"]

@@ -413,6 +413,7 @@ static void snaps_reset(vfb_ctx *c)           // the table was cleared (after a 
 // one (a submit), not a one-off (a merge's absorb).
 static int table_reserve(vfb_ctx *c, uint64_t new_keys, uint64_t new_bytes, bool stream_of_batches)
 {
+    c->table_used = true;
     snaps_poll(c, false);
     uint64_t want_rows = c->ub_rows + new_keys, want_arena = c->ub_arena + new_bytes;
     auto fits = [&]() {
@@ -708,15 +709,15 @@ int vfb_destroy(vfb_ctx *c)
     for (auto &side : c->side) side.d_code.release();
     c->diag_fwd.release(); c->diag_rev.release();
     DevBuf *bufs[] = {&c->d_generic_scratch, &c->t_slots,
-                      &c->t_row_hash, &c->t_row_off, &c->t_row_len, &c->t_row_slot, &c->t_arena, &c->t_counters, &c->t_row_count,
+                      &c->t_row_hash, &c->t_row_off, &c->t_row_len, &c->t_row_slot, &c->t_arena, &c->t_counters, &c->t_row_count, &c->t_row_mol,
                       &c->m_part_rows, &c->m_part_keys, &c->m_cursors, &c->m_chunk_off, &c->m_send, &c->m_recv,
                       &c->d_aligned_text, &c->d_span_sum,
-                      &c->x_block_bytes, &c->x_block_rows, &c->x_offsets, &c->x_counts, &c->x_data,
+                      &c->x_block_bytes, &c->x_block_rows, &c->x_offsets, &c->x_counts, &c->x_data, &c->x_mol,
                       &c->p_tiles, &c->p_line_end, &c->p_err, &c->g_tail, &c->g_info};
     for (auto *b : bufs) b->release();
     c->g_pin.release(); c->m_pin.release(); c->snap_pin.release();
     for (auto &sn : c->snaps) if (sn.ev) cudaEventDestroy(sn.ev);
-    c->h_offsets.release(); c->h_counts.release(); c->h_data.release();
+    c->h_offsets.release(); c->h_counts.release(); c->h_data.release(); c->h_mol.release();
     for (auto &ev : c->evpool) if (ev) cudaEventDestroy(ev);
     if (c->m_filled) cudaEventDestroy(c->m_filled);
     if (c->st_compute && c->own_compute_stream) cudaStreamDestroy(c->st_compute);
@@ -751,6 +752,7 @@ int vfb_table_clear(vfb_ctx *c)
     snaps_reset(c);
     VFB_CUDA(cudaMemsetAsync(c->tab.slots, 0, c->tab.capacity * 8 * VFB_SLOT_WORDS, c->st_compute));
     VFB_CUDA(cudaMemsetAsync(c->tab.counters, 0, 8 * 8, c->st_compute));
+    c->table_used = false;
     return VFB_OK;
 }
 
@@ -763,6 +765,35 @@ int vfb_reset(vfb_ctx *c)
     memset(&c->stats, 0, sizeof c->stats);
     c->stats.dp_kernel_kind = kind;
     c->diag_valid = false;
+    c->umi_info = vfb_umi_info{};
+    return VFB_OK;
+}
+
+}  // extern "C"
+
+// The values alone are checked first, so that they are rejected even without a context (and before any device use).
+int vfb_internal_umi_check(const vfb_ctx *c, uint32_t umi_offset, uint32_t umi_length)
+{
+    if (umi_length > 64) { set_error("umi_length must be at most 64"); return VFB_ERR_VALUE; }
+    if ((uint64_t)umi_offset + umi_length > 65536) { set_error("umi_offset + umi_length must be at most 65536"); return VFB_ERR_VALUE; }
+    if (umi_offset && !umi_length) { set_error("umi_offset needs a umi_length"); return VFB_ERR_VALUE; }
+    if (!c) { set_error("null context"); return VFB_ERR_ARG; }
+    if (umi_length && c->prm.collapse_ratio != 0.) {
+        set_error("umi_length cannot be combined with collapse_ratio");
+        return VFB_ERR_VALUE;
+    }
+    if (c->table_used) { set_error("umi_length can only be set while the table is empty (after create, reset or clear)"); return VFB_ERR_ARG; }
+    return VFB_OK;
+}
+
+extern "C" {
+
+int vfb_set_umi(vfb_ctx *c, uint32_t umi_offset, uint32_t umi_length)
+{
+    const int rc = vfb_internal_umi_check(c, umi_offset, umi_length);
+    if (rc) return rc;
+    c->umi_offset = umi_offset;
+    c->umi_len = umi_length;
     return VFB_OK;
 }
 
@@ -912,6 +943,7 @@ static int queue_keys_count(vfb_ctx *c, Lane &ln, cudaStream_t st, const Pass &p
     kj.klen = ln.d_klen.as<uint32_t>(); kj.khash = ln.d_khash.as<uint64_t>();
     kj.hash_bits = c->prm.debug_hash_bits;
     kj.flank_bytes = (uint32_t)(c->side[PRE].seq.size() + c->side[SUF].seq.size());
+    const UmiArgs umi{c->umi_offset, c->umi_len, ln.d_t64.as<unsigned long long>() + T_UMISHORT};
     // the table work of a batch claims slots by batch-relative index, and the fused key kernel reads slots without
     // fences: one batch at a time from here on
     bool k4_waited = false;
@@ -921,11 +953,11 @@ static int queue_keys_count(vfb_ctx *c, Lane &ln, cudaStream_t st, const Pass &p
     int frc = -1;
     if (c->fused_count && probe) {
         if (k4_wait) { VFB_CUDA(cudaStreamWaitEvent(st, c->ev_k4, 0)); k4_waited = true; }
-        frc = launch_keys_count(kj, c->tab, ln.d_c32.as<uint32_t>() + C_NMISS, st);
+        frc = launch_keys_count(kj, c->tab, ln.d_c32.as<uint32_t>() + C_NMISS, st, umi);
         if (frc > 0) return frc;
         if (frc == VFB_OK) { ij.n_keys_dev = ln.d_c32.as<uint32_t>() + C_NMISS; ++c->stats.fused_batches; }
     }
-    if (frc != VFB_OK && (rc = launch_keys(kj, st))) return rc;
+    if (frc != VFB_OK && (rc = launch_keys(kj, st, umi))) return rc;
     if (pev) VFB_CUDA(cudaEventRecord(pev[6], st));
 
     if (k4_wait && !k4_waited) VFB_CUDA(cudaStreamWaitEvent(st, c->ev_k4, 0));
@@ -968,7 +1000,7 @@ static int process_batch(vfb_ctx *c, const uint8_t *d_text, const vfb_span *d_sp
     for (int s = 0; s < 2; ++s)
         if (c->side[s].align) { if ((rc = ln.d_list[s].ensure((size_t)n * 4))) return rc; if ((rc = ln.d_fb[s].ensure((size_t)n * 4))) return rc; }
     // keys: sum of padded key lengths <= bytes/(3|1) + 16 per read
-    const uint64_t key_bytes_ub = (c->prm.skip_translation ? span_bytes_upper : span_bytes_upper / 3) + 16ull * n;
+    const uint64_t key_bytes_ub = (c->prm.skip_translation ? span_bytes_upper : span_bytes_upper / 3) + (16ull + c->umi_len) * n;
     if ((rc = ln.d_keys.ensure(key_bytes_ub))) return rc;
     if ((rc = ln.d_koff.ensure((size_t)n * 8))) return rc;
     if ((rc = ln.d_klen.ensure((size_t)n * 4))) return rc;
@@ -1595,6 +1627,30 @@ int vfb_get_collapse_info(vfb_ctx *c, vfb_collapse_info *out)
     return VFB_OK;
 }
 
+int vfb_get_umi_info(vfb_ctx *c, vfb_umi_info *out)
+{
+    if (!c || !out) { set_error("null argument"); return VFB_ERR_ARG; }
+    int rc = vfb_sync(c);
+    if (rc) return rc;
+    c->umi_info.reads_short = 0;
+    for (auto &ln : c->lanes) {
+        unsigned long long v = 0;
+        VFB_CUDA(cudaMemcpy(&v, ln.d_t64.as<unsigned long long>() + T_UMISHORT, 8, cudaMemcpyDeviceToHost));
+        c->umi_info.reads_short += v;
+    }
+    *out = c->umi_info;
+    return VFB_OK;
+}
+
+int vfb_get_molecules(vfb_ctx *c, const uint64_t **col)
+{
+    if (!c || !col) { set_error("null argument"); return VFB_ERR_ARG; }
+    if (!c->umi_len) { set_error("the context counts no UMIs (umi_length is off)"); return VFB_ERR_ARG; }
+    if (!c->mol_valid) { set_error("no vfb_finish has returned a molecules column since the last change"); return VFB_ERR_ARG; }
+    *col = (const uint64_t *)c->h_mol.p;
+    return VFB_OK;
+}
+
 int vfb_get_diag(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
 {
     if (!c || !out) { set_error("null argument"); return VFB_ERR_ARG; }
@@ -1640,6 +1696,9 @@ int vfb_get_diag_reverse(vfb_ctx *c, vfb_read_diag *out, uint64_t n_reads)
 int vfb_internal_export_sizes(vfb_ctx *c, uint64_t *rows_out, uint64_t *bytes_out, bool collapse)
 {
     *rows_out = 0; *bytes_out = 0;
+    // umi_info describes this finish, also when it finds no rows (reads_short is kept by the lanes)
+    c->umi_info.pairs = c->umi_info.rows_out = 0;
+    c->umi_info.ms = 0.;
     int rc = vfb_sync(c);
     if (rc) return rc;
     const uint64_t before = g_launches;
@@ -1662,8 +1721,16 @@ int vfb_internal_export_sizes(vfb_ctx *c, uint64_t *rows_out, uint64_t *bytes_ou
             return rc;
         c->collapse_info.ms = ms;
     }
+    if (c->umi_len) {
+        float ms = 0.f;
+        if ((rc = c->t_row_mol.ensure(rows * 8))) return rc;
+        if ((rc = umi_group_rows(c->tab, c->t_row_count.as<unsigned long long>(), c->t_row_mol.as<unsigned long long>(), rows,
+                                 c->umi_len, c->prm.debug_hash_bits, c->st_compute, &c->umi_info.pairs, &c->umi_info.rows_out, &ms)))
+            return rc;
+        c->umi_info.ms = ms;
+    }
     if ((rc = launch_export_sizes(c->tab, rows, c->t_row_count.as<unsigned long long>(), c->x_block_bytes.as<unsigned long long>(),
-                                  c->x_block_rows.as<unsigned long long>(), d_totals, c->st_compute))) return rc;
+                                  c->x_block_rows.as<unsigned long long>(), d_totals, c->st_compute, c->umi_len))) return rc;
     unsigned long long totals[2] = {0, 0};
     VFB_CUDA(cudaMemcpyAsync(totals, d_totals, 16, cudaMemcpyDeviceToHost, c->st_compute));
     VFB_CUDA(cudaStreamSynchronize(c->st_compute));
@@ -1676,7 +1743,8 @@ int vfb_internal_export_sizes(vfb_ctx *c, uint64_t *rows_out, uint64_t *bytes_ou
 
 // Export, pass 2 (asynchronous on the compute stream): h_offsets receives x_rows offsets (byte_base + ...; the
 // closing offset is the caller's), h_counts x_rows counts, h_data x_bytes key bytes.  Pinned destinations.
-int vfb_internal_export_write(vfb_ctx *c, uint64_t byte_base, uint64_t *h_offsets, uint64_t *h_counts, uint8_t *h_data)
+int vfb_internal_export_write(vfb_ctx *c, uint64_t byte_base, uint64_t *h_offsets, uint64_t *h_counts, uint8_t *h_data,
+                              uint64_t *h_molecules)
 {
     VFB_CUDA(cudaSetDevice(c->device));
     if (c->x_rows == 0) return VFB_OK;
@@ -1685,10 +1753,16 @@ int vfb_internal_export_write(vfb_ctx *c, uint64_t byte_base, uint64_t *h_offset
     if ((rc = c->x_offsets.ensure(c->x_rows * 8))) return rc;
     if ((rc = c->x_counts.ensure(c->x_rows * 8))) return rc;
     if ((rc = c->x_data.ensure(c->x_bytes ? c->x_bytes : 16))) return rc;
+    if (c->umi_len && (rc = c->x_mol.ensure(c->x_rows * 8))) return rc;
     if ((rc = launch_export_gather(c->tab, c->x_table_rows, c->t_row_count.as<unsigned long long>(),
                                    c->x_block_bytes.as<unsigned long long>(), c->x_block_rows.as<unsigned long long>(), byte_base,
                                    c->x_offsets.as<unsigned long long>(), c->x_counts.as<unsigned long long>(),
-                                   c->x_data.as<uint8_t>(), c->st_compute))) return rc;
+                                   c->x_data.as<uint8_t>(), c->st_compute, c->umi_len, c->t_row_mol.as<unsigned long long>(),
+                                   c->x_mol.as<unsigned long long>()))) return rc;
+    if (c->umi_len) {
+        VFB_CUDA(cudaMemcpyAsync(h_molecules, c->x_mol.p, c->x_rows * 8, cudaMemcpyDeviceToHost, c->st_compute));
+        c->stats.d2h_bytes += c->x_rows * 8;
+    }
     VFB_CUDA(cudaMemcpyAsync(h_offsets, c->x_offsets.p, c->x_rows * 8, cudaMemcpyDeviceToHost, c->st_compute));
     VFB_CUDA(cudaMemcpyAsync(h_counts, c->x_counts.p, c->x_rows * 8, cudaMemcpyDeviceToHost, c->st_compute));
     if (c->x_bytes) VFB_CUDA(cudaMemcpyAsync(h_data, c->x_data.p, c->x_bytes, cudaMemcpyDeviceToHost, c->st_compute));
@@ -1706,6 +1780,7 @@ int vfb_finish(vfb_ctx *c, vfb_table *out)
     uint64_t rows = 0, bytes = 0;
     const bool collapse = c->prm.collapse_ratio != 0.;
     if (collapse) c->collapse_info = vfb_collapse_info{};
+    c->mol_valid = false;
     int rc = vfb_internal_export_sizes(c, &rows, &bytes, collapse);
     if (rc) return rc;
     // The columns are compacted on the device and land in pinned host buffers owned by the
@@ -1713,15 +1788,17 @@ int vfb_finish(vfb_ctx *c, vfb_table *out)
     if ((rc = c->h_offsets.ensure((rows + 1) * 8))) return rc;
     if ((rc = c->h_counts.ensure((rows ? rows : 1) * 8))) return rc;
     if ((rc = c->h_data.ensure(bytes ? bytes : 16))) return rc;
+    if (c->umi_len && (rc = c->h_mol.ensure((rows ? rows : 1) * 8))) return rc;
     out->rows = rows;
     out->key_bytes = bytes;
     out->offsets = (uint64_t *)c->h_offsets.p;
     out->counts = (uint64_t *)c->h_counts.p;
     out->data = (uint8_t *)c->h_data.p;
     out->owner = c;
-    if ((rc = vfb_internal_export_write(c, 0, out->offsets, out->counts, out->data))) return rc;
+    if ((rc = vfb_internal_export_write(c, 0, out->offsets, out->counts, out->data, (uint64_t *)c->h_mol.p))) return rc;
     VFB_CUDA(cudaStreamSynchronize(c->st_compute));
     out->offsets[rows] = bytes;
+    c->mol_valid = c->umi_len != 0;
     return VFB_OK;
 }
 
@@ -1732,15 +1809,15 @@ int vfb_finish(vfb_ctx *c, vfb_table *out)
 namespace {
 struct ArrowHolder {
     std::atomic<int> refs{0};
-    PinBuf offsets, data, counts;
-    vfb_arrow_array children[2];
-    vfb_arrow_array *child_ptrs[2];
-    const void *seq_bufs[3], *cnt_bufs[2], *top_bufs[1];
+    PinBuf offsets, data, counts, molecules;
+    vfb_arrow_array children[3];
+    vfb_arrow_array *child_ptrs[3];
+    const void *seq_bufs[3], *cnt_bufs[2], *mol_bufs[2], *top_bufs[1];
 };
 void holder_unref(ArrowHolder *h)
 {
     if (h->refs.fetch_sub(1) == 1) {
-        h->offsets.release(); h->data.release(); h->counts.release();
+        h->offsets.release(); h->data.release(); h->counts.release(); h->molecules.release();
         delete h;
     }
 }
@@ -1755,21 +1832,21 @@ void arrow_top_release(vfb_arrow_array *a)
 {
     if (!a || !a->release) return;
     ArrowHolder *h = static_cast<ArrowHolder *>(a->private_data);
-    for (int i = 0; i < 2; ++i)                     // children the consumer has not moved out
+    for (int i = 0; i < 3; ++i)                     // children the consumer has not moved out
         if (h->children[i].release) h->children[i].release(&h->children[i]);
     a->release = nullptr;
     holder_unref(h);
 }
 struct SchemaHolder {
-    vfb_arrow_schema children[2];
-    vfb_arrow_schema *child_ptrs[2];
+    vfb_arrow_schema children[3];
+    vfb_arrow_schema *child_ptrs[3];
 };
 void schema_child_release(vfb_arrow_schema *s) { if (s) s->release = nullptr; }
 void schema_top_release(vfb_arrow_schema *s)
 {
     if (!s || !s->release) return;
     SchemaHolder *h = static_cast<SchemaHolder *>(s->private_data);
-    for (int i = 0; i < 2; ++i)
+    for (int i = 0; i < 3; ++i)
         if (h->children[i].release) h->children[i].release(&h->children[i]);
     s->release = nullptr;
     delete h;
@@ -1778,13 +1855,15 @@ void schema_top_release(vfb_arrow_schema *s)
 
 }  // extern "C"
 
-// Wraps three pinned columns (ownership moves into the array) as the Arrow struct array of vfb_finish_arrow.
+// Wraps three (four with molecules) pinned columns (ownership moves into the array) as the Arrow struct array of
+// vfb_finish_arrow.
 int vfb_internal_arrow_wrap(PinBuf offsets, PinBuf data, PinBuf counts, uint64_t rows, vfb_arrow_array *out_array,
-                            vfb_arrow_schema *out_schema)
+                            vfb_arrow_schema *out_schema, PinBuf molecules)
 {
+    const int n_ch = molecules.p ? 3 : 2;
     ArrowHolder *h = new ArrowHolder;
-    h->offsets = offsets; h->data = data; h->counts = counts;
-    h->refs = 3;
+    h->offsets = offsets; h->data = data; h->counts = counts; h->molecules = molecules;
+    h->refs = 1 + n_ch;
     h->seq_bufs[0] = nullptr; h->seq_bufs[1] = offsets.p; h->seq_bufs[2] = data.p;
     h->cnt_bufs[0] = nullptr; h->cnt_bufs[1] = counts.p;
     h->top_bufs[0] = nullptr;
@@ -1795,9 +1874,17 @@ int vfb_internal_arrow_wrap(PinBuf offsets, PinBuf data, PinBuf counts, uint64_t
     cnt.length = (int64_t)rows; cnt.n_buffers = 2; cnt.buffers = h->cnt_bufs;
     cnt.release = arrow_child_release; cnt.private_data = h;
     h->child_ptrs[0] = &seq; h->child_ptrs[1] = &cnt;
+    vfb_arrow_array &mol = h->children[2];
+    memset(&mol, 0, sizeof mol);
+    if (n_ch == 3) {
+        h->mol_bufs[0] = nullptr; h->mol_bufs[1] = molecules.p;
+        mol.length = (int64_t)rows; mol.n_buffers = 2; mol.buffers = h->mol_bufs;
+        mol.release = arrow_child_release; mol.private_data = h;
+        h->child_ptrs[2] = &mol;
+    }
     memset(out_array, 0, sizeof *out_array);
     out_array->length = (int64_t)rows; out_array->n_buffers = 1; out_array->buffers = h->top_bufs;
-    out_array->n_children = 2; out_array->children = h->child_ptrs;
+    out_array->n_children = n_ch; out_array->children = h->child_ptrs;
     out_array->release = arrow_top_release; out_array->private_data = h;
 
     SchemaHolder *sh = new SchemaHolder;
@@ -1805,8 +1892,12 @@ int vfb_internal_arrow_wrap(PinBuf offsets, PinBuf data, PinBuf counts, uint64_t
     sh->children[0].format = "U"; sh->children[0].name = "sequence"; sh->children[0].release = schema_child_release;
     sh->children[1].format = "L"; sh->children[1].name = "count"; sh->children[1].release = schema_child_release;
     sh->child_ptrs[0] = &sh->children[0]; sh->child_ptrs[1] = &sh->children[1];
+    if (n_ch == 3) {
+        sh->children[2].format = "L"; sh->children[2].name = "molecules"; sh->children[2].release = schema_child_release;
+        sh->child_ptrs[2] = &sh->children[2];
+    }
     memset(out_schema, 0, sizeof *out_schema);
-    out_schema->format = "+s"; out_schema->name = ""; out_schema->n_children = 2; out_schema->children = sh->child_ptrs;
+    out_schema->format = "+s"; out_schema->name = ""; out_schema->n_children = n_ch; out_schema->children = sh->child_ptrs;
     out_schema->release = schema_top_release; out_schema->private_data = sh;
     return VFB_OK;
 }
@@ -1819,10 +1910,13 @@ int vfb_finish_arrow(vfb_ctx *c, vfb_arrow_array *out_array, vfb_arrow_schema *o
     vfb_table t;
     int rc = vfb_finish(c, &t);
     if (rc) return rc;
-    // the context gives its pinned columns away; its next vfb_finish takes fresh ones from the pool
-    PinBuf o = c->h_offsets, d = c->h_data, n = c->h_counts;
+    // the context gives its pinned columns away; its next vfb_finish takes fresh ones from the pool.  The molecules
+    // column goes along only when this finish wrote it (h_mol may hold an earlier finish's column while UMIs are off).
+    PinBuf o = c->h_offsets, d = c->h_data, n = c->h_counts, mo = c->mol_valid ? c->h_mol : PinBuf();
     c->h_offsets = PinBuf(); c->h_data = PinBuf(); c->h_counts = PinBuf();
-    return vfb_internal_arrow_wrap(o, d, n, t.rows, out_array, out_schema);
+    if (c->mol_valid) c->h_mol = PinBuf();
+    c->mol_valid = false;
+    return vfb_internal_arrow_wrap(o, d, n, t.rows, out_array, out_schema, mo);
 }
 
 void vfb_table_free(vfb_table *t)
@@ -1854,7 +1948,7 @@ int vfb_internal_partition_count(vfb_ctx *c, uint32_t n_parts, uint32_t self, ui
     if ((rc = c->m_part_rows.ensure((size_t)n_parts * 16))) return rc;
     VFB_CUDA(cudaMemsetAsync(c->m_part_rows.p, 0, (size_t)n_parts * 16, c->st_compute));
     if (rows && (rc = launch_partition_count(c->tab, rows, n_parts, self, c->m_part_rows.as<unsigned long long>(),
-                                             c->m_part_rows.as<unsigned long long>() + n_parts, c->st_compute))) return rc;
+                                             c->m_part_rows.as<unsigned long long>() + n_parts, c->st_compute, c->umi_len))) return rc;
     if (table_rows) *table_rows = rows;
     bump_launches(c, before);
     return VFB_OK;
@@ -1873,7 +1967,8 @@ int vfb_internal_partition_fill(vfb_ctx *c, uint32_t n_parts, uint32_t self, boo
     VFB_CUDA(cudaMemcpyAsync(c->m_chunk_off.p, chunk_offsets, (size_t)n_parts * 8, cudaMemcpyHostToDevice, c->st_compute));
     if ((rc = launch_partition_fill(c->tab, c->x_table_rows, n_parts, self, release, d_buf,
                                     c->m_chunk_off.as<uint64_t>(), c->m_part_rows.as<uint64_t>(),
-                                    c->m_part_rows.as<uint64_t>() + n_parts, c->m_cursors.as<unsigned long long>(), c->st_compute)))
+                                    c->m_part_rows.as<uint64_t>() + n_parts, c->m_cursors.as<unsigned long long>(), c->st_compute,
+                                    c->umi_len)))
         return rc;
     bump_launches(c, before);
     return VFB_OK;

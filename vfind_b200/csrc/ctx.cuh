@@ -157,8 +157,10 @@ enum { C_NPRE = 0, C_NSUF, C_FBPRE, C_FBSUF, C_FB2PRE, C_FB2SUF, C_NWINPRE, C_NW
        C_NMISS = 160,        // fused key + count kernel: keys left for the insert kernels
        C_COUNT32 = 192 };
 // 64-bit device counters
-// (T_GATHER: the gather cursor of the batch; T_REVREADS / T_REVCOUNTED: both_strands statistics)
-enum { T_CELLS = 0, T_DPPRE, T_DPSUF, T_KEYBYTES, T_CELLSCOMP, T_WINDOWS, T_GATHER, T_REVREADS, T_REVCOUNTED, T_COUNT64 };
+// (T_GATHER: the gather cursor of the batch; T_REVREADS / T_REVCOUNTED: both_strands statistics; T_UMISHORT: reads
+// dropped for a short UMI)
+enum { T_CELLS = 0, T_DPPRE, T_DPSUF, T_KEYBYTES, T_CELLSCOMP, T_WINDOWS, T_GATHER, T_REVREADS, T_REVCOUNTED, T_UMISHORT,
+       T_COUNT64 };
 
 }  // namespace vfb
 
@@ -195,6 +197,7 @@ struct vfb_ctx {
     // table
     vfb::DevTable tab{};
     vfb::DevBuf t_slots, t_row_hash, t_row_off, t_row_len, t_row_slot, t_arena, t_counters, t_row_count;
+    vfb::DevBuf t_row_mol;                // umi_length: molecules of the group each exported row represents
     // Host-side upper bounds of rows / arena bytes = the last counter snapshot that has come back + what the batches
     // queued since may add.  A snapshot (rows, arena bytes) is copied to pinned memory behind every batch's insert
     // and picked up without blocking: the bounds stay within a few batches of the truth and no batch waits for them.
@@ -217,8 +220,8 @@ struct vfb_ctx {
     bool p_err_init = false;
 
     // export: device-side Arrow compaction and pinned host columns
-    vfb::DevBuf x_block_bytes, x_block_rows, x_offsets, x_counts, x_data;
-    vfb::PinBuf h_offsets, h_counts, h_data;
+    vfb::DevBuf x_block_bytes, x_block_rows, x_offsets, x_counts, x_data, x_mol;
+    vfb::PinBuf h_offsets, h_counts, h_data, h_mol;
     uint64_t x_rows = 0, x_bytes = 0, x_table_rows = 0;   // vfb_internal_export_sizes -> _write
 
     // merge scratch
@@ -237,6 +240,10 @@ struct vfb_ctx {
     size_t ev_used = 0;
     vfb_stats stats{};
     vfb_collapse_info collapse_info{};   // the last finish that collapsed (collapse_ratio)
+    uint32_t umi_offset = 0, umi_len = 0;   // vfb_set_umi (umi_len 0 = off)
+    vfb_umi_info umi_info{};             // the last finish that grouped UMIs (reads_short comes from the lanes)
+    bool table_used = false;             // a batch or an absorb may have added rows since create / clear
+    bool mol_valid = false;              // h_mol holds the molecules of the last vfb_finish
 };
 
 // ---- internal hooks between api.cu, ingest.cu and multi.cu (not part of the C ABI)
@@ -245,7 +252,9 @@ struct vfb_ctx {
 // copied to the given PINNED host pointers on the compute stream (asynchronous; vfb_sync waits).  `collapse`: the
 // exported counts are collapsed first (prm.collapse_ratio; the count table keeps its rows and counts).
 int vfb_internal_export_sizes(vfb_ctx *ctx, uint64_t *rows, uint64_t *key_bytes, bool collapse);
-int vfb_internal_export_write(vfb_ctx *ctx, uint64_t byte_base, uint64_t *h_offsets, uint64_t *h_counts, uint8_t *h_data);
+// With UMIs on, h_molecules receives x_rows molecule counts.
+int vfb_internal_export_write(vfb_ctx *ctx, uint64_t byte_base, uint64_t *h_offsets, uint64_t *h_counts, uint8_t *h_data,
+                              uint64_t *h_molecules = nullptr);
 // Merge building blocks.  export: partition the rows (all of them, or with self < n_parts only the rows other
 // parts own) into one chunk per part in the context's send buffer; sizes land in chunk_bytes / chunk_offsets
 // (synchronous for them), `m_filled` is recorded when the buffer is complete; exported rows give up their count
@@ -255,8 +264,11 @@ int vfb_internal_merge_export(vfb_ctx *ctx, uint32_t n_parts, uint32_t self, boo
 int vfb_internal_absorb_known(vfb_ctx *ctx, const uint8_t *d_chunk, uint64_t rows, uint64_t key_bytes);
 int vfb_internal_partition_count(vfb_ctx *ctx, uint32_t n_parts, uint32_t self, uint64_t *table_rows);
 int vfb_internal_partition_fill(vfb_ctx *ctx, uint32_t n_parts, uint32_t self, bool release, uint8_t *d_buf, const uint64_t *chunk_offsets);
+// `molecules` (umi_length; an empty buffer = none) becomes a third child.
 int vfb_internal_arrow_wrap(vfb::PinBuf offsets, vfb::PinBuf data, vfb::PinBuf counts, uint64_t rows,
-                            vfb_arrow_array *out_array, vfb_arrow_schema *out_schema);
+                            vfb_arrow_array *out_array, vfb_arrow_schema *out_schema, vfb::PinBuf molecules = vfb::PinBuf());
+// vfb_set_umi's checks that need no device
+int vfb_internal_umi_check(const vfb_ctx *ctx, uint32_t umi_offset, uint32_t umi_length);
 // One file over n_ctx contexts, one per device (ingest.cu).
 int vfb_internal_run_file(vfb_ctx **ctxs, uint32_t n_ctx, const char *path, uint32_t flags, uint64_t *n_reads_out);
 void bump_launches_for(vfb_ctx *ctx, uint64_t launches_before);

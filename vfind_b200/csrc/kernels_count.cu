@@ -129,9 +129,62 @@ __device__ __forceinline__ uint64_t k3_lane(const Key3Tables &T, const uint32_t 
     return acc;
 }
 
+// umi_length: appends the UMI (ulen bytes at `u`, read from global memory) to a key of kr bytes in out[]: key byte
+// kr + j = UMI byte j.  The hash accumulator is updated word by word (the region's partial last word is replaced), and
+// the composite key is zero-padded to 16 bytes.  No translation past kr.
+__device__ __forceinline__ void umi_append(const uint8_t *u, uint32_t ulen, uint32_t kr, uint32_t *out, uint64_t &acc,
+                                           const uint64_t *mult)
+{
+    const uintptr_t va = reinterpret_cast<uintptr_t>(u);
+    const uint32_t *g = reinterpret_cast<const uint32_t *>(va & ~(uintptr_t)3);
+    const uint32_t *limit = reinterpret_cast<const uint32_t *>((va + ulen + 3) & ~(uintptr_t)3);
+    const uint32_t sh = (uint32_t)(va & 3u) * 8u;
+    const uint32_t w0 = kr >> 2, d = kr & 3u, nw = (kr + ulen + 3) >> 2, npad = ((kr + ulen + 15u) & ~15u) >> 2;
+    uint32_t prev = 0, g0 = k3_word<false>(g, 0, limit);
+    for (uint32_t m = 0; w0 + m < nw; ++m) {
+        uint32_t um = 0;                                   // UMI bytes 4m .. 4m+3
+        if (4 * m < ulen) {
+            const uint32_t g1 = k3_word<false>(g, m + 1, limit);
+            um = __funnelshift_r(g0, g1, sh);
+            g0 = g1;
+            const uint32_t left = ulen - 4 * m;
+            if (left < 4) um &= (1u << (8 * left)) - 1u;
+        }
+        const uint32_t wi = w0 + m;
+        uint32_t word = __funnelshift_rc(prev, um, 32u - 8u * d);   // UMI bytes 4m - d .. 4m - d + 3
+        const uint64_t M = wi < KEY_MULTS ? mult[wi] : vfb_hash_mult(wi);
+        if (m == 0 && d) {
+            const uint32_t was = out[wi];
+            word |= was;
+            acc -= (uint64_t)(was ^ VFB_HASH_K) * M;
+        }
+        acc += (uint64_t)(word ^ VFB_HASH_K) * M;
+        out[wi] = word;
+        prev = um;
+    }
+    for (uint32_t wi = nw; wi < npad; ++wi) out[wi] = 0u;
+}
+
+// A read with a key (klen != 0, region at roff, V bytes) gets its UMI appended: klen grows by umi.len and uoff is where
+// the UMI sits in the text.  A read shorter than offset + len gets no key and is counted in n_short, unless its region
+// is not UTF-8 (a byte key that would not have been counted anyway; only the region is checked).
 template <bool TRANSLATE>
+__device__ __forceinline__ void umi_plan(const UmiArgs &umi, const KeyJob &job, const vfb_span &sp, uint32_t roff, uint32_t V,
+                                         uint32_t &klen, uint32_t &uoff, uint32_t &n_short)
+{
+    if (!klen) return;
+    if (sp.len < umi.offset + umi.len) {
+        n_short += (TRANSLATE || utf8_valid(job.text + roff, V)) ? 1u : 0u;
+        klen = 0;
+    } else {
+        klen += umi.len;
+        uoff = sp.off + umi.offset;
+    }
+}
+
+template <bool TRANSLATE, bool UMI>
 __global__ void __launch_bounds__(K3T_WARPS_MAX * 32)
-k3_keys_tile(const __grid_constant__ KeyJob job, const uint32_t tile_bytes)
+k3_keys_tile(const __grid_constant__ KeyJob job, const uint32_t tile_bytes, const __grid_constant__ UmiArgs umi)
 {
     extern __shared__ __align__(128) uint8_t dyn[];
     __shared__ Key3Tables T;
@@ -158,6 +211,7 @@ k3_keys_tile(const __grid_constant__ KeyJob job, const uint32_t tile_bytes)
     uint32_t *out32 = reinterpret_cast<uint32_t *>(tile + tile_bytes + K3T_SLACK);
     const uint32_t bar = k3_smem_u32(bars + warp), tile_s = k3_smem_u32(tile);
     uint32_t parity = 0;
+    uint32_t n_short = 0;                                  // UMI: reads of this warp's units whose UMI does not fit
     const uint32_t n_units = (job.n_reads + 31) / 32;
     for (uint32_t unit = blockIdx.x * n_warps + warp; unit < n_units; unit += gridDim.x * n_warps) {
         // ---- one lane per read: key length, key space (one atomic per 32 reads)
@@ -176,6 +230,8 @@ k3_keys_tile(const __grid_constant__ KeyJob job, const uint32_t tile_bytes)
                 }
             }
         }
+        uint32_t uoff = 0;                             // UMI: byte offset of the UMI in the text
+        if constexpr (UMI) umi_plan<TRANSLATE>(umi, job, job.spans[r], roff, V, klen, uoff, n_short);
         const unsigned owners = __ballot_sync(0xffffffffu, klen != 0);
         if (owners == 0) {
             if (r < job.n_reads) job.klen[r] = 0;
@@ -219,15 +275,17 @@ k3_keys_tile(const __grid_constant__ KeyJob job, const uint32_t tile_bytes)
         uint32_t high = 0;
         if (klen) {
             uint32_t *out = out_staged ? out32 + (local >> 2) : reinterpret_cast<uint32_t *>(job.keys + base + local);
+            const uint32_t kr = UMI ? klen - umi.len : klen;          // the region's part of the key
             if (staged) {
                 const uint32_t toff = lead_tile + (roff - lo);
-                acc = k3_lane<true, TRANSLATE>(T, tile32 + (toff >> 2), nullptr, (toff & 3u) * 8u, klen, out, high);
+                acc = k3_lane<true, TRANSLATE>(T, tile32 + (toff >> 2), nullptr, (toff & 3u) * 8u, kr, out, high);
             } else {
                 const uintptr_t va = reinterpret_cast<uintptr_t>(job.text + roff);
                 const uint32_t *limit = reinterpret_cast<const uint32_t *>((va + V + 3) & ~(uintptr_t)3);
                 acc = k3_lane<false, TRANSLATE>(T, reinterpret_cast<const uint32_t *>(va & ~(uintptr_t)3), limit,
-                                                (uint32_t)(va & 3u) * 8u, klen, out, high);
+                                                (uint32_t)(va & 3u) * 8u, kr, out, high);
             }
+            if constexpr (UMI) umi_append(job.text + uoff, umi.len, kr, out, acc, T.mult);
         }
         __syncwarp();
         if (out_staged) {
@@ -245,6 +303,11 @@ k3_keys_tile(const __grid_constant__ KeyJob job, const uint32_t tile_bytes)
         }
         if (r < job.n_reads) job.klen[r] = klen;
     }
+    if constexpr (UMI) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) n_short += __shfl_xor_sync(0xffffffffu, n_short, o);
+        if (lane == 0 && n_short) atomicAdd(umi.n_short, (unsigned long long)n_short);
+    }
 }
 
 // Shared memory of a k3_keys_tile block of `w` warps: their tiles and key staging (dynamic), the tables and barriers,
@@ -255,8 +318,8 @@ static constexpr size_t keys_tile_block_smem(size_t tile, int w)
 }
 static_assert(keys_tile_block_smem(VFB_TILE_BYTES_MAX, 1) <= VFB_SMEM_BLOCK_MAX, "a block of one warp fits any tile");
 
-template <bool TRANSLATE>
-static int launch_keys_tile(const KeyJob &job, cudaStream_t st)
+template <bool TRANSLATE, bool UMI>
+static int launch_keys_tile(const KeyJob &job, cudaStream_t st, const UmiArgs &umi)
 {
     const uint32_t tile = vfb_tile_bytes_for(job.text_bytes, job.n_reads);
     int best_w = 1, best_total = 0;
@@ -266,19 +329,21 @@ static int launch_keys_tile(const KeyJob &job, cudaStream_t st)
         if (bps * w > best_total) { best_total = bps * w; best_w = w; }
     }
     const size_t smem = (size_t)best_w * (tile + K3T_SLACK + K3T_OUT_BYTES);
-    VFB_CUDA(cudaFuncSetAttribute(k3_keys_tile<TRANSLATE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    VFB_CUDA(cudaFuncSetAttribute(k3_keys_tile<TRANSLATE, UMI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const uint32_t units = (job.n_reads + 31) / 32;
     uint32_t blocks = (units + best_w - 1) / best_w;
     const uint32_t cap = 148u * (uint32_t)(best_total / best_w);
     if (blocks > cap) blocks = cap;
-    k3_keys_tile<TRANSLATE><<<blocks, best_w * 32, smem, st>>>(job, tile);
+    k3_keys_tile<TRANSLATE, UMI><<<blocks, best_w * 32, smem, st>>>(job, tile, umi);
     return VFB_OK;
 }
 
-int launch_keys(const KeyJob &job, cudaStream_t st)
+int launch_keys(const KeyJob &job, cudaStream_t st, const UmiArgs &umi)
 {
     if (job.n_reads == 0) return VFB_OK;
-    const int rc = job.skip_translation ? launch_keys_tile<false>(job, st) : launch_keys_tile<true>(job, st);
+    int rc;
+    if (!umi.len) rc = job.skip_translation ? launch_keys_tile<false, false>(job, st, umi) : launch_keys_tile<true, false>(job, st, umi);
+    else rc = job.skip_translation ? launch_keys_tile<false, true>(job, st, umi) : launch_keys_tile<true, true>(job, st, umi);
     if (rc != VFB_OK) return rc;
     ++g_launches;
     VFB_CUDA(cudaGetLastError());
@@ -342,7 +407,10 @@ struct Key34Tables {
     uint32_t agg_cnt[K34_AGG];
 };
 
-// four amino acids of a group that holds a byte other than a canonical base: the per-byte tables (rare; out of line)
+// four amino acids of a group that holds a byte other than a canonical base: the per-byte tables (rare; out of line).
+// One copy per UMI mode: a copy called from one kernel only lets that kernel's tables stay where the compiler put them
+// before UMIs existed.
+template <bool UMI>
 __device__ __noinline__ uint32_t k34_group_slow(const Key3Tables *K, uint32_t x0, uint32_t x1, uint32_t x2)
 {
     const uint32_t i0 = K->lut25[x0 & 0xFFu] + K->lut5[(x0 >> 8) & 0xFFu] + K->lut1[(x0 >> 16) & 0xFFu];
@@ -353,12 +421,13 @@ __device__ __noinline__ uint32_t k34_group_slow(const Key3Tables *K, uint32_t x0
 }
 
 // twelve bases -> four amino acids (codon a = bytes 3a .. 3a+2 of the 12; translate, src/lib.rs:16-44)
+template <bool UMI>
 __device__ __forceinline__ uint32_t k34_group(const Key34Tables &T, uint32_t x0, uint32_t x1, uint32_t x2)
 {
     uint32_t i0, i1, i2, i3;
     if (tf_codons12(x0, x1, x2, i0, i1, i2, i3))
         return (uint32_t)T.codon[i0] | ((uint32_t)T.codon[i1] << 8) | ((uint32_t)T.codon[i2] << 16) | ((uint32_t)T.codon[i3] << 24);
-    return k34_group_slow(&T.k3, x0, x1, x2);
+    return k34_group_slow<UMI>(&T.k3, x0, x1, x2);
 }
 
 // The common case: region in the shared-memory tile, key block in shared memory, at most 32 key words.  The loop
@@ -372,6 +441,7 @@ __device__ __forceinline__ uint32_t k34_group_fast(const Key34Tables &T, uint32_
     return (uint32_t)T.codon[i0] | ((uint32_t)T.codon[i1] << 8) | ((uint32_t)T.codon[i2] << 16) | ((uint32_t)T.codon[i3] << 24);
 }
 
+template <bool UMI>
 __device__ __forceinline__ uint64_t k34_lane_hot(const Key34Tables &T, const uint32_t *w, uint32_t sh, uint32_t kl, uint32_t *out)
 {
     const uint32_t nw = (kl + 3) >> 2, npad = ((kl + 15u) & ~15u) >> 2;
@@ -406,7 +476,7 @@ __device__ __forceinline__ uint64_t k34_lane_hot(const Key34Tables &T, const uin
         const uint32_t g = (uint32_t)__ffs((int)bad) - 1u;
         bad &= bad - 1u;
         const uint32_t *q = w + 3 * g;
-        uint32_t word = k34_group_slow(&T.k3, __funnelshift_r(q[0], q[1], sh), __funnelshift_r(q[1], q[2], sh), __funnelshift_r(q[2], q[3], sh));
+        uint32_t word = k34_group_slow<UMI>(&T.k3, __funnelshift_r(q[0], q[1], sh), __funnelshift_r(q[1], q[2], sh), __funnelshift_r(q[2], q[3], sh));
         if (g + 1 == nw) word &= last_mask;
         const uint32_t was = out[g];
         acc += ((uint64_t)(word ^ VFB_HASH_K) - (uint64_t)(was ^ VFB_HASH_K)) * T.k3.mult[g];
@@ -416,7 +486,7 @@ __device__ __forceinline__ uint64_t k34_lane_hot(const Key34Tables &T, const uin
 }
 
 // Everything else: regions read from global memory, keys written straight to the batch's key space, long keys.
-template <bool SMEM>
+template <bool SMEM, bool UMI>
 __device__ __forceinline__ uint64_t k34_lane_translate(const Key34Tables &T, const uint32_t *w, const uint32_t *limit, uint32_t sh,
                                                        uint32_t kl, uint32_t *out)
 {
@@ -426,7 +496,7 @@ __device__ __forceinline__ uint64_t k34_lane_translate(const Key34Tables &T, con
     for (uint32_t wi = 0; wi < nw; ++wi) {
         const uint32_t t1 = k3_word<SMEM>(w, wp, limit), t2 = k3_word<SMEM>(w, wp + 1, limit), t3 = k3_word<SMEM>(w, wp + 2, limit);
         wp += 3;
-        uint32_t word = k34_group(T, __funnelshift_r(t0, t1, sh), __funnelshift_r(t1, t2, sh), __funnelshift_r(t2, t3, sh));
+        uint32_t word = k34_group<UMI>(T, __funnelshift_r(t0, t1, sh), __funnelshift_r(t1, t2, sh), __funnelshift_r(t2, t3, sh));
         t0 = t3;
         const uint32_t left = kl - 4 * wi;                 // key bytes from this word on, >= 1
         if (left < 4) word &= (1u << (8 * left)) - 1u;
@@ -551,10 +621,10 @@ __device__ __forceinline__ void k34_emit_misses(const KeyJob &job, uint32_t *n_m
 
 #define K34_WARPS_MAX 16
 
-template <bool TRANSLATE>
+template <bool TRANSLATE, bool UMI>
 __global__ void __maxnreg__(128)
 k34_keys_count(const __grid_constant__ KeyJob job, const __grid_constant__ DevTable tab, uint32_t *n_miss,
-               const uint32_t tile_bytes, const uint32_t out_bytes)
+               const uint32_t tile_bytes, const uint32_t out_bytes, const __grid_constant__ UmiArgs umi)
 {
     extern __shared__ __align__(128) uint8_t dyn[];
     __shared__ Key34Tables T;
@@ -589,6 +659,7 @@ k34_keys_count(const __grid_constant__ KeyJob job, const __grid_constant__ DevTa
     const uint64_t mask = tab.capacity - 1;
     uint32_t parity = 0;
     uint32_t my_hits = 0;                                  // reads this lane counted
+    uint32_t my_short = 0;                                 // UMI: reads of this lane whose UMI does not fit
     const uint32_t n_units = (job.n_reads + 31) / 32;
     const uint32_t stride = gridDim.x * n_warps;
 
@@ -628,6 +699,9 @@ k34_keys_count(const __grid_constant__ KeyJob job, const __grid_constant__ DevTa
 
     uint32_t unit = blockIdx.x * n_warps + warp;
     Plan cur;
+    // UMI: where the current / next unit's UMIs sit (the plans' klen include them; a unit's tile still covers the
+    // regions of reads whose UMI does not fit)
+    uint32_t cur_uoff = 0, nxt_uoff = 0;
     {
         const uint32_t r = unit * 32 + lane;
         const bool in = unit < n_units && r < job.n_reads;
@@ -635,6 +709,7 @@ k34_keys_count(const __grid_constant__ KeyJob job, const __grid_constant__ DevTa
         vfb_span sp; sp.off = 0; sp.len = 0;
         if (in) { s = job.start[r]; e = job.end[r]; sp = job.spans[r]; }
         cur = make_plan(in, s, e, sp);
+        if constexpr (UMI) umi_plan<TRANSLATE>(umi, job, sp, cur.roff, cur.V, cur.klen, cur_uoff, my_short);
         issue_tile(cur);
     }
     // pipeline registers: p1 = the previous unit (slot asked for), p2 = the one before (row asked for)
@@ -697,19 +772,21 @@ k34_keys_count(const __grid_constant__ KeyJob job, const __grid_constant__ DevTa
             if (klen) {
                 uint64_t acc;
                 uint32_t high = 0;
+                const uint32_t kr = UMI ? klen - umi.len : klen;      // the region's part of the key
                 if (cur.staged) {
                     const uint32_t toff = cur.lead + (cur.roff - cur.lo);
-                    if (TRANSLATE && out_staged && klen <= 128u)
-                        acc = k34_lane_hot(T, tile32 + (toff >> 2), (toff & 3u) * 8u, klen, blk + (local >> 2));
-                    else if (TRANSLATE) acc = k34_lane_translate<true>(T, tile32 + (toff >> 2), nullptr, (toff & 3u) * 8u, klen, out);
-                    else acc = k3_lane<true, false>(T.k3, tile32 + (toff >> 2), nullptr, (toff & 3u) * 8u, klen, out, high);
+                    if (TRANSLATE && out_staged && kr <= 128u)
+                        acc = k34_lane_hot<UMI>(T, tile32 + (toff >> 2), (toff & 3u) * 8u, kr, blk + (local >> 2));
+                    else if (TRANSLATE) acc = k34_lane_translate<true, UMI>(T, tile32 + (toff >> 2), nullptr, (toff & 3u) * 8u, kr, out);
+                    else acc = k3_lane<true, false>(T.k3, tile32 + (toff >> 2), nullptr, (toff & 3u) * 8u, kr, out, high);
                 } else {
                     const uintptr_t va = reinterpret_cast<uintptr_t>(job.text + cur.roff);
                     const uint32_t *limit = reinterpret_cast<const uint32_t *>((va + cur.V + 3) & ~(uintptr_t)3);
                     const uint32_t *w = reinterpret_cast<const uint32_t *>(va & ~(uintptr_t)3);
-                    if (TRANSLATE) acc = k34_lane_translate<false>(T, w, limit, (uint32_t)(va & 3u) * 8u, klen, out);
-                    else acc = k3_lane<false, false>(T.k3, w, limit, (uint32_t)(va & 3u) * 8u, klen, out, high);
+                    if (TRANSLATE) acc = k34_lane_translate<false, UMI>(T, w, limit, (uint32_t)(va & 3u) * 8u, kr, out);
+                    else acc = k3_lane<false, false>(T.k3, w, limit, (uint32_t)(va & 3u) * 8u, kr, out, high);
                 }
+                if constexpr (UMI) umi_append(job.text + cur_uoff, umi.len, kr, out, acc, T.k3.mult);
                 h = vfb_hash_finish(acc, klen);
                 if (job.hash_bits > 0 && job.hash_bits < 64) h &= (1ull << job.hash_bits) - 1;
                 // String::from_utf8 (:295): only regions holding a byte >= 0x80 need the validator
@@ -718,7 +795,8 @@ k34_keys_count(const __grid_constant__ KeyJob job, const __grid_constant__ DevTa
         }
         __syncwarp();                                      // the tile has been read by every lane
         // ---- the next unit's tile starts its journey now
-        const Plan nxt = make_plan(n_in, ns, ne, nsp);
+        Plan nxt = make_plan(n_in, ns, ne, nsp);
+        if constexpr (UMI) umi_plan<TRANSLATE>(umi, job, nsp, nxt.roff, nxt.V, nxt.klen, nxt_uoff, my_short);
         issue_tile(nxt);
 
         // ---- what was asked for an iteration ago has landed
@@ -826,6 +904,7 @@ k34_keys_count(const __grid_constant__ KeyJob job, const __grid_constant__ DevTa
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
         cur = nxt;
+        if constexpr (UMI) cur_uoff = nxt_uoff;
         bi = bi == 2u ? 0u : bi + 1u;
     }
     // ---- reads counted by this warp, block-level counts
@@ -838,21 +917,26 @@ k34_keys_count(const __grid_constant__ KeyJob job, const __grid_constant__ DevTa
             atomicAdd(&tab.counters[3], (unsigned long long)hits);
         }
     }
+    if constexpr (UMI) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) my_short += __shfl_xor_sync(0xffffffffu, my_short, o);
+        if (lane == 0 && my_short) atomicAdd(umi.n_short, (unsigned long long)my_short);
+    }
     __syncthreads();
     for (int e = threadIdx.x; e < K34_AGG; e += blockDim.x)
         if (T.agg_slot[e] != VFB_NONE && T.agg_cnt[e])
             atomicAdd(&tab.slots[(uint64_t)T.agg_slot[e] * VFB_SLOT_WORDS + 1], (unsigned long long)T.agg_cnt[e]);
 }
 
-template <bool TRANSLATE>
-static int launch_keys_count_t(const KeyJob &job, const DevTable &tab, uint32_t *n_miss, cudaStream_t st)
+template <bool TRANSLATE, bool UMI>
+static int launch_keys_count_t(const KeyJob &job, const DevTable &tab, uint32_t *n_miss, cudaStream_t st, const UmiArgs &umi)
 {
     const uint32_t tile = vfb_tile_bytes_for(job.text_bytes, job.n_reads);
     // a key block holds the 32 keys of a unit at their expected length (a third of what the adapters leave of the
-    // read for amino acids)
+    // read for amino acids, plus the UMI)
     const uint64_t stride = job.n_reads ? job.text_bytes / job.n_reads : 0;
     const uint64_t region_ub = stride > job.flank_bytes ? stride - job.flank_bytes : 0;
-    const uint64_t key_ub = TRANSLATE ? region_ub / 3 : region_ub;
+    const uint64_t key_ub = (TRANSLATE ? region_ub / 3 : region_ub) + umi.len;
     uint32_t out_bytes = (uint32_t)(32 * ((key_ub + 15) & ~15ull));
     if (out_bytes < 1024) out_bytes = 1024;
     if (out_bytes > 4096u) out_bytes = 4096u;
@@ -867,22 +951,25 @@ static int launch_keys_count_t(const KeyJob &job, const DevTable &tab, uint32_t 
     }
     if (best_total == 0) return -1;
     const size_t smem = (size_t)best_w * per_warp;
-    VFB_CUDA(cudaFuncSetAttribute(k34_keys_count<TRANSLATE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    VFB_CUDA(cudaFuncSetAttribute(k34_keys_count<TRANSLATE, UMI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const uint32_t units = (job.n_reads + 31) / 32;
     uint32_t blocks = (units + best_w - 1) / best_w;
     const uint32_t cap = 148u * (uint32_t)(best_total / best_w);
     if (blocks > cap) blocks = cap;
-    k34_keys_count<TRANSLATE><<<blocks, best_w * 32, smem, st>>>(job, tab, n_miss, tile, out_bytes);
+    k34_keys_count<TRANSLATE, UMI><<<blocks, best_w * 32, smem, st>>>(job, tab, n_miss, tile, out_bytes, umi);
     return VFB_OK;
 }
 
 // Fused key + count launch: afterwards *n_miss keys sit in job.koff / klen / khash (compact) for launch_insert.
 // Returns -1 when the tile kernel does not apply (the caller then runs launch_keys + launch_insert over all reads).
-int launch_keys_count(const KeyJob &job, const DevTable &tab, uint32_t *n_miss, cudaStream_t st)
+int launch_keys_count(const KeyJob &job, const DevTable &tab, uint32_t *n_miss, cudaStream_t st, const UmiArgs &umi)
 {
     if (job.n_reads == 0 || job.text_bytes == 0) return -1;
-    const int rc = job.skip_translation ? launch_keys_count_t<false>(job, tab, n_miss, st)
-                                        : launch_keys_count_t<true>(job, tab, n_miss, st);
+    int rc;
+    if (!umi.len) rc = job.skip_translation ? launch_keys_count_t<false, false>(job, tab, n_miss, st, umi)
+                                            : launch_keys_count_t<true, false>(job, tab, n_miss, st, umi);
+    else rc = job.skip_translation ? launch_keys_count_t<false, true>(job, tab, n_miss, st, umi)
+                                   : launch_keys_count_t<true, true>(job, tab, n_miss, st, umi);
     if (rc != VFB_OK) return rc;
     ++g_launches;
     VFB_CUDA(cudaGetLastError());
@@ -1121,15 +1208,16 @@ int launch_export_counts(const DevTable &t, uint64_t rows, unsigned long long *r
 // back to back (the arena pads every key to 16 bytes).
 #define EXP_ROWS 1024   // rows per block
 
+template <bool UMI>
 __global__ void __launch_bounds__(256)
 k_export_sums(const uint32_t *__restrict__ row_len, const unsigned long long *__restrict__ row_count, uint64_t rows,
-              unsigned long long *__restrict__ block_bytes, unsigned long long *__restrict__ block_rows)
+              unsigned long long *__restrict__ block_bytes, unsigned long long *__restrict__ block_rows, uint32_t trim)
 {
     __shared__ unsigned long long s_part[8], s_rows[8];
     const uint64_t r0 = (uint64_t)blockIdx.x * EXP_ROWS;
     unsigned long long acc = 0, kept = 0;
     for (uint32_t k = threadIdx.x; k < EXP_ROWS; k += 256)
-        if (r0 + k < rows && row_count[r0 + k]) { acc += row_len[r0 + k]; ++kept; }
+        if (r0 + k < rows && row_count[r0 + k]) { acc += row_len[r0 + k] - (UMI ? trim : 0u); ++kept; }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         acc += __shfl_xor_sync(0xffffffffu, acc, o);
@@ -1184,11 +1272,13 @@ k_export_scan(unsigned long long *block_sums, uint64_t n_blocks, unsigned long l
     if (threadIdx.x == 0) *total = s_carry;
 }
 
+template <bool UMI>
 __global__ void __launch_bounds__(256)
 k_export_gather(const DevTable t, uint64_t rows, const unsigned long long *__restrict__ row_count,
                 const unsigned long long *__restrict__ block_off, const unsigned long long *__restrict__ block_row,
                 unsigned long long byte_base, unsigned long long *__restrict__ offsets,
-                unsigned long long *__restrict__ counts, uint8_t *__restrict__ data)
+                unsigned long long *__restrict__ counts, uint8_t *__restrict__ data, uint32_t trim,
+                const unsigned long long *__restrict__ row_mol, unsigned long long *__restrict__ molecules)
 {
     __shared__ unsigned long long s_off[EXP_ROWS];       // ~0 = row not exported
     __shared__ unsigned long long s_warp[8];
@@ -1204,7 +1294,7 @@ k_export_gather(const DevTable t, uint64_t rows, const unsigned long long *__res
     for (int k = 0; k < 4; ++k) {
         const uint64_t r = r0 + threadIdx.x * 4 + k;
         cnt[k] = r < rows ? row_count[r] : 0ull;
-        len[k] = cnt[k] ? t.row_len[r] : 0u;
+        len[k] = cnt[k] ? t.row_len[r] - (UMI ? trim : 0u) : 0u;
         mine += len[k];
         mine_rows += cnt[k] ? 1u : 0u;
     }
@@ -1229,6 +1319,7 @@ k_export_gather(const DevTable t, uint64_t rows, const unsigned long long *__res
         if (cnt[k]) {
             offsets[ri] = byte_base + o;
             counts[ri] = cnt[k];
+            if (UMI) molecules[ri] = row_mol[r0 + threadIdx.x * 4 + k];
             ++ri;
         }
         o += len[k];
@@ -1239,7 +1330,7 @@ k_export_gather(const DevTable t, uint64_t rows, const unsigned long long *__res
         const uint64_t r = r0 + k;
         if (r >= rows) break;
         if (s_off[k] == ~0ull) continue;
-        const uint32_t n = t.row_len[r];
+        const uint32_t n = t.row_len[r] - (UMI ? trim : 0u);
         const uint8_t *src = t.arena + t.row_off[r];
         uint8_t *dst = data + s_off[k];
         for (uint32_t b = lane; b < n; b += 32) dst[b] = src[b];
@@ -1249,11 +1340,12 @@ k_export_gather(const DevTable t, uint64_t rows, const unsigned long long *__res
 // Pass 1: block sums and their scans; totals[0] = key bytes, totals[1] = rows that will be exported.
 int launch_export_sizes(const DevTable &t, uint64_t rows, const unsigned long long *row_count,
                         unsigned long long *block_bytes, unsigned long long *block_rows, unsigned long long *totals,
-                        cudaStream_t st)
+                        cudaStream_t st, uint32_t umi_len)
 {
     if (rows == 0) return VFB_OK;
     const uint64_t nb = (rows + EXP_ROWS - 1) / EXP_ROWS;
-    k_export_sums<<<(uint32_t)nb, 256, 0, st>>>(t.row_len, row_count, rows, block_bytes, block_rows);
+    if (umi_len) k_export_sums<true><<<(uint32_t)nb, 256, 0, st>>>(t.row_len, row_count, rows, block_bytes, block_rows, umi_len);
+    else k_export_sums<false><<<(uint32_t)nb, 256, 0, st>>>(t.row_len, row_count, rows, block_bytes, block_rows, 0);
     k_export_scan<<<1, 1024, 0, st>>>(block_bytes, nb, totals);
     k_export_scan<<<1, 1024, 0, st>>>(block_rows, nb, totals + 1);
     g_launches += 3;
@@ -1265,11 +1357,17 @@ int launch_export_sizes(const DevTable &t, uint64_t rows, const unsigned long lo
 int launch_export_gather(const DevTable &t, uint64_t rows, const unsigned long long *row_count,
                          const unsigned long long *block_bytes, const unsigned long long *block_rows,
                          unsigned long long byte_base, unsigned long long *offsets, unsigned long long *counts,
-                         uint8_t *data, cudaStream_t st)
+                         uint8_t *data, cudaStream_t st, uint32_t umi_len, const unsigned long long *row_mol,
+                         unsigned long long *molecules)
 {
     if (rows == 0) return VFB_OK;
     const uint64_t nb = (rows + EXP_ROWS - 1) / EXP_ROWS;
-    k_export_gather<<<(uint32_t)nb, 256, 0, st>>>(t, rows, row_count, block_bytes, block_rows, byte_base, offsets, counts, data);
+    if (umi_len)
+        k_export_gather<true><<<(uint32_t)nb, 256, 0, st>>>(t, rows, row_count, block_bytes, block_rows, byte_base, offsets, counts,
+                                                            data, umi_len, row_mol, molecules);
+    else
+        k_export_gather<false><<<(uint32_t)nb, 256, 0, st>>>(t, rows, row_count, block_bytes, block_rows, byte_base, offsets,
+                                                             counts, data, 0, nullptr, nullptr);
     ++g_launches;
     VFB_CUDA(cudaGetLastError());
     return VFB_OK;
@@ -1299,11 +1397,13 @@ __device__ __forceinline__ void part_group(uint32_t p, bool valid, uint32_t padd
 
 // Rows take part in a merge when their count is not zero and, if `self` names a part (self < n_parts), when
 // they are owned by another part: a rank keeps the rows it owns where they are.
+// UMI: the owner is that of the variant (the key without its last umi_len bytes); the chunk still carries the full hash.
+template <bool UMI>
 __device__ __forceinline__ bool part_of(const DevTable &t, uint64_t r, uint32_t n_parts, uint32_t self, uint64_t *h_out,
-                                        uint32_t *p_out, unsigned long long **cnt_out)
+                                        uint32_t *p_out, unsigned long long **cnt_out, uint32_t umi_len)
 {
     const uint64_t h = t.row_hash[r];
-    const uint32_t p = vfb_hash_owner(h, n_parts);
+    const uint32_t p = vfb_hash_owner(UMI ? vfb_hash_bytes(t.arena + t.row_off[r], t.row_len[r] - umi_len) : h, n_parts);
     *h_out = h;
     *p_out = p;
     if (p == self) return false;
@@ -1312,9 +1412,10 @@ __device__ __forceinline__ bool part_of(const DevTable &t, uint64_t r, uint32_t 
     return *cnt != 0ull;
 }
 
+template <bool UMI>
 __global__ void __launch_bounds__(256)
 k5_partition_count(const DevTable t, uint64_t rows, uint32_t n_parts,
-                   uint32_t self, unsigned long long *part_rows, unsigned long long *part_keybytes)
+                   uint32_t self, unsigned long long *part_rows, unsigned long long *part_keybytes, uint32_t umi_len)
 {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     const int lane = threadIdx.x & 31;
@@ -1323,7 +1424,7 @@ k5_partition_count(const DevTable t, uint64_t rows, uint32_t n_parts,
         uint64_t h = 0;
         uint32_t p = 0;
         unsigned long long *cnt = nullptr;
-        const bool valid = r < rows && part_of(t, r, n_parts, self, &h, &p, &cnt);
+        const bool valid = r < rows && part_of<UMI>(t, r, n_parts, self, &h, &p, &cnt, umi_len);
         const uint32_t padded = valid ? (t.row_len[r] + 15u) & ~15u : 0u;
         unsigned peers;
         uint32_t rank, brank, gbytes;
@@ -1337,12 +1438,13 @@ k5_partition_count(const DevTable t, uint64_t rows, uint32_t n_parts,
 
 int launch_partition_count(const DevTable &t, uint64_t rows, uint32_t n_parts,
                            uint32_t self, unsigned long long *part_rows, unsigned long long *part_keybytes,
-                           cudaStream_t st)
+                           cudaStream_t st, uint32_t umi_len)
 {
     if (rows == 0) return VFB_OK;
     uint64_t blocks = (rows + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;
-    k5_partition_count<<<(uint32_t)blocks, 256, 0, st>>>(t, rows, n_parts, self, part_rows, part_keybytes);
+    if (umi_len) k5_partition_count<true><<<(uint32_t)blocks, 256, 0, st>>>(t, rows, n_parts, self, part_rows, part_keybytes, umi_len);
+    else k5_partition_count<false><<<(uint32_t)blocks, 256, 0, st>>>(t, rows, n_parts, self, part_rows, part_keybytes, 0);
     ++g_launches;
     VFB_CUDA(cudaGetLastError());
     return VFB_OK;
@@ -1351,11 +1453,12 @@ int launch_partition_count(const DevTable &t, uint64_t rows, uint32_t n_parts,
 // Chunk headers are written by the kernel too (block 0), from the part sizes the count pass left on the device.  An
 // export of the whole table (self >= n_parts, vfb_table_partition_fill) gives every part a chunk, an empty one a
 // header of zero rows; a keep-own merge sends no chunk for an empty part, and its offset is the next part's.
+template <bool UMI>
 __global__ void __launch_bounds__(256)
 k5_partition_fill(const DevTable t, uint64_t rows, uint32_t n_parts, uint32_t self, bool release,
                   uint8_t *buf, const uint64_t *chunk_off,
                   const uint64_t *part_rows, const uint64_t *part_keybytes,
-                  unsigned long long *cursors)
+                  unsigned long long *cursors, uint32_t umi_len)
 {
     if (blockIdx.x == 0)
         for (uint32_t p = threadIdx.x; p < n_parts; p += blockDim.x)
@@ -1370,7 +1473,7 @@ k5_partition_fill(const DevTable t, uint64_t rows, uint32_t n_parts, uint32_t se
         uint64_t h = 0;
         uint32_t p = 0;
         unsigned long long *cnt = nullptr;
-        const bool valid = r < rows && part_of(t, r, n_parts, self, &h, &p, &cnt);
+        const bool valid = r < rows && part_of<UMI>(t, r, n_parts, self, &h, &p, &cnt, umi_len);
         const uint32_t len = valid ? t.row_len[r] : 0u;
         const uint32_t padded = (len + 15u) & ~15u;
         unsigned peers;
@@ -1407,13 +1510,17 @@ k5_partition_fill(const DevTable t, uint64_t rows, uint32_t n_parts, uint32_t se
 int launch_partition_fill(const DevTable &t, uint64_t rows, uint32_t n_parts, uint32_t self, bool release,
                           uint8_t *buf, const uint64_t *d_chunk_off, const uint64_t *d_part_rows,
                           const uint64_t *d_part_keybytes, unsigned long long *cursors,
-                          cudaStream_t st)
+                          cudaStream_t st, uint32_t umi_len)
 {
     uint64_t blocks = (rows + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;
     if (blocks < 1) blocks = 1;
-    k5_partition_fill<<<(uint32_t)blocks, 256, 0, st>>>(t, rows, n_parts, self, release, buf, d_chunk_off,
-                                                        d_part_rows, d_part_keybytes, cursors);
+    if (umi_len)
+        k5_partition_fill<true><<<(uint32_t)blocks, 256, 0, st>>>(t, rows, n_parts, self, release, buf, d_chunk_off,
+                                                                  d_part_rows, d_part_keybytes, cursors, umi_len);
+    else
+        k5_partition_fill<false><<<(uint32_t)blocks, 256, 0, st>>>(t, rows, n_parts, self, release, buf, d_chunk_off,
+                                                                   d_part_rows, d_part_keybytes, cursors, 0);
     ++g_launches;
     VFB_CUDA(cudaGetLastError());
     return VFB_OK;

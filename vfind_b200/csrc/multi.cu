@@ -207,6 +207,8 @@ struct vfb_multi {
     std::vector<vfb_ctx *> ctx;
     bool peers_enabled = false;
     PinBuf h_offsets, h_counts, h_data;     // the merged result columns
+    PinBuf h_mol;                           // umi_length: the molecules column
+    bool mol_valid = false;
     vfb_collapse_info collapse_info{};      // the last finish that collapsed (collapse_ratio)
 };
 
@@ -259,7 +261,7 @@ int vfb_multi_destroy(vfb_multi *m)
 {
     if (!m) return VFB_OK;
     for (vfb_ctx *c : m->ctx) vfb_destroy(c);
-    m->h_offsets.release(); m->h_counts.release(); m->h_data.release();
+    m->h_offsets.release(); m->h_counts.release(); m->h_data.release(); m->h_mol.release();
     delete m;
     return VFB_OK;
 }
@@ -367,8 +369,10 @@ int vfb_multi_get_stats(vfb_multi *m, vfb_stats *out)
 // Merge, then every device writes its partition into its piece of one set of pinned host columns.
 static int multi_export(vfb_multi *m, uint64_t *rows_out, uint64_t *bytes_out)
 {
+    m->mol_valid = false;
     int rc = vfb_multi_merge(m);
     if (rc) return rc;
+    const bool umi = m->ctx[0]->umi_len != 0;
     const size_t n = m->ctx.size();
     std::vector<uint64_t> rows(n), bytes(n);
     uint64_t tr = 0, tb = 0;
@@ -379,15 +383,17 @@ static int multi_export(vfb_multi *m, uint64_t *rows_out, uint64_t *bytes_out)
     if ((rc = m->h_offsets.ensure((tr + 1) * 8))) return rc;
     if ((rc = m->h_counts.ensure((tr ? tr : 1) * 8))) return rc;
     if ((rc = m->h_data.ensure(tb ? tb : 16))) return rc;
+    if (umi && (rc = m->h_mol.ensure((tr ? tr : 1) * 8))) return rc;
     uint64_t r0 = 0, b0 = 0;
     for (size_t i = 0; i < n; ++i) {
         if ((rc = vfb_internal_export_write(m->ctx[i], b0, (uint64_t *)m->h_offsets.p + r0, (uint64_t *)m->h_counts.p + r0,
-                                            (uint8_t *)m->h_data.p + b0))) return rc;
+                                            (uint8_t *)m->h_data.p + b0, umi ? (uint64_t *)m->h_mol.p + r0 : nullptr))) return rc;
         r0 += rows[i]; b0 += bytes[i];
     }
     if ((rc = vfb_multi_sync(m))) return rc;
     ((uint64_t *)m->h_offsets.p)[tr] = tb;
     *rows_out = tr; *bytes_out = tb;
+    m->mol_valid = umi;
     const vfb_ctx *c0 = m->ctx[0];
     if (c0->prm.collapse_ratio == 0.) return VFB_OK;
     // keys are partitioned by hash, so neighbours sit on different devices: the merged columns go back to the first
@@ -408,6 +414,37 @@ int vfb_multi_get_collapse_info(vfb_multi *m, vfb_collapse_info *out)
 {
     if (!m || !out) { set_error("null argument"); return VFB_ERR_ARG; }
     *out = m->collapse_info;
+    return VFB_OK;
+}
+
+int vfb_multi_set_umi(vfb_multi *m, uint32_t umi_offset, uint32_t umi_length)
+{
+    if (const int rc = vfb_internal_umi_check(m && !m->ctx.empty() ? m->ctx[0] : nullptr, umi_offset, umi_length)) return rc;
+    for (vfb_ctx *c : m->ctx) { const int rc = vfb_internal_umi_check(c, umi_offset, umi_length); if (rc) return rc; }
+    for (vfb_ctx *c : m->ctx) { const int rc = vfb_set_umi(c, umi_offset, umi_length); if (rc) return rc; }
+    return VFB_OK;
+}
+
+int vfb_multi_get_umi_info(vfb_multi *m, vfb_umi_info *out)
+{
+    if (!m || !out) { set_error("null argument"); return VFB_ERR_ARG; }
+    memset(out, 0, sizeof *out);
+    for (vfb_ctx *c : m->ctx) {
+        vfb_umi_info u;
+        const int rc = vfb_get_umi_info(c, &u);
+        if (rc) return rc;
+        out->pairs += u.pairs; out->rows_out += u.rows_out; out->reads_short += u.reads_short;
+        if (u.ms > out->ms) out->ms = u.ms;
+    }
+    return VFB_OK;
+}
+
+int vfb_multi_get_molecules(vfb_multi *m, const uint64_t **col)
+{
+    if (!m || !col || m->ctx.empty()) { set_error("null argument"); return VFB_ERR_ARG; }
+    if (!m->ctx[0]->umi_len) { set_error("the context counts no UMIs (umi_length is off)"); return VFB_ERR_ARG; }
+    if (!m->mol_valid) { set_error("no vfb_multi_finish has returned a molecules column since the last change"); return VFB_ERR_ARG; }
+    *col = (const uint64_t *)m->h_mol.p;
     return VFB_OK;
 }
 
@@ -432,9 +469,11 @@ int vfb_multi_finish_arrow(vfb_multi *m, vfb_arrow_array *out_array, vfb_arrow_s
     uint64_t rows = 0, bytes = 0;
     const int rc = multi_export(m, &rows, &bytes);
     if (rc) return rc;
-    PinBuf o = m->h_offsets, d = m->h_data, n = m->h_counts;
+    PinBuf o = m->h_offsets, d = m->h_data, n = m->h_counts, mo = m->mol_valid ? m->h_mol : PinBuf();
     m->h_offsets = PinBuf(); m->h_data = PinBuf(); m->h_counts = PinBuf();
-    return vfb_internal_arrow_wrap(o, d, n, rows, out_array, out_schema);
+    if (m->mol_valid) m->h_mol = PinBuf();
+    m->mol_valid = false;
+    return vfb_internal_arrow_wrap(o, d, n, rows, out_array, out_schema, mo);
 }
 
 }  // extern "C"

@@ -159,12 +159,19 @@ struct KeyJob {
     int hash_bits;            // 0 = 64
     uint32_t flank_bytes;     // prefix + suffix adapter length: a region is at most a read minus this (sizes key blocks)
 };
-int launch_keys(const KeyJob &job, cudaStream_t st);
+// umi_length: the key kernels append bytes [offset, offset + len) of the read (in the orientation of the pass) to every
+// key, so the table counts (variant, UMI) pairs.  A read with a key but fewer than offset + len bytes gets no key and
+// is counted in *n_short.  len = 0: off (the kernels without UMIs run).
+struct UmiArgs {
+    uint32_t offset, len;
+    unsigned long long *n_short;
+};
+int launch_keys(const KeyJob &job, cudaStream_t st, const UmiArgs &umi);
 struct DevTable;
 // Fused keys + count (k34_keys_count): reads whose key already has a row in `tab` are counted by the key kernel;
 // the others are left in job.koff / klen / khash as a compact list of *n_miss entries for launch_insert
 // (InsertJob::n_keys_dev).  -1: the tile kernel does not apply to this batch (run launch_keys + launch_insert).
-int launch_keys_count(const KeyJob &job, const DevTable &tab, uint32_t *n_miss, cudaStream_t st);
+int launch_keys_count(const KeyJob &job, const DevTable &tab, uint32_t *n_miss, cudaStream_t st, const UmiArgs &umi);
 
 // Open-addressing table in device memory.  A slot is ONE 32-byte sector of four words:
 //   [0] (tag << 32 | ref)   tag = high 32 hash bits, ref = row id + 1 (bit31 clear) or, only inside the
@@ -205,14 +212,24 @@ int launch_rehash(const DevTable &old_t, const DevTable &new_t, cudaStream_t st)
 int launch_export_counts(const DevTable &t, uint64_t rows, unsigned long long *row_count, cudaStream_t st);
 // Export of the rows with a non-zero count, in two passes: sizes (block_bytes / block_rows hold ceil(rows/1024)
 // words of scratch each; totals[0] = key bytes, totals[1] = exported rows), then offsets (+ byte_base), counts and
-// the keys back to back.
+// the keys back to back.  umi_len > 0 (grouped UMI rows): every key loses its last umi_len bytes, and the gather writes
+// row_mol of each exported row to `molecules`.
 int launch_export_sizes(const DevTable &t, uint64_t rows, const unsigned long long *row_count,
                         unsigned long long *block_bytes, unsigned long long *block_rows, unsigned long long *totals,
-                        cudaStream_t st);
+                        cudaStream_t st, uint32_t umi_len = 0);
 int launch_export_gather(const DevTable &t, uint64_t rows, const unsigned long long *row_count,
                          const unsigned long long *block_bytes, const unsigned long long *block_rows,
                          unsigned long long byte_base, unsigned long long *offsets, unsigned long long *counts,
-                         uint8_t *data, cudaStream_t st);
+                         uint8_t *data, cudaStream_t st, uint32_t umi_len = 0, const unsigned long long *row_mol = nullptr,
+                         unsigned long long *molecules = nullptr);
+
+// ---------------------------------------------------------------- umi_length (kernels_umi.cu)
+// Groups the (variant, UMI) rows of the export's count column by variant (the key without its last umi_len bytes): each
+// group's first-claiming row ends with the group's summed count and row_mol = its number of rows, the other rows with
+// count 0.  Membership is decided on the variant bytes.  Synchronous; *pairs = rows with a count, *groups = variant
+// rows, *ms = elapsed time on `st`.  row_mol holds `rows` words.
+int umi_group_rows(const DevTable &t, unsigned long long *count, unsigned long long *row_mol, uint64_t rows, uint32_t umi_len,
+                   int hash_bits, cudaStream_t st, uint64_t *pairs, uint64_t *groups, float *ms);
 
 // ---------------------------------------------------------------- collapse_ratio (kernels_collapse.cu)
 // Folds the rows of a row view (row r: keys[off[r] .. off[r] + len[r]), count[r]) into their roots, in place on `st`:
@@ -247,14 +264,15 @@ __host__ __device__ __forceinline__ uint64_t chunk_bytes_for(uint64_t rows, uint
 }
 // `self` < n_parts: rows owned by that part stay where they are (keep-own merge); self >= n_parts: every row
 // with a non-zero count is exported.  `release`: the rows written to a chunk give up their count (they keep their
-// slot, so a later read with the same key finds the row again).
+// slot, so a later read with the same key finds the row again).  umi_len > 0: a row's owner is that of the hash of
+// its key without the last umi_len bytes, so all (variant, UMI) rows of one variant go to one part.
 int launch_partition_count(const DevTable &t, uint64_t rows, uint32_t n_parts,
                            uint32_t self, unsigned long long *part_rows, unsigned long long *part_keybytes,
-                           cudaStream_t st);
+                           cudaStream_t st, uint32_t umi_len);
 int launch_partition_fill(const DevTable &t, uint64_t rows, uint32_t n_parts, uint32_t self, bool release,
                           uint8_t *buf, const uint64_t *d_chunk_off, const uint64_t *d_part_rows,
                           const uint64_t *d_part_keybytes, unsigned long long *cursors,
-                          cudaStream_t st);
+                          cudaStream_t st, uint32_t umi_len);
 
 // ---------------------------------------------------------------- FASTQ parse (ingest)
 // d_text holds n_lines complete lines (n_records = n_lines / 4 records, text starts at a record
